@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BSR sampling hot path on B200: MH proposals scored/s (+ tree-node evals/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5|c1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5|c1] [--dump-outputs DIR]
 
 A *step* is `sweeps_per_step` sweeps (each sweep = K newProp calls per chain, codes/bsr_class.py:179) of every chain over
 the synthetic data set.  Default workload = BASELINE.json configs[1] (SURVEY.md C2): K=3, 4096 chains, n=1000 rows, d=2, and
@@ -559,9 +559,33 @@ def setup_engine(D, args, name, w):
     return eng, run, X, y, C, n, lo
 
 
-def measure(D, args, name, w, steps, warmup, full):
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, eng, stats, chain_offset):
+    """--dump-outputs: what the timed bsr_run calls leave for their caller -- bsr_get_stats and the live and the reported
+    trees (bsr_get_trees) of this rank's chains -- as float64 DIR/<name>.npy, first axis = chain.  Tree tokens are
+    op | op_ind << 8 | feature << 16 (include/bsr_b200.h); slots past a tree's node count are written as 0.  When the chains
+    need more than DUMP_BYTES, a fixed seeded sample of them is written; chain_id.npy holds the global ids written."""
+    arrays = dict(stats)
+    for prefix, current in (("tree", True), ("roots", False)):
+        tok, pa, pb, nn = eng.get_trees(current=current)
+        used = np.arange(tok.shape[-1]) < nn[..., None]
+        arrays.update({prefix + "_tok": tok * used, prefix + "_a": pa * used, prefix + "_b": pb * used, prefix + "_nodes": nn})
+    arrays["chain_id"] = chain_offset + np.arange(eng.C)
+    per_chain = sum(8 * (a.size // eng.C) for a in arrays.values())
+    budget = DUMP_BYTES - 256 * len(arrays)                       # (npy headers)
+    idx = np.arange(eng.C)
+    if eng.C * per_chain > budget:
+        idx = np.sort(np.random.default_rng(0).choice(eng.C, budget // per_chain, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a)[idx].astype(np.float64))
+
+
+def measure(D, args, name, w, steps, warmup, full, dump_dir=None):
     """Device-timed steps + per-stage profile + e2e of one workload on the ranks of D.  `full`: also the roofline object and
-    the slower extras of the headline line."""
+    the slower extras of the headline line.  `dump_dir`: see dump_outputs."""
     import torch
     K, d = w["K"], w["d"]
     S = args.sweeps_per_step or w["sweeps"]
@@ -592,7 +616,10 @@ def measure(D, args, name, w, steps, warmup, full):
     n_launches = eng.launch_count() - l0
     clocks = sampler.result()
     ms_total = float(sum(a.elapsed_time(b) for a, b in evs))
-    c1 = eng.get_stats()["counters"].sum(axis=0)
+    stats = eng.get_stats()
+    c1 = stats["counters"].sum(axis=0)
+    if dump_dir and D.rank == 0:
+        dump_outputs(dump_dir, eng, stats, lo)
     dc = c1 - c0
     ms_max = D.vmax(ms_total)
     props, ev_ref, ev_exec, accepts, rank_rej, fp64_sw, cap_rej = D.vsum([dc[0], dc[5], dc[6], dc[1], dc[2], dc[4], dc[3]])
@@ -758,7 +785,7 @@ def run_ours(args, name, w):
     import __graft_entry__ as g
     g.build()
     D = Dist()
-    main = measure(D, args, name, w, args.steps, args.warmup, True)
+    main = measure(D, args, name, w, args.steps, args.warmup, True, dump_dir=args.dump_outputs)
     row_sharded = bool(w.get("row_sharded"))
     line = dict(metric="mh_proposals_per_sec", value=main["value"], unit="proposals/s", n_gpus=D.world, steps=args.steps, warmup=args.warmup,
                 ms_per_step=main["ms_per_step"], higher_is_better=True, scaling="strong" if w.get("strong") else "weak", vs_baseline=None,
@@ -839,7 +866,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip from_init, fit_e2e and the short runs of the other workloads")
     ap.add_argument("--extra-workloads", default="c4,c5,c3", help="other BASELINE configs measured briefly after the headline workload")
     ap.add_argument("--groups", type=int, default=0, help="chain groups pipelined on separate streams (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step left for the caller (stats, trees of rank 0's chains) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, args.workload, w)

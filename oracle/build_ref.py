@@ -22,7 +22,6 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_ROOT = os.environ.get("BSR_REFERENCE_ROOT", "/root/reference")
-DEST = os.path.join(HERE, "_ref", "bsr")
 FILES = ("__init__.py", "funcs.py", "bsr_class.py")
 
 
@@ -33,16 +32,18 @@ def sha256(path):
     return h.hexdigest()
 
 
-def build(verbose=True):
-    """Returns the manifest dict, or None when neither the reference nor an earlier copy is available."""
-    src = os.path.join(REF_ROOT, "codes")
-    manifest_path = os.path.join(HERE, "_ref", "MANIFEST.json")
+def build(verbose=True, ref_root=REF_ROOT, ref_dir=os.path.join(HERE, "_ref")):
+    """Copies <ref_root>/codes into <ref_dir>/bsr.  Returns the manifest dict, or None when neither the reference nor an
+    earlier copy is available."""
+    src = os.path.join(ref_root, "codes")
+    dest = os.path.join(ref_dir, "bsr")
+    manifest_path = os.path.join(ref_dir, "MANIFEST.json")
     if os.path.isdir(src):
-        os.makedirs(DEST, exist_ok=True)
+        os.makedirs(dest, exist_ok=True)
         man = dict(source=src, files={})
         for f in FILES:
-            shutil.copyfile(os.path.join(src, f), os.path.join(DEST, f))
-            man["files"][f] = sha256(os.path.join(DEST, f))
+            shutil.copyfile(os.path.join(src, f), os.path.join(dest, f))
+            man["files"][f] = sha256(os.path.join(dest, f))
         with open(manifest_path, "w") as fh:
             json.dump(man, fh, indent=1)
         if verbose:
@@ -52,8 +53,8 @@ def build(verbose=True):
         with open(manifest_path) as fh:
             man = json.load(fh)
         for f, digest in man["files"].items():
-            if sha256(os.path.join(DEST, f)) != digest:
-                raise RuntimeError("oracle/_ref/bsr/%s does not match its manifest" % f)
+            if sha256(os.path.join(dest, f)) != digest:
+                raise RuntimeError("%s does not match its manifest" % os.path.join(dest, f))
         return man
     return None
 

@@ -12,13 +12,13 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REF_DIR = os.path.join(HERE, "_ref")
 
 
-def available():
-    return os.path.exists(os.path.join(REF_DIR, "bsr", "funcs.py"))
+def available(ref_dir=REF_DIR):
+    return os.path.exists(os.path.join(ref_dir, "bsr", "funcs.py"))
 
 
-def load():
+def load(ref_dir=REF_DIR):
     """Returns the reference package (``bsr``: BSR, newProp, grow, allcal, ... as codes/__init__.py exports them)."""
-    if not available():
+    if not available(ref_dir):
         raise RuntimeError("oracle/_ref is empty: run `python oracle/build_ref.py` where /root/reference exists")
     try:
         import matplotlib.pyplot  # noqa: F401
@@ -28,9 +28,9 @@ def load():
         mpl.pyplot = plt
         sys.modules["matplotlib"] = mpl
         sys.modules["matplotlib.pyplot"] = plt
-    if REF_DIR not in sys.path:
-        sys.path.insert(0, REF_DIR)
+    if ref_dir not in sys.path:
+        sys.path.insert(0, ref_dir)
     import bsr
-    if not os.path.abspath(bsr.__file__).startswith(REF_DIR):
+    if not os.path.abspath(bsr.__file__).startswith(ref_dir):
         raise RuntimeError("another package named `bsr` shadows oracle/_ref: %s" % bsr.__file__)
     return bsr

@@ -1,8 +1,10 @@
 import gzip
 import json
+import lzma
 import os
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,7 +37,13 @@ def pytest_collection_modifyitems(config, items):
 
 def load_golden(name):
     with gzip.open(os.path.join(GOLDEN, name), "rt") as f:
-        return json.load(f)
+        g = json.load(f)
+    if "tape_file" in g:
+        # a long RNG tape is kept beside the fixture as xz-compressed little-endian float64: as JSON text it would make the
+        # fixture larger than 1 MB
+        with lzma.open(os.path.join(GOLDEN, g.pop("tape_file"))) as f:
+            g["tape"] = np.frombuffer(f.read(), dtype="<f8").tolist()
+    return g
 
 
 @pytest.fixture(scope="session")

@@ -15,6 +15,7 @@ The reference arithmetic is untouched; only np.random.* / scipy rvs are wrapped 
 import builtins
 import gzip
 import json
+import lzma
 import os
 import sys
 
@@ -163,6 +164,11 @@ def dump(obj, fname):
         json.dump(obj, f, separators=(",", ":"))
 
 
+def dump_tape(tape, fname):
+    with lzma.open(os.path.join(HERE, fname), "wb", preset=9 | lzma.PRESET_EXTREME) as f:
+        f.write(np.asarray(tape, dtype="<f8").tobytes())
+
+
 if __name__ == "__main__":
     gen_steps("f1_d2_k3", "f1", n=64, d=2, K=3, beta=-1, n_chains=24, n_steps=60, seed=11)
     gen_steps("mix_d8_k5", "mix", n=48, d=8, K=5, beta=-1, n_chains=12, n_steps=60, seed=12)
@@ -194,8 +200,10 @@ def gen_plateau():
         print("plateau probe seed", seed, "accepts", len(e), "draws", len(rec.tape), "fired", fired, flush=True)
         if fired and len(rec.tape) < 600000:
             Xt = rng.uniform(-3, 3, (9, 2))
+            # the 138 k-draw tape goes beside the fixture in binary (tests/conftest.py:load_golden): as JSON text it passes 1 MB
+            dump_tape(rec.tape, "fits_plateau.tape.f64.xz")
             out = dict(name="plateau", kind="noise", n=6, d=2, K=2, MM=1, val=2500, beta=-1, seed=seed, X=X.tolist(), y=y.tolist(),
-                       Xtest=Xt.tolist(), tape=rec.tape, roots=[[encode(r) for r in rs] for rs in est.roots_],
+                       Xtest=Xt.tolist(), tape_file="fits_plateau.tape.f64.xz", roots=[[encode(r) for r in rs] for rs in est.roots_],
                        betas=[np.asarray(b).ravel().tolist() for b in est.betas_],
                        train_err=[[float(v) for v in el] for el in est.train_err_], model=est.model(), model_first=est.model(last_ind=1),
                        complexity=int(est.complexity()), predict=est.predict(Xt).ravel().tolist(), predict_train=est.predict(X).ravel().tolist())
