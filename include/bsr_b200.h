@@ -97,15 +97,32 @@ int bsr_destroy(bsr_handle* h);
  * exactly as a numpy array / DataFrame.values; the library builds its own column-major fp32 (+fp64) copies.
  * n_total is the global row count when rows are sharded (n_total == n otherwise). */
 int bsr_set_data_host(bsr_handle* h, const double* X_rowmajor, const double* y, int64_t n, int32_t d, int64_t n_total);
-/* Same, from device memory: fp32 column-major X (leading dimension ld >= n) and fp32 y, used in place. */
+/* Same, from device memory: fp32 column-major X (leading dimension ld >= n) and fp32 y, used in place.
+ * Both leave the handle with one data set, every chain on it. */
 int bsr_set_data_device(bsr_handle* h, const float* X_colmajor, const float* y, int64_t n, int32_t d, int64_t ld,
                         int64_t n_total);
+/* n_datasets data sets of the same shape in one handle: X row-major [n_datasets][n][d], y [n_datasets][n]; chain c fits data set
+ * chain_dataset[c] (each in [0, n_datasets); n_datasets * d * n below 2^32 elements).  Chains never interact, so with chains keyed as
+ * a handle of one data set would key them (bsr_init_chains_keyed), the chains of data set b end exactly -- bit for bit -- where that
+ * handle's chains end, whenever both handles have the same window geometry (bsr_get_window_geometry).  They do for n < 16384 rows
+ * (one row split, same tile); with more rows and few chains the split count depends on the chain count, and the results then agree
+ * up to the fp64 summation order of the splits.  Several data sets run on the window path of bsr_run only: the proposal-by-proposal
+ * pipeline (bsr_set_pipeline), the phase API (bsr_sweep_*), bsr_peer_export / bsr_peer_import and bsr_eval_trees refuse them.
+ * Row-sharded handles (a slice of one data set, with its global row count) refuse this call; they use bsr_set_data_*.  A failed
+ * call leaves the handle without data.  Lets one run fit a replication study, bootstrap refits or several targets on the same
+ * features. */
+int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, int64_t n, int32_t d,
+                          const int32_t* chain_dataset);
 
 /* Prior initialisation of every chain: sigma ~ IG(1), per tree sigma_a, sigma_b ~ IG(1) and grow()
  * (codes/bsr_class.py:123-142, codes/funcs.py:74-119), then the initial intercept OLS (bsr_class.py:147-163). */
+/* Every chain draws from Philox under its own key (seed, id): bsr_init_chains keys chain c with (seed, chain_offset + c),
+ * bsr_init_chains_keyed with (seeds[c], ids[c]) (host arrays [n_chains] each). */
 int bsr_init_chains(bsr_handle* h, uint64_t seed);
+int bsr_init_chains_keyed(bsr_handle* h, const uint64_t* seeds, const int64_t* ids);
 /* Load an explicit state instead (host arrays; tok/pa/pb are [n_chains][K][BSR_MAX_NODES], nn/sa/sb are
- * [n_chains][K], sigma is [n_chains]) and compute the initial fit.  Used for replaying reference states. */
+ * [n_chains][K], sigma is [n_chains]) and compute the initial fit; the chains are keyed as by bsr_init_chains(h, seed).
+ * Used for replaying reference states. */
 int bsr_set_state(bsr_handle* h, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
                   const double* sigma, const double* sa, const double* sb, uint64_t seed);
 
@@ -145,7 +162,7 @@ int bsr_sweep_resolve(bsr_handle* h, void* stream);
 /* Device buffer holding, per chain, the partial sums (to SUM-allreduce) followed by the partial max-abs values
  * (to MAX-allreduce): [n_chains][n_sum] doubles then [n_chains][n_max] doubles. */
 int bsr_gram_buffer(bsr_handle* h, void** device_ptr, int64_t* n_sum_per_chain, int64_t* n_max_per_chain);
-/* Row-sharded mode only.  sum(y), y'y are computed over the local rows by bsr_set_data_*; the caller all-reduces
+/* Row-sharded mode only (one data set).  sum(y), y'y are computed over the local rows by bsr_set_data_*; the caller all-reduces
  * them and writes the global values back.  bsr_init_chains / bsr_set_state then leave the initial Gram partials in
  * bsr_gram_buffer; after all-reducing them the caller completes the initial fit with bsr_finish_init. */
 int bsr_get_y_stats(bsr_handle* h, double* sum_y, double* yy);

@@ -69,9 +69,7 @@ class BSR(BaseEstimator, RegressorMixin):
         if X.shape[0] != y.shape[0]:
             raise ValueError("train_data and train_y disagree on the number of rows")
         MM, K = int(self.itrNum), int(self.treeNum)
-        ops = list(self.ops) if self.ops is not None else list(DEFAULT_OPS)
-        opcodes = [NAME_OP[o] if isinstance(o, str) else int(o) for o in ops]
-        w = list(self.op_weights) if self.op_weights is not None else [1.0 / len(ops)] * len(ops)
+        opcodes, w = self._op_tables()
         seed = self.seed
         if seed is None:          # the reference draws from the global numpy state; so does the default seed
             seed = int(np.random.randint(0, 2 ** 31 - 1))
@@ -111,6 +109,64 @@ class BSR(BaseEstimator, RegressorMixin):
             c = res["counters"]
             print("chains: %d  proposals: %d  accepts: %d  rank-rejects: %d" % (MM, c[:, 0].sum(), c[:, 1].sum(), c[:, 2].sum()))
         return
+
+    def fit_many(self, datasets, seeds=None):
+        """Fit this estimator to each of several data sets in one GPU run; returns one fitted ``BSR`` per data set.
+
+        ``datasets``: a sequence of (X, y) pairs of the same shape (n rows, d features).  The ``itrNum`` restarts of every data
+        set run as chains of one handle (chains never interact), so the B fits share one upload, one sequence of launches
+        and one result read.  Estimator b is identical -- ``roots_`` / ``model()``, ``betas_``, ``train_err_``,
+        ``train_err_truncated_``, ``counters_``, ``done_``, ``final_rmse_`` and every ``predict*`` -- to
+        ``clone(self).set_params(seed=seeds[b]).fit(*datasets[b])``: its chains draw from Philox under the keys
+        (seeds[b], 0 ... itrNum - 1) that fit gives them.  This holds whenever the window geometry of the batch equals that of
+        a single fit, which it always does below 16384 rows; above, with few chains, the row-split count depends on the chain
+        count and the results agree up to the fp64 summation order of the splits.  ``n_sweeps_`` reports the sweeps of the
+        whole batch (the stop rules are checked for all chains together), not the count a single fit would have needed.
+
+        ``seeds``: one seed per data set; None gives every data set ``self.seed``, or, when that is None, draws one seed per
+        data set from numpy's global state, in order, exactly as a loop of ``fit`` calls would.  The returned estimators
+        carry the parameters of ``self``."""
+        data = [(_as_matrix(X), np.asarray(y, dtype=np.float64).ravel()) for X, y in datasets]
+        check_datasets(data)
+        B = len(data)
+        seeds = dataset_seeds(self.seed, B, seeds)
+        MM, K = int(self.itrNum), int(self.treeNum)
+        opcodes, w = self._op_tables()
+        dist = parallel.context(self.distributed)
+        seeds = [dist.broadcast_int(s) for s in seeds]
+        lo, hi = parallel.shard_range(B * MM, dist.rank, dist.world)
+        fixed = self.fixed_sweeps is not None
+        res = None
+        if hi > lo:
+            eng = capi.Engine(K, hi - lo, opcodes, w, beta=float(self.beta), val=(0 if fixed else int(self.val)),
+                              plateau_rule=(self.plateau_rule and not fixed), precision=self.precision,
+                              err_cap=int(self.err_cap), device=self._device_index(), chain_offset=lo)
+            try:
+                g = np.arange(lo, hi)
+                ds, ids = g // MM, g % MM
+                eng.set_datasets(np.stack([X for X, _ in data]), np.stack([y for _, y in data]), ds)
+                eng.init_chains_keyed(np.asarray(seeds, dtype=object)[ds], ids)
+                if fixed:
+                    eng.run(int(self.fixed_sweeps))
+                    sweeps = int(self.fixed_sweeps)
+                else:
+                    sweeps = eng.run_until_done(int(self.max_sweeps), check_every=32)
+                res = parallel.collect(eng)
+                res["sweeps"] = sweeps
+            finally:
+                eng.close()
+        res = dist.gather_results(res, B * MM, K)
+        fits = []
+        for part in parallel.split_results(res, B, MM):
+            est = type(self)(**self.get_params())
+            est._set_results(part)
+            fits.append(est)
+        open_sets = [b for b, est in enumerate(fits) if not np.all(est.done_)]
+        if open_sets and not fixed:
+            import warnings
+            warnings.warn("BSR.fit_many: data sets %s have restarts that had not met their stop rule after max_sweeps = %d sweeps; "
+                          "their roots_ / betas_ hold the current states (see done_)" % (open_sets, int(self.max_sweeps)), RuntimeWarning)
+        return fits
 
     # ---- beyond the reference: what a batch of restarts allows (SURVEY.md 8f 1, 3) ----------------------
     def best_chain(self):
@@ -155,6 +211,12 @@ class BSR(BaseEstimator, RegressorMixin):
         return out
 
     # ---- helpers ------------------------------------------------------------------------------------
+    def _op_tables(self):
+        ops = list(self.ops) if self.ops is not None else list(DEFAULT_OPS)
+        opcodes = [NAME_OP[o] if isinstance(o, str) else int(o) for o in ops]
+        w = list(self.op_weights) if self.op_weights is not None else [1.0 / len(ops)] * len(ops)
+        return opcodes, w
+
     def _device_index(self):
         if self.device is not None:
             return int(self.device)
@@ -230,6 +292,32 @@ class _LazyRoots:
 
     def __getstate__(self):
         return dict(_pk=self._pk, _cache={})
+
+
+def check_datasets(data):
+    """``fit_many``'s data sets, as (X (n, d), y) pairs, must share n and d, and each X must agree with its y: else ValueError."""
+    if len(data) == 0:
+        raise ValueError("fit_many: no data sets")
+    n, d = data[0][0].shape
+    for b, (X, y) in enumerate(data):
+        if X.shape[0] != y.shape[0]:
+            raise ValueError("fit_many: data set %d: train_data and train_y disagree on the number of rows" % b)
+        if X.shape != (n, d):
+            raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape"
+                             % (b, X.shape[0], X.shape[1], n, d))
+
+
+def dataset_seeds(seed, n_datasets, seeds=None):
+    """One seed per data set of ``fit_many``: ``seeds`` as given, else ``seed`` for all, else (seed None) one draw per data set from
+    numpy's global state -- the draws a loop of ``fit`` calls would make, in the same order."""
+    if seeds is not None:
+        seeds = [int(s) for s in seeds]
+        if len(seeds) != n_datasets:
+            raise ValueError("fit_many: %d seeds for %d data sets" % (len(seeds), n_datasets))
+        return seeds
+    if seed is not None:
+        return [int(seed)] * n_datasets
+    return [int(np.random.randint(0, 2 ** 31 - 1)) for _ in range(n_datasets)]
 
 
 def _as_matrix(data):

@@ -33,7 +33,9 @@ _SIGS = {
     "bsr_destroy": (C.c_int, [_P]),
     "bsr_set_data_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int64]),
     "bsr_set_data_device": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int64, C.c_int64]),
+    "bsr_set_datasets_host": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, C.c_int32, _P]),
     "bsr_init_chains": (C.c_int, [_P, C.c_uint64]),
+    "bsr_init_chains_keyed": (C.c_int, [_P, _P, _P]),
     "bsr_set_state": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_uint64]),
     "bsr_run": (C.c_int, [_P, C.c_int32, _P]),
     "bsr_get_launch_count": (C.c_int, [_P, C.POINTER(C.c_int64)]),
@@ -254,6 +256,18 @@ class Engine:
         self.n, self.d = X.shape
         _ck(self._lib.bsr_set_data_host(self._h, _ptr(X), _ptr(y), self.n, self.d, int(n_total)))
 
+    def set_datasets(self, X, y, chain_dataset):
+        """D data sets of the same shape: X (D, n, d), y (D, n); chain c fits data set ``chain_dataset[c]``."""
+        X = np.ascontiguousarray(X, dtype=np.float64)
+        y = np.ascontiguousarray(y, dtype=np.float64)
+        if X.ndim != 3 or y.ndim != 2 or X.shape[:2] != y.shape:
+            raise ValueError("X must be (D, n, d) and y (D, n)")
+        cd = np.ascontiguousarray(chain_dataset, dtype=np.int32).ravel()
+        if cd.size != self.C:
+            raise ValueError("chain_dataset must hold one data set index per chain")
+        _ck(self._lib.bsr_set_datasets_host(self._h, X.shape[0], _ptr(X), _ptr(y), X.shape[1], X.shape[2], _ptr(cd)))
+        self.n, self.d = X.shape[1], X.shape[2]
+
     def set_data_device(self, x_ptr, y_ptr, n, d, ld, n_total=0):
         self.n, self.d = int(n), int(d)
         _ck(self._lib.bsr_set_data_device(self._h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), int(n), int(d), int(ld), int(n_total)))
@@ -261,6 +275,14 @@ class Engine:
     # ---- state ------------------------------------------------------------------------------------
     def init_chains(self, seed):
         _ck(self._lib.bsr_init_chains(self._h, C.c_uint64(int(seed) & (2 ** 64 - 1))))
+
+    def init_chains_keyed(self, seeds, ids):
+        """Prior initialisation with chain c drawing from Philox under the key (seeds[c], ids[c])."""
+        seeds = np.array([int(v) & (2 ** 64 - 1) for v in np.ravel(seeds)], dtype=np.uint64)
+        ids = np.ascontiguousarray(ids, dtype=np.int64).ravel()
+        if seeds.size != self.C or ids.size != self.C:
+            raise ValueError("seeds and ids must hold one entry per chain")
+        _ck(self._lib.bsr_init_chains_keyed(self._h, _ptr(seeds), _ptr(ids)))
 
     def set_state(self, tok, pa, pb, nn, sigma, sa, sb, seed=0):
         CK = self.C * self.K

@@ -90,12 +90,15 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
   rc |= dalloc(h, &st.pinfo, CK_);
   rc |= dalloc(h, &st.lfs, 2 * CK_);
   rc |= dalloc(h, &st.lcnt, CK_);
+  rc |= dalloc(h, &st.key_seed, (size_t)C);
+  rc |= dalloc(h, &st.key_id, (size_t)C);
+  rc |= dalloc(h, &st.ds, (size_t)C);
   const int P = 2 * K;
   rc |= dalloc(h, &h->gram, (size_t)2 * C * (gram_n_sum(P) + P));   // [sums | maxs | per-chain scratch records]
   rc |= dalloc(h, &h->need64, (size_t)C);
   rc |= dalloc(h, &h->split_cnt, (size_t)C);
   rc |= dalloc(h, &h->d_count, 2);      // [1]: abort flag of the peer-memory exchange (k_wwait)
-  rc |= dalloc(h, &h->d_ystats, 2);
+  rc |= dalloc(h, &h->ystats, 2);
   if (rc) { bsr_destroy(h); return 1; }
   for (int i = 0; i < 8; ++i) cudaEventCreate(&h->ev[i]);
   if (const char* e = getenv("BSR_SEQ_PIPELINE")) h->seq_pipeline = atoi(e) != 0;
@@ -175,10 +178,10 @@ static int setup_col_cache(bsr_handle* h) {
 static int finish_data(bsr_handle* h) {
   if (setup_col_cache(h)) return 1;
   if (h->initialised) h->needs_refit = true;
-  // y statistics over the local rows; in row-sharded mode the caller replaces them with the global values
-  k_y_stats<<<1, 1024>>>(h->y64, h->n, h->d_ystats);
+  // y statistics over the local rows of every data set; in row-sharded mode the caller replaces them with the global values
+  k_y_stats<<<h->n_ds, 1024>>>(h->y64, h->n, h->ld, h->ystats);
   double s[2];
-  CK(cudaMemcpy(s, h->d_ystats, sizeof s, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(s, h->ystats, sizeof s, cudaMemcpyDeviceToHost));
   h->sum_y = s[0]; h->yy = s[1];
   return build_tables(h);
 }
@@ -189,33 +192,83 @@ static void free_data(bsr_handle* h) {
   h->X32 = nullptr; h->y32 = nullptr; h->X64 = nullptr; h->y64 = nullptr;
 }
 
-int bsr_set_data_host(bsr_handle* h, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
-  if (!h || !X || !y) return fail("bsr_set_data_host: null argument");
-  if (n < 1 || d < 1 || d > 65535) return fail("bsr_set_data_host: need n >= 1 and 1 <= d <= 65535");
-  if ((n + 3) / 4 * 4 * (int64_t)d >= (int64_t)1 << 32) return fail("bsr_set_data_host: d * n must stay below 2^32 elements per device (shard the rows)");
-  CK(cudaSetDevice(h->cfg.device));
-  const bool same_shape = h->own_x32 && h->X32 != nullptr && h->n == n && h->d == d;
+// Number of data sets and the data set of every chain (nullptr: all chains on data set 0), committed once the data of the D data
+// sets is in place.  On failure the caller drops the data (free_data): no entry point then runs on chains that name data sets the
+// handle does not hold.
+static int set_chain_datasets(bsr_handle* h, int D, const int32_t* chain_dataset) {
+  if (D != h->n_ds) {
+    double* ys = nullptr;
+    if (dalloc(h, &ys, 2 * (size_t)D)) return 1;
+    dfree(h, h->ystats);
+    h->ystats = ys;
+    h->n_ds = D;
+  }
+  if (chain_dataset) CK(cudaMemcpy(h->st.ds, chain_dataset, (size_t)h->st.C * sizeof(int), cudaMemcpyHostToDevice));
+  else CK(cudaMemset(h->st.ds, 0, (size_t)h->st.C * sizeof(int)));
+  return 0;
+}
+
+// D data sets of n rows x d features from host memory (X row-major [D][n][d], y [D][n]) into the handle's buffers.
+static int upload_host(bsr_handle* h, int D, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
+  const bool same_shape = h->own_x32 && h->X32 != nullptr && h->n == n && h->d == d && h->n_ds == D;
+  const size_t ld = (size_t)(n + 3) / 4 * 4;
   if (!same_shape) {
     CK(cudaDeviceSynchronize());
     free_data(h);
-    h->n = n; h->d = d; h->ld = (n + 3) / 4 * 4;
+    h->n = n; h->d = d; h->ld = (int64_t)ld;
     h->own_x32 = true;
-    if (dalloc(h, &h->X32, (size_t)h->ld * d) || dalloc(h, &h->X64, (size_t)h->ld * d) || dalloc(h, &h->y32, (size_t)h->ld) ||
-        dalloc(h, &h->y64, (size_t)h->ld)) return 1;
+    if (dalloc(h, &h->X32, D * ld * d) || dalloc(h, &h->X64, D * ld * d) || dalloc(h, &h->y32, D * ld) || dalloc(h, &h->y64, D * ld)) return 1;
     if (h->stage) cudaFree(h->stage);
     h->stage = nullptr;
-    CK(cudaMalloc((void**)&h->stage, (size_t)n * d * sizeof(double)));
+    CK(cudaMalloc((void**)&h->stage, (size_t)D * n * d * sizeof(double)));
   }
   h->n_total = n_total > 0 ? n_total : n;
   // stream-ordered after any sweep still in flight on the default stream; the copies from pageable memory are synchronous
-  CK(cudaMemcpy(h->stage, X, (size_t)n * d * sizeof(double), cudaMemcpyHostToDevice));
-  int blocks = (int)std::min<int64_t>(((int64_t)n * d + 255) / 256, 148 * 16);
+  CK(cudaMemcpy(h->stage, X, (size_t)D * n * d * sizeof(double), cudaMemcpyHostToDevice));
+  const dim3 blocks((unsigned)std::min<int64_t>(((int64_t)n * d + 255) / 256, 148 * 16), (unsigned)D);
   k_transpose_in<float><<<blocks, 256>>>(h->stage, h->X32, n, d, h->ld);
   k_transpose_in<double><<<blocks, 256>>>(h->stage, h->X64, n, d, h->ld);
-  CK(cudaMemcpy(h->y64, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice));
-  k_convert<double, float><<<blocks, 256>>>(h->y64, h->y32, n);
+  // y [D][n] -> [D][ld]: the padding rows stay the zeros of the allocation
+  CK(cudaMemcpy2D(h->y64, ld * sizeof(double), y, (size_t)n * sizeof(double), (size_t)n * sizeof(double), (size_t)D, cudaMemcpyHostToDevice));
+  k_convert<double, float><<<blocks.x, 256>>>(h->y64, h->y32, (int64_t)(D * ld));
   CK(cudaGetLastError());
+  return 0;
+}
+
+static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total,
+                         const int32_t* chain_dataset) {
+  const std::string f(fn);
+  if (n < 1 || d < 1 || d > 65535) return fail(f + ": need n >= 1 and 1 <= d <= 65535");
+  if ((n + 3) / 4 * 4 * (int64_t)d * D >= (int64_t)1 << 32)
+    return fail(f + ": n_datasets * d * n must stay below 2^32 elements per device (shard the rows, or fit fewer data sets per handle)");
+  CK(cudaSetDevice(h->cfg.device));
+  if (upload_host(h, D, X, y, n, d, n_total) || set_chain_datasets(h, D, chain_dataset)) {
+    free_data(h);
+    return 1;
+  }
   return finish_data(h);
+}
+
+int bsr_set_data_host(bsr_handle* h, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
+  if (!h || !X || !y) return fail("bsr_set_data_host: null argument");
+  return set_data_host(h, "bsr_set_data_host", 1, X, y, n, d, n_total, nullptr);
+}
+
+int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X, const double* y, int64_t n, int32_t d,
+                          const int32_t* chain_dataset) {
+  if (!h || !X || !y || !chain_dataset) return fail("bsr_set_datasets_host: null argument");
+  if (n_datasets < 1 || n_datasets > 65535) return fail("bsr_set_datasets_host: n_datasets must be in [1, 65535]");
+  for (int c = 0; c < h->st.C; ++c)
+    if (chain_dataset[c] < 0 || chain_dataset[c] >= n_datasets) {
+      char msg[160];
+      snprintf(msg, sizeof msg, "bsr_set_datasets_host: chain_dataset[%d] = %d is outside [0, %d)", c, (int)chain_dataset[c], (int)n_datasets);
+      return fail(msg);
+    }
+  // (a row-sharded handle holds a slice of the rows of one data set: bsr_set_data_* with the global row count)
+  if (h->cfg.row_sharded) return fail("bsr_set_datasets_host: not available on row-sharded handles (use bsr_set_data_host)");
+  if (n_datasets > 1 && h->seq_pipeline)
+    return fail("bsr_set_datasets_host: several data sets need the window path of bsr_run (this handle uses the proposal-by-proposal pipeline)");
+  return set_data_host(h, "bsr_set_datasets_host", n_datasets, X, y, n, d, 0, chain_dataset);
 }
 
 int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n, int32_t d, int64_t ld, int64_t n_total) {
@@ -229,17 +282,38 @@ int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n
   h->n = n; h->d = d; h->ld = ld; h->n_total = n_total > 0 ? n_total : n;
   h->own_x32 = false;
   h->X32 = const_cast<float*>(X); h->y32 = const_cast<float*>(y);
-  if (dalloc(h, &h->X64, (size_t)ld * d) || dalloc(h, &h->y64, (size_t)ld)) return 1;
-  int blocks = 148 * 16;
-  k_convert<float, double><<<blocks, 256>>>(X, h->X64, ld * (int64_t)d);
-  k_convert<float, double><<<blocks, 256>>>(y, h->y64, n);
-  CK(cudaDeviceSynchronize());
+  auto upload = [&]() -> int {
+    if (dalloc(h, &h->X64, (size_t)ld * d) || dalloc(h, &h->y64, (size_t)ld)) return 1;
+    int blocks = 148 * 16;
+    k_convert<float, double><<<blocks, 256>>>(X, h->X64, ld * (int64_t)d);
+    k_convert<float, double><<<blocks, 256>>>(y, h->y64, n);
+    CK(cudaDeviceSynchronize());
+    return 0;
+  };
+  if (upload() || set_chain_datasets(h, 1, nullptr)) {
+    free_data(h);
+    return 1;
+  }
   return finish_data(h);
 }
 
-// global sum(y), y'y for row-sharded runs (the caller all-reduces the local values)
-int bsr_get_y_stats(bsr_handle* h, double* sum_y, double* yy) { *sum_y = h->sum_y; *yy = h->yy; return 0; }
-int bsr_set_y_stats(bsr_handle* h, double sum_y, double yy) { h->sum_y = sum_y; h->yy = yy; return 0; }
+// global sum(y), y'y for row-sharded runs (the caller all-reduces the local values): entry 0 of the data sets' statistics
+int bsr_get_y_stats(bsr_handle* h, double* sum_y, double* yy) {
+  if (!h || !sum_y || !yy) return fail("bsr_get_y_stats: null argument");
+  CK(cudaSetDevice(h->cfg.device));
+  double s[2];
+  CK(cudaMemcpy(s, h->ystats, sizeof s, cudaMemcpyDeviceToHost));
+  *sum_y = s[0]; *yy = s[1];
+  return 0;
+}
+int bsr_set_y_stats(bsr_handle* h, double sum_y, double yy) {
+  if (!h) return fail("bsr_set_y_stats: null handle");
+  CK(cudaSetDevice(h->cfg.device));
+  const double s[2] = {sum_y, yy};
+  CK(cudaMemcpy(h->ystats, s, sizeof s, cudaMemcpyHostToDevice));
+  h->sum_y = sum_y; h->yy = yy;
+  return 0;
+}
 
 }  // extern "C"
 
@@ -264,22 +338,28 @@ static int check_ready(bsr_handle* h) {
   return 0;
 }
 
+// the proposal-by-proposal pipeline and the phase API read one data set
+static int check_one_dataset(bsr_handle* h, const char* fn) {
+  if (h->n_ds > 1) return fail(std::string(fn) + ": not available on a handle with several data sets (bsr_set_datasets_host); use bsr_run");
+  return 0;
+}
+
 extern "C" {
 
 int bsr_sweep_propose(bsr_handle* h, void* stream) {
-  if (check_ready(h)) return 1;
+  if (check_ready(h) || check_one_dataset(h, "bsr_sweep_propose")) return 1;
   if (h->tape_mode && h->tape_pos >= h->tape_steps)
     return fail("tape exhausted: call bsr_set_tape again (or with NULL to return to Philox)");
   return bsr_launch_propose(h, (cudaStream_t)stream, 0, h->cfg.n_chains);
 }
 
 int bsr_sweep_eval(bsr_handle* h, void* stream) {
-  if (check_ready(h)) return 1;
+  if (check_ready(h) || check_one_dataset(h, "bsr_sweep_eval")) return 1;
   return launch_eval(h, (cudaStream_t)stream, 0);
 }
 
 int bsr_sweep_resolve(bsr_handle* h, void* stream) {
-  if (check_ready(h)) return 1;
+  if (check_ready(h) || check_one_dataset(h, "bsr_sweep_resolve")) return 1;
   if (bsr_launch_resolve(h, (cudaStream_t)stream, 0, 0, h->cfg.n_chains)) return 1;
   h->sg_dirty = true;     // an accept here rewrites the live Gram from the sweep kernels' values: a later bsr_run refits first
   h->sweep += 1;
@@ -336,11 +416,23 @@ static int reset_run_state(bsr_handle* h) {
   return 0;
 }
 
-int bsr_init_chains(bsr_handle* h, uint64_t seed) {
-  if (!h) return fail("null handle");
+// Philox keys of the chains: explicit (seeds, ids), or (seed, chain_offset + c)
+static int upload_keys(bsr_handle* h, const uint64_t* seeds, const int64_t* ids) {
+  CK(cudaMemcpy(h->st.key_seed, seeds, (size_t)h->st.C * sizeof(uint64_t), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(h->st.key_id, ids, (size_t)h->st.C * sizeof(int64_t), cudaMemcpyHostToDevice));
+  return 0;
+}
+static void handle_keys(const bsr_handle* h, uint64_t seed, std::vector<uint64_t>& seeds, std::vector<int64_t>& ids) {
+  seeds.assign((size_t)h->st.C, seed);
+  ids.resize((size_t)h->st.C);
+  for (int c = 0; c < h->st.C; ++c) ids[(size_t)c] = h->cfg.chain_offset + c;
+}
+
+int bsr_init_chains_keyed(bsr_handle* h, const uint64_t* seeds, const int64_t* ids) {
+  if (!h || !seeds || !ids) return fail("bsr_init_chains_keyed: null argument");
   if (!h->X32) return fail("no data: call bsr_set_data_* first");
   CK(cudaSetDevice(h->cfg.device));
-  h->seed = seed;
+  if (upload_keys(h, seeds, ids)) return 1;
   if (reset_run_state(h)) return 1;
   if (bsr_launch_init_chains(h, 0)) return 1;
   h->initialised = true;
@@ -348,13 +440,23 @@ int bsr_init_chains(bsr_handle* h, uint64_t seed) {
   return initial_fit(h);
 }
 
+int bsr_init_chains(bsr_handle* h, uint64_t seed) {
+  if (!h) return fail("null handle");
+  std::vector<uint64_t> seeds;
+  std::vector<int64_t> ids;
+  handle_keys(h, seed, seeds, ids);
+  return bsr_init_chains_keyed(h, seeds.data(), ids.data());
+}
+
 int bsr_set_state(bsr_handle* h, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
                   const double* sigma, const double* sa, const double* sb, uint64_t seed) {
   if (!h) return fail("null handle");
   if (!h->X32) return fail("no data: call bsr_set_data_* first");
   CK(cudaSetDevice(h->cfg.device));
-  h->seed = seed;
-  if (reset_run_state(h)) return 1;
+  std::vector<uint64_t> seeds;
+  std::vector<int64_t> ids;
+  handle_keys(h, seed, seeds, ids);
+  if (upload_keys(h, seeds.data(), ids.data()) || reset_run_state(h)) return 1;
   ChainState& st = h->st;
   const size_t CKn = (size_t)st.C * st.K;
   for (size_t g = 0; g < CKn; ++g)
@@ -469,6 +571,7 @@ int bsr_set_window(bsr_handle* h, int32_t window) {
 
 int bsr_set_pipeline(bsr_handle* h, int32_t sequential) {
   if (!h) return fail("null handle");
+  if (sequential && check_one_dataset(h, "bsr_set_pipeline")) return 1;
   if (h->X32) return fail("bsr_set_pipeline: call before bsr_set_data_*");
   h->seq_pipeline = sequential != 0;
   return 0;
@@ -838,6 +941,7 @@ int bsr_get_err_trace(bsr_handle* h, double* err) {
 int bsr_eval_trees(bsr_handle* h, int32_t n_trees, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
                    int32_t precision, double* out) {
   if (!h || !h->X32) return fail("bsr_eval_trees: no data");
+  if (check_one_dataset(h, "bsr_eval_trees")) return 1;
   CK(cudaSetDevice(h->cfg.device));
   uint32_t* d_tok; double *d_a, *d_b, *d_out; int* d_nn;
   const size_t TN = (size_t)n_trees * BSR_MAXN;

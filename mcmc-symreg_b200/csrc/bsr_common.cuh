@@ -91,6 +91,10 @@ struct ChainState {
   int* lcnt;          // [C][K] node count | lt nodes << 8 | terminals << 16 | detransform candidates << 24 (0: not computed)
   unsigned char* live_bad;   // [C][K] live column has values outside the fp32 range: the chain's sweeps run in fp64
   unsigned char* prop_bad;   // [C][K] same for the proposal of the current sweep
+  // Philox key of every chain (bsr_init_chains: the handle's seed and the chain's global id) and the data set it fits
+  uint64_t* key_seed; // [C]
+  int64_t* key_id;    // [C]
+  int* ds;            // [C]  index into the handle's data sets ([D][d][ld] X, [D][ld] y, [D][2] y statistics)
   int err_cap;
   int val;
   int plateau_rule;

@@ -11,17 +11,17 @@ struct bsr_handle {
   PriorTables* d_pt = nullptr;   // device copy (the kernels read the tables from global memory)
   ChainState st;
   std::vector<void*> allocs;
-  // data
+  // data: n_ds data sets of the same shape, X column-major [n_ds][d][ld], y [n_ds][ld]
   float* X32 = nullptr; double* X64 = nullptr; float* y32 = nullptr; double* y64 = nullptr;
+  int n_ds = 1;
   bool own_x32 = false;
-  double* stage = nullptr;       // device staging of the row-major host X (bsr_set_data_host)
+  double* stage = nullptr;       // device staging of the row-major host X (bsr_set_data_host / bsr_set_datasets_host)
   void* gt_dev = nullptr; void* gt_host = nullptr; size_t gt_bytes = 0;   // gather staging of bsr_get_trees (device, pinned host)
   void* pk_head = nullptr; size_t pk_head_bytes = 0;   // packed results (bsr_pack_trees): counts / offsets / node counts / scan scratch
   void* pk_body = nullptr; size_t pk_body_bytes = 0;   //                                   lt parameter pairs, then tokens
   long long pk_nodes = 0, pk_lt = 0;
   int64_t n = 0, ld = 0, n_total = 0;
   int d = 0;
-  double sum_y = 0, yy = 0;
   bool y_stats_external = false;
   // sweep buffers
   double* gram = nullptr;   // [C][n_sum] then [C][P]
@@ -30,8 +30,8 @@ struct bsr_handle {
   double* part = nullptr;        // row-split partial records
   size_t part_cap = 0;
   int* d_count = nullptr;
-  double* d_ystats = nullptr;
-  uint64_t seed = 0;
+  double* ystats = nullptr;      // [n_ds][2] sum(y), y'y of every data set (row-sharded handles: the global values, bsr_set_y_stats)
+  double sum_y = 0, yy = 0;      // entry 0 of ystats on the host: the window kernels of one data set take it by value
   int64_t sweep = 0;
   bool initialised = false;
   bool col_cache_wanted = false;

@@ -12,8 +12,6 @@
 #include "bsr_solve.cuh"
 
 struct ProposeCtx {
-  uint64_t seed;
-  int64_t chain_offset;
   int64_t sweep;
   const double* tape;
   const int64_t* tape_off;
@@ -25,13 +23,13 @@ struct ProposeCtx {
 };
 
 template <int MODE>
-__global__ void k_init_chains(ChainState st, const PriorTables* __restrict__ ptp, uint64_t seed, int64_t chain_offset) {
+__global__ void k_init_chains(ChainState st, const PriorTables* __restrict__ ptp) {
   const PriorTables& pt = *ptp;   // tables live in global memory: indexed divergently, and out-of-line callees take them by reference
   int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= st.C * st.K) return;
   int c = g / st.K, k = g % st.K;
   Draws<MODE> dr;
-  dr.init_philox(seed, (uint64_t)(chain_offset + c), (uint32_t)k, 0u);
+  dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)k, 0u);
   size_t slot = (size_t)g * BSR_MAXN;
   double sa, sb;
   init_tree<MODE>(pt, dr, st.tok[0] + slot, st.pa[0] + slot, st.pb[0] + slot, st.nn[0] + g, sa, sb);
@@ -40,7 +38,7 @@ __global__ void k_init_chains(ChainState st, const PriorTables* __restrict__ ptp
   st.nn[1][g] = 0;
   if (k == 0) {
     Draws<MODE> ds;
-    ds.init_philox(seed, (uint64_t)(chain_offset + c), (uint32_t)st.K, 0u);
+    ds.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)st.K, 0u);
     st.sigma[c] = ds.invgamma(1);                                             // bsr_class.py:123
   }
 }
@@ -54,7 +52,7 @@ __global__ void k_propose(ChainState st, const PriorTables* __restrict__ ptp, Pr
   int c = g / st.K, k = g % st.K;
   if (st.done[c]) return;
   Draws<MODE> dr;
-  dr.init_philox(pc.seed, (uint64_t)(pc.chain_offset + c), (uint32_t)(pc.sweep * st.K + k), 1u);
+  dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)(pc.sweep * st.K + k), 1u);
   if (MODE == 1) {
     size_t s = (size_t)c * pc.steps + pc.step_base + k;
     dr.init_tape(pc.tape, (int)pc.tape_off[s], (int)pc.tape_off[s + 1]);

@@ -117,9 +117,11 @@ __global__ void k_convert(const TI* in, TO* out, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = (TO)in[i];
 }
 
-// row-major float64 (n x d) -> column-major T (d x ld)
+// row-major float64 (n x d) -> column-major T (d x ld); blockIdx.y: data set ([D][n][d] -> [D][d][ld])
 template <typename TO>
 __global__ void k_transpose_in(const double* in, TO* out, int64_t n, int d, int64_t ld) {
+  in += (size_t)blockIdx.y * n * d;
+  out += (size_t)blockIdx.y * d * ld;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n * d; i += (int64_t)gridDim.x * blockDim.x) {
     int64_t row = i / d;
     int col = (int)(i % d);
@@ -127,9 +129,11 @@ __global__ void k_transpose_in(const double* in, TO* out, int64_t n, int d, int6
   }
 }
 
-// y statistics: sum(y), y'y in fp64 (single block, deterministic order per launch geometry)
-__global__ void k_y_stats(const double* y, int64_t n, double* out2) {
+// y statistics: sum(y), y'y in fp64 (one block per data set, deterministic order per launch geometry): y [D][ld] -> out2 [D][2]
+__global__ void k_y_stats(const double* y, int64_t n, int64_t ld, double* out2) {
   __shared__ double s1[32], s2[32];
+  y += (size_t)blockIdx.x * ld;
+  out2 += 2 * (size_t)blockIdx.x;
   double a = 0.0, b = 0.0;
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) { double v = y[i]; a += v; b = fma(v, v, b); }
   a = warp_sum(a); b = warp_sum(b);

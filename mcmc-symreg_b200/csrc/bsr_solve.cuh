@@ -293,10 +293,8 @@ __device__ __forceinline__ void store_live_gram(const GramView& gv, const int* i
 struct ResolveCtx {
   double n_total;      // global number of rows
   double n_local;      // rows on this rank (for the executed node-eval counter)
-  double sum_y, yy;    // sum(y), y'y over all rows
+  const double* ystats; // sum(y), y'y over all rows: entry 0 of the handle's [D][2] (this pipeline runs on one data set)
   double pivot_tol;
-  uint64_t seed;
-  int64_t chain_offset;
   int64_t sweep;       // global sweep index (Philox counter)
   // tape / trace window (may be null)
   const double* tape;
@@ -328,7 +326,7 @@ __device__ __forceinline__ void precompute_slot(const ResolveCtx& rc, int K, int
   bool finite_cols = true;
   for (int j = 0; j < K; ++j) { idx[j] = (j == k) ? (K + k) : j; finite_cols = finite_cols && (gv.mx(idx[j]) <= DBL_MAX); }
   if (!finite_cols || rank_deficient<LD>(gv, idx, K, rc.n_total, rc.pivot_tol)) { rank_rej = true; return; }
-  sse_new = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.sum_y, rc.yy, beta);
+  sse_new = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.ystats[0], rc.ystats[1], beta);
 }
 
 // pinfo: the K PropInfo records of this chain (any address space).  pre_rank / pre_sse: results of precompute_slot
@@ -346,8 +344,8 @@ __device__ void resolve_chain(const ChainState& st, const ResolveCtx& rc, int c,
 
   if (init_only) {   // initial fit of a fresh state (bsr_class.py:147-163) + the state's K-column SSE
     for (int j = 0; j < K; ++j) idx[j] = j;
-    st.sse[c] = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.sum_y, rc.yy, beta);
-    (void)ridge_sse<LD, true>(gv, idx, K, rc.n_total, rc.sum_y, rc.yy, beta);
+    st.sse[c] = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.ystats[0], rc.ystats[1], beta);
+    (void)ridge_sse<LD, true>(gv, idx, K, rc.n_total, rc.ystats[0], rc.ystats[1], beta);
     for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = beta[j];
     if (st.sg != nullptr) store_live_gram(gv, idx, K, st.sg + (size_t)c * sg_size(K));
     return;
@@ -394,7 +392,7 @@ __device__ void resolve_chain(const ChainState& st, const ResolveCtx& rc, int c,
         bool finite_cols = true;
         for (int j = 0; j < K; ++j) finite_cols = finite_cols && (gv.mx(idx[j]) <= DBL_MAX);
         deficient = !finite_cols || rank_deficient<LD>(gv, idx, K, rc.n_total, rc.pivot_tol);
-        if (!deficient) sse_new = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.sum_y, rc.yy, beta);
+        if (!deficient) sse_new = ridge_sse<LD, false>(gv, idx, K, rc.n_total, rc.ystats[0], rc.ystats[1], beta);
       }
       if (deficient) {
         rank_rej = true;                                                     // funcs.py:1226-1228: no accept draw
@@ -416,7 +414,7 @@ __device__ void resolve_chain(const ChainState& st, const ResolveCtx& rc, int c,
           u = (lo < hi) ? rc.tape[lo] : 0.5;
         } else {
           Draws<0> dr;
-          dr.init_philox(rc.seed, (uint64_t)(rc.chain_offset + c), (uint32_t)(rc.sweep * K + k), 2u);
+          dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)(rc.sweep * K + k), 2u);
           u = dr.u01();
         }
         accepted = !(log(u) >= alpha);                                       // funcs.py:1300
@@ -443,7 +441,7 @@ __device__ void resolve_chain(const ChainState& st, const ResolveCtx& rc, int c,
       if (st.live_bad != nullptr) st.live_bad[c * K + k] = st.prop_bad[c * K + k];
       any_accept = true;
       // intercept refit + RMSE (bsr_class.py:211-233)
-      double sse_i = ridge_sse<LD, true>(gv, cur, K, rc.n_total, rc.sum_y, rc.yy, beta);
+      double sse_i = ridge_sse<LD, true>(gv, cur, K, rc.n_total, rc.ystats[0], rc.ystats[1], beta);
       for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = beta[j];
       double rmse = sqrt(sse_i / rc.n_total);
       if (nerr < st.err_cap) st.err[(size_t)c * st.err_cap + nerr] = rmse;

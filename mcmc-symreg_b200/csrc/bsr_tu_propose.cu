@@ -5,7 +5,7 @@
 
 int bsr_launch_init_chains(bsr_handle* h, cudaStream_t s) {
   const int total = h->cfg.n_chains * h->cfg.K;
-  k_init_chains<0><<<(total + 63) / 64, 64, 0, s>>>(h->st, h->d_pt, h->seed, h->cfg.chain_offset);
+  k_init_chains<0><<<(total + 63) / 64, 64, 0, s>>>(h->st, h->d_pt);
   CK(cudaGetLastError());
   return 0;
 }
@@ -13,7 +13,7 @@ int bsr_launch_init_chains(bsr_handle* h, cudaStream_t s) {
 int bsr_launch_propose(bsr_handle* h, cudaStream_t s, int c0, int cn) {
   const int total = cn * h->cfg.K;
   ProposeCtx pc;
-  pc.seed = h->seed; pc.chain_offset = h->cfg.chain_offset; pc.sweep = h->sweep;
+  pc.sweep = h->sweep;
   pc.tape = h->tape; pc.tape_off = h->tape_off; pc.steps = h->tape_steps; pc.step_base = h->tape_pos;
   pc.rec = h->rec; pc.rec_count = h->rec_count; pc.rec_steps = h->rec_steps; pc.rec_cap = h->rec_cap; pc.rec_base = h->rec_pos;
   pc.c0 = c0; pc.cn = cn;

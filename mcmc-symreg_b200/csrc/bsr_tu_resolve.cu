@@ -5,9 +5,9 @@
 
 static ResolveCtx make_rc(bsr_handle* h) {
   ResolveCtx rc;
-  rc.n_total = (double)h->n_total; rc.n_local = (double)h->n; rc.sum_y = h->sum_y; rc.yy = h->yy;
+  rc.n_total = (double)h->n_total; rc.n_local = (double)h->n; rc.ystats = h->ystats;
   rc.pivot_tol = h->cfg.precision == 1 ? 1e-13 : 3e-13;
-  rc.seed = h->seed; rc.chain_offset = h->cfg.chain_offset; rc.sweep = h->sweep;
+  rc.sweep = h->sweep;
   rc.tape = h->tape_mode ? h->tape : nullptr; rc.tape_off = h->tape_off;
   rc.trace = (h->tape_pos < h->tape_steps) ? h->trace : nullptr;
   rc.steps = h->tape_steps; rc.step_base = h->tape_pos;

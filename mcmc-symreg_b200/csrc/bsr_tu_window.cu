@@ -174,10 +174,10 @@ static int ensure_window(bsr_handle* h, int S) {
   return 0;
 }
 
-template <typename T, int KC, bool EXACT>
+template <typename T, int KC, bool EXACT, bool MULTI>
 static int launch_weval_t(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads) {
   const size_t smem = win_smem_layout<T>(h->cfg.K, ws.W, threads / 32, wc.TR).total;
-  CK(cudaFuncSetAttribute(k_weval<T, KC, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  CK(cudaFuncSetAttribute(k_weval<T, KC, EXACT, MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   {
     // leave the rest of the unified L1 / shared-memory array to L1: the interpreter's operand stack (local memory) and
     // the leaf loads of X live there.  Ask for just enough shared memory for the blocks the register file admits.
@@ -185,9 +185,9 @@ static int launch_weval_t(bsr_handle* h, const WinState& ws, cudaStream_t s, con
     const size_t need = (size_t)resident * (smem + 1024);
     int pct = (int)((need * 100 + 228 * 1024 - 1) / (228 * 1024));
     if (const char* e = getenv("BSR_WEVAL_CARVEOUT")) pct = atoi(e);
-    CK(cudaFuncSetAttribute(k_weval<T, KC, EXACT>, cudaFuncAttributePreferredSharedMemoryCarveout, std::min(100, std::max(0, pct))));
+    CK(cudaFuncSetAttribute(k_weval<T, KC, EXACT, MULTI>, cudaFuncAttributePreferredSharedMemoryCarveout, std::min(100, std::max(0, pct))));
   }
-  k_weval<T, KC, EXACT><<<dim3(wc.cn, ws.S), threads, smem, s>>>(h->st, ws, wc);
+  k_weval<T, KC, EXACT, MULTI><<<dim3(wc.cn, ws.S), threads, smem, s>>>(h->st, ws, wc);
   CK(cudaGetLastError());
   return 0;
 }
@@ -215,19 +215,24 @@ static int launch_wlive_t(bsr_handle* h, const WinState& ws, cudaStream_t s, con
   }
 #endif
 
-static int launch_weval(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads) {
+template <bool MULTI>
+static int launch_weval_m(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads) {
   if (h->cfg.precision == 0) {
-#define EX(KC) launch_weval_t<float, KC, true>(h, ws, s, wc, threads)
-#define GEN() launch_weval_t<float, BSR_MAXK, false>(h, ws, s, wc, threads)
+#define EX(KC) launch_weval_t<float, KC, true, MULTI>(h, ws, s, wc, threads)
+#define GEN() launch_weval_t<float, BSR_MAXK, false, MULTI>(h, ws, s, wc, threads)
     BSR_WIN_DISPATCH(EX, GEN)
 #undef EX
 #undef GEN
   }
-#define EX(KC) launch_weval_t<double, KC, true>(h, ws, s, wc, threads)
-#define GEN() launch_weval_t<double, BSR_MAXK, false>(h, ws, s, wc, threads)
+#define EX(KC) launch_weval_t<double, KC, true, MULTI>(h, ws, s, wc, threads)
+#define GEN() launch_weval_t<double, BSR_MAXK, false, MULTI>(h, ws, s, wc, threads)
   BSR_WIN_DISPATCH(EX, GEN)
 #undef EX
 #undef GEN
+}
+// a handle of one data set runs the instances without a data-set term (k_weval)
+static int launch_weval(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads) {
+  return h->n_ds > 1 ? launch_weval_m<true>(h, ws, s, wc, threads) : launch_weval_m<false>(h, ws, s, wc, threads);
 }
 static int launch_wlive(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads, double* lrec) {
   if (h->cfg.precision == 0) {
@@ -263,26 +268,30 @@ static int launch_wpropose(bsr_handle* h, const WinState& ws, cudaStream_t s, Wi
   return 0;
 }
 
-static int launch_wresolve(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc) {
+template <bool MULTI>
+static int launch_wresolve_m(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc) {
   const int K = h->cfg.K;
   const int threads = 128, lpc = ws.W > 32 ? 64 : 32, cpb = threads / lpc, blocks = (wc.cn + cpb - 1) / cpb;
   const size_t smem = (size_t)cpb * (sg_size(K) * sizeof(double) + 8 * sizeof(unsigned));
   switch (K) {
-    case 1: k_wresolve<1><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 2: k_wresolve<2><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 3: k_wresolve<3><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 4: k_wresolve<4><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 5: k_wresolve<5><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 10: k_wresolve<10><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;     // BASELINE configs[2]
-    default: k_wresolve<0><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 1: k_wresolve<1, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 2: k_wresolve<2, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 3: k_wresolve<3, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 4: k_wresolve<4, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 5: k_wresolve<5, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 10: k_wresolve<10, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;     // BASELINE configs[2]
+    default: k_wresolve<0, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
   }
   CK(cudaGetLastError());
   return 0;
 }
+static int launch_wresolve(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc) {
+  return h->n_ds > 1 ? launch_wresolve_m<true>(h, ws, s, wc) : launch_wresolve_m<false>(h, ws, s, wc);
+}
 
 static WinCtx make_wc(bsr_handle* h, long long p_start, long long p_target, uint32_t rps, uint32_t TR) {
   WinCtx wc;
-  wc.seed = h->seed; wc.chain_offset = h->cfg.chain_offset; wc.p_target = p_target;
+  wc.p_target = p_target;
   wc.c0 = 0; wc.cn = h->cfg.n_chains;
   const bool recording = h->rec != nullptr && h->rec_pos < h->rec_steps;
   wc.rec_draws = recording ? h->rec : nullptr; wc.rec_count = h->rec_count; wc.rec_steps = h->rec_steps; wc.rec_cap = h->rec_cap;
@@ -293,13 +302,13 @@ static WinCtx make_wc(bsr_handle* h, long long p_start, long long p_target, uint
   wc.tape = taped ? h->tape : nullptr; wc.tape_off = h->tape_off;
   wc.log_tok = tracing ? h->log_tok : nullptr; wc.log_pa = h->log_pa; wc.log_pb = h->log_pb; wc.log_nn = h->log_nn;
   wc.X32 = h->X32; wc.X64 = h->X64; wc.y64 = h->y64;
-  wc.n = (uint32_t)h->n; wc.ld = (uint32_t)h->ld; wc.precision = h->cfg.precision;
+  wc.n = (uint32_t)h->n; wc.ld = (uint32_t)h->ld; wc.ds_stride = (uint32_t)(h->d * h->ld); wc.precision = h->cfg.precision;
   wc.rows_per_split = rps; wc.TR = TR;
   // 2: repeated trees are interpreted once per window AND trees of the chain's earlier windows in the ring take their record from there;
   // 1: within the window only (BSR_WIN_NO_CACHE); 0: every slot is interpreted (BSR_WIN_NO_DEDUP) -- for A/B runs and tests
   wc.dedup = getenv("BSR_WIN_NO_DEDUP") ? 0 : (getenv("BSR_WIN_NO_CACHE") ? 1 : 2);
   wc.checked_m = getenv("BSR_WIN_NO_CHECKED") ? (1 << 30) : BSR_CHECKED_M;      // (A/B runs and tests)
-  wc.n_total = (double)h->n_total; wc.n_local = (double)h->n; wc.sum_y = h->sum_y; wc.yy = h->yy;
+  wc.n_total = (double)h->n_total; wc.n_local = (double)h->n; wc.sum_y = h->sum_y; wc.yy = h->yy; wc.ystats = h->ystats;
   wc.pivot_tol = h->cfg.precision == 1 ? 1e-13 : 3e-13;
   wc.n_peers = 0;
   for (int r = 0; r < BSR_MAX_PEERS; ++r) { wc.peer_rec[r] = nullptr; wc.peer_bad[r] = nullptr; wc.peer_lrec[r] = nullptr; }
@@ -519,6 +528,7 @@ int bsr_get_window_geometry(bsr_handle* h, int64_t* geom5) {
 
 int bsr_peer_export(bsr_handle* h, int32_t world, void* ipc_handle_out) {
   if (!h || !ipc_handle_out) return bsr_fail("bsr_peer_export: null argument");
+  if (h->n_ds > 1) return bsr_fail("bsr_peer_export: not available on a handle with several data sets (bsr_set_datasets_host)");
   if (!h->cfg.row_sharded) return bsr_fail("bsr_peer_export: the handle was not created with row_sharded = 1");
   if (!h->X32) return bsr_fail("bsr_peer_export: call bsr_set_data_* first (the exchange buffer is sized from the data)");
   if (world < 1 || world > BSR_MAX_PEERS) return bsr_fail("bsr_peer_export: world must be in [1, 8]");
@@ -548,6 +558,7 @@ int bsr_peer_export(bsr_handle* h, int32_t world, void* ipc_handle_out) {
 
 int bsr_peer_import(bsr_handle* h, int32_t rank, int32_t world, const void* ipc_handles) {
   if (!h || !ipc_handles) return bsr_fail("bsr_peer_import: null argument");
+  if (h->n_ds > 1) return bsr_fail("bsr_peer_import: not available on a handle with several data sets (bsr_set_datasets_host)");
   if (!h->xbuf) return bsr_fail("bsr_peer_import: call bsr_peer_export first");
   if (world < 1 || world > BSR_MAX_PEERS || rank < 0 || rank >= world) return bsr_fail("bsr_peer_import: bad rank / world");
   CK(cudaSetDevice(h->cfg.device));

@@ -6,7 +6,7 @@
 // proposals is generated from the SAME live state, all W are evaluated and scored in parallel, and the window is then
 // consumed in order up to and including its first accept (or a stop rule); the proposals behind an accept were
 // generated from a stale state and are discarded -- the next window regenerates them from the new state.  Every
-// random draw is a Philox function of (seed, global chain id, proposal index, purpose), so the chain is exactly the
+// random draw is a Philox function of (the chain's key, proposal index, purpose), so the chain is exactly the
 // one the proposal-by-proposal pipeline (bsr_kernels.cuh) produces; only the order of the work changes:
 //
 //   k_wpropose  one thread per (chain, window slot): Prop + auxProp + fStruc     codes/funcs.py:1188-1210
@@ -39,8 +39,6 @@
 #endif
 
 struct WinCtx {
-  uint64_t seed;
-  int64_t chain_offset;
   long long p_target;      // chains stop consuming at this proposal index
   int c0, cn;              // chain range of this launch
   int* bucket;             // [BSR_N_BINS][bucket_stride] window slots (ci * W + i) of this launch sorted by bin
@@ -54,16 +52,18 @@ struct WinCtx {
   const double* tape; const int64_t* tape_off;
   // proposed trees of the consumed proposals, by trace row (tests: bit-exact comparison with the reference's proposals)
   uint32_t* log_tok; double* log_pa; double* log_pb; int* log_nn;
-  // data
+  // data: D data sets of the same shape, X [D][d][ld], y [D][ld]; chain c reads data set st.ds[c], whose X starts at
+  // ds * ds_stride (folded into the leaf offsets by stage_tokens) and whose y at ds * ld
   const float* X32; const double* X64; const double* y64;
-  uint32_t n, ld;
+  uint32_t n, ld, ds_stride;
   int precision;
   uint32_t rows_per_split;   // multiple of 4
   uint32_t TR;               // rows per shared-memory tile, multiple of 4
   int checked_m;             // node count from which k_weval's first pass tells finite from out-of-range vectors itself (K > 5 kernels)
   int dedup;                 // 0: every slot is interpreted; 1: repeated trees of a window once; 2: and trees of the chain's earlier windows (ring) not at all
   // resolve
-  double n_total, n_local, sum_y, yy, pivot_tol;
+  double n_total, n_local, sum_y, yy, pivot_tol;   // sum_y, yy: data set 0 (the kernels of one data set take them by value)
+  const double* ystats;      // [D][2] sum(y), y'y of every data set
   // row-sharded handles: the records / out-of-range masks of this window on every rank (peer memory over NVLink,
   // index = rank); n_peers == 0: single device, ws.rec / ws.bad
   int n_peers;
@@ -180,7 +180,7 @@ static __global__ void k_wclassify(ChainState st, WinState ws, WinCtx wc) {
           }
         } else {
           Draws<0> dr;
-          dr.init_philox(wc.seed, (uint64_t)(wc.chain_offset + c), (uint32_t)p, 1u);
+          dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)p, 1u);
           test = dr.u01();
         }
         mv = select_move(L, Nt, D, test) * BSR_N_SIZE_CLASSES + (BSR_N_SIZE_CLASSES == 4 ? (m <= 4 ? 0 : (m <= 8 ? 1 : (m <= 16 ? 2 : 3))) : (BSR_N_SIZE_CLASSES == 2 ? (L > 0 ? 1 : 0) : 0));
@@ -242,7 +242,7 @@ __global__ void __launch_bounds__(64, BSR_WPROP_MINB) k_wpropose(ChainState st, 
   const int k = (int)(p % K);
   const int g = c * K + k;
   Draws<MODE> dr;
-  dr.init_philox(wc.seed, (uint64_t)(wc.chain_offset + c), (uint32_t)p, 1u);
+  dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)p, 1u);
   const long long ri = p - wc.rec_origin;
   const bool recording = MODE == 2 && wc.rec_draws != nullptr && ri >= 0 && ri < wc.rec_steps;
   if (recording) dr.init_record(wc.rec_draws + ((size_t)c * wc.rec_steps + ri) * wc.rec_cap, wc.rec_cap);
@@ -292,7 +292,7 @@ __host__ __device__ inline WinSmem win_smem_layout(int K, int W, int NW, uint32_
   s.ltok = o; o += (size_t)K * BSR_MAXN * sizeof(EvTok<T>);
   s.ptok = o; o += (size_t)NW * BSR_MAXN * sizeof(EvTok<T>);
   o = (o + 15) / 16 * 16;
-  s.lm = o; o += (size_t)(K + (K & 1) + 8) * sizeof(int);   // + three 64-bit slot masks (second pass needed / its vectors already known / column not finite), + the work counter
+  s.lm = o; o += (size_t)(K + (K & 1) + 8) * sizeof(int);   // + three 64-bit slot masks (second pass needed / its vectors already known / column not finite), + the work counter, + the data set
   o = (o + 15) / 16 * 16;
   s.dd = o; o += 320;                                                   // results of the duplicate search (sizeof(DedupSmem))
   s.bm = o; if (sizeof(T) == 4 && K > 5) o += (size_t)W * 8 * sizeof(unsigned);   // per slot: which of the tile's <= 256 vectors are out of range (large trees, see k_weval)
@@ -300,13 +300,14 @@ __host__ __device__ inline WinSmem win_smem_layout(int K, int W, int NW, uint32_
   return s;
 }
 
+// xbase: offset of the chain's data set in X (ds * d * ld): the interpreters reach X through the leaf offsets alone
 template <typename T>
-__device__ __forceinline__ void stage_tokens(const uint32_t* tok, const double* pa, const double* pb, int m, uint32_t ld,
+__device__ __forceinline__ void stage_tokens(const uint32_t* tok, const double* pa, const double* pb, int m, uint32_t xbase, uint32_t ld,
                                              EvTok<T>* dst, int t0, int step) {
   for (int t = t0; t < m; t += step) {
     const uint32_t tk = tok[t];
     EvTok<T> e;
-    e.op = tok_op(tk); e.off = (uint32_t)tok_ft(tk) * ld;
+    e.op = tok_op(tk); e.off = xbase + (uint32_t)tok_ft(tk) * ld;
     e.a = (T)0; e.b = (T)0;
     if (e.op == OP_LT) { e.a = (T)pa[t]; e.b = (T)pb[t]; }      // one operator in ten: the other tokens cost one load, not three
     dst[t] = e;
@@ -361,12 +362,13 @@ static __device__ BSR_WIDE_INLINE double2 eval_tree_wide2(const EvTok<float>* tk
 }
 
 // The K live columns and y on rows [row_lo, row_lo + tile_rows) -> shared memory (fp64).  Block-cooperative; the
-// caller synchronises before and after.  Rows >= n are written as zeros.
+// caller synchronises before and after.  Rows >= n are written as zeros.  ds: the chain's data set (its y; the live tokens
+// were staged with its X offset).
 // lcol (fp32 mode, k_weval only; nullptr otherwise): the cache of live columns (WinState::lcol ...).  A column whose flag is set is
 // loaded instead of interpreted -- the same fp32 values; an interpreted one is written to the cache, k_wresolve sets its flag when the
 // window is over (unless the tree was replaced or the column had an out-of-range vector: *wide_mask).
 template <typename T>
-__device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc, int c, int K, const EvTok<T>* s_ltok, const int* s_lm,
+__device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc, int c, int K, uint32_t ds, const EvTok<T>* s_ltok, const int* s_lm,
                                           uint32_t row_lo, uint32_t tile_rows, double2* s_live, float* lcol = nullptr, long long lcol_ld = 0,
                                           const unsigned char* lcol_ok = nullptr, unsigned* wide_mask = nullptr) {
   constexpr int R = RowVec<T>::R, NP = R / 2;
@@ -422,7 +424,7 @@ __device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc
   const uint32_t tv2 = tv * NP;
   for (uint32_t q2 = threadIdx.x; q2 < tv2; q2 += blockDim.x) {
     const uint32_t r0 = row_lo + q2 * 2;
-    const double2 yv = *reinterpret_cast<const double2*>(wc.y64 + r0);
+    const double2 yv = *reinterpret_cast<const double2*>(wc.y64 + (size_t)ds * wc.ld + r0);
     double2 d;
     d.x = (r0 < wc.n) ? yv.x : 0.0;
     d.y = (r0 + 1 < wc.n) ? yv.y : 0.0;
@@ -678,7 +680,7 @@ __device__ __forceinline__ void add_record(const WAcc<KC>& a, double* d, int K, 
 // it must not cost the fp32 loop of k_weval a register.  Must be called by every thread of the block.
 template <int KC>
 static __device__ BSR_WIDE_INLINE void careful_tile(const uint32_t* __restrict__ tok, const double* __restrict__ pa, const double* __restrict__ pb, int m,
-                                                 const float* __restrict__ X32, const double* __restrict__ X64, uint32_t ld, uint32_t n, int K, int i,
+                                                 const float* __restrict__ X32, const double* __restrict__ X64, uint32_t xbase, uint32_t ld, uint32_t n, int K, int i,
                                                  uint32_t t_lo, uint32_t tile_rows, const double2* s_live, EvTok<float>* s_tok, double* s_part,
                                                  double* s_acc, unsigned long long* s_dead, const unsigned* bm) {
   const int RECN = K + 4;
@@ -690,7 +692,7 @@ static __device__ BSR_WIDE_INLINE void careful_tile(const uint32_t* __restrict__
   unsigned short* s_list = reinterpret_cast<unsigned short*>(reinterpret_cast<unsigned char*>(s_tok) + 2560);   // [<= tv] their indices, ascending
   const int nsteps = (int)((tv + blockDim.x - 1) / blockDim.x);       // <= 8 (tile budget of win_geometry: tv <= 640)
   __syncthreads();
-  stage_tokens<float>(tok, pa, pb, m, ld, s_tok, threadIdx.x, blockDim.x);
+  stage_tokens<float>(tok, pa, pb, m, xbase, ld, s_tok, threadIdx.x, blockDim.x);
   __syncthreads();
   WAcc<KC> a;
   a.zero();
@@ -762,7 +764,10 @@ static __device__ BSR_WIDE_INLINE void careful_tile(const uint32_t* __restrict__
                             // (64 registers, 220 KB of shared memory, ~28 KB left for L1) measured slower: the interpreter's
                             // local-memory stack then misses L1 (hit rate 60 %, long-scoreboard stalls on top)
 #endif
-template <typename T, int KC, bool EXACT>
+// MULTI: the handle holds several data sets and every chain reads its own (st.ds).  The instances of one data set (MULTI = false)
+// have no data-set term at all: whatever the term is written as, ptxas allocates the 80-register tile loop differently for it, with
+// more spills in some instances (DESIGN.md section 5), and a handle of one data set must not pay for that.
+template <typename T, int KC, bool EXACT, bool MULTI>
 __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 : (KC <= 5 ? 3 : 2))) k_weval(ChainState st, WinState ws, WinCtx wc) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int c = wc.c0 + blockIdx.x;
@@ -781,11 +786,13 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
   unsigned long long* s_dead = s_flag + 1;                                                  // slots whose column is not finite even in double range
   unsigned long long* s_pre = s_dead + 1;                                                   // slots of this tile whose out-of-range vectors the first pass listed (s_bm)
   int* s_next = reinterpret_cast<int*>(s_pre + 1);
+  int* s_ds = s_next + 1;                                                                   // (MULTI) the chain's data set: read where it is
+                                                                                            // used, so that the tile loop holds no register for it
   unsigned* s_bm = reinterpret_cast<unsigned*>(smem_raw + L.bm);
   const T* X = (sizeof(T) == 4) ? reinterpret_cast<const T*>(wc.X32) : reinterpret_cast<const T*>(wc.X64);
   DedupSmem& dd = *reinterpret_cast<DedupSmem*>(smem_raw + L.dd);
   const unsigned char* s_rep = dd.rep;
-  if (threadIdx.x == 0) { *s_flag = 0ull; *s_dead = 0ull; }
+  if (threadIdx.x == 0) { *s_flag = 0ull; *s_dead = 0ull; if (MULTI) *s_ds = st.ds[c]; }
   const int head = ws.chead[c];                   // ring index of the chain's last window (still valid for the live state), or -1
   const int nprev = (head >= 0 && wc.dedup >= 2) ? (int)ws.cvalid[c] : 0;
   const WinState wv = win_half(ws, head >= 0 ? ((head + 1) % ws.R) : 0, K);     // this window's slots (win_parity)
@@ -798,13 +805,14 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
     dd.m[threadIdx.x] = (wv.hash[wi] != 0ull) ? (unsigned char)wv.nn[wi] : (unsigned char)0;
   }
   if (n_eval > 0) {
+    const uint32_t xbase = MULTI ? (uint32_t)st.ds[c] * wc.ds_stride : 0u;
     for (int j = 0; j < K; ++j) {
       const int g = c * K + j;
       const int w = st.which[g];
       const int m = st.nn[w][g];
       if (threadIdx.x == 0) s_lm[j] = m;
       const size_t slot = (size_t)g * BSR_MAXN;
-      stage_tokens<T>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, wc.ld, s_ltok + j * BSR_MAXN, threadIdx.x, blockDim.x);
+      stage_tokens<T>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, xbase, wc.ld, s_ltok + j * BSR_MAXN, threadIdx.x, blockDim.x);
     }
     for (int i = threadIdx.x; i < W * RECN; i += blockDim.x) s_acc[i] = 0.0;
   }
@@ -820,8 +828,8 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
     if (n_eval == 0) continue;                     // every tree of this window has its record already (block-uniform)
     // (the cache of live columns and the checked first pass belong to the K > 5 kernels: the 80-register kernels of K <= 5 pay for the
     // extra paths in spills -- measured: C4 -3 %, C5 -7 % -- what the cache gives their 4-node trees)
-    if (KC > 5) live_tile<T>(st, wc, c, K, s_ltok, s_lm, t_lo, tile_rows, s_live, ws.lcol, ws.lcol_ld, ws.lcol_ok, ws.lcol_wide);
-    else live_tile<T>(st, wc, c, K, s_ltok, s_lm, t_lo, tile_rows, s_live);
+    if (KC > 5) live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, s_ltok, s_lm, t_lo, tile_rows, s_live, ws.lcol, ws.lcol_ld, ws.lcol_ok, ws.lcol_wide);
+    else live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, s_ltok, s_lm, t_lo, tile_rows, s_live);
     __syncthreads();
     const uint32_t tv = (tile_rows + R - 1) / R;
     const unsigned long long dead = *s_dead;      // columns found non-finite on an earlier tile: their record is settled (reject)
@@ -838,7 +846,8 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
       const size_t wi = (size_t)c * W + i;
       const int m = dd.m[i];                     // (node count of the slot, staged with the results of the duplicate search)
       __syncwarp();
-      stage_tokens<T>(wv.tok + wi * BSR_MAXN, wv.pa + wi * BSR_MAXN, wv.pb + wi * BSR_MAXN, m, wc.ld, s_ptok, lane, 32);
+      stage_tokens<T>(wv.tok + wi * BSR_MAXN, wv.pa + wi * BSR_MAXN, wv.pb + wi * BSR_MAXN, m, MULTI ? (uint32_t)*s_ds * wc.ds_stride : 0u, wc.ld, s_ptok, lane,
+                      32);
       __syncwarp();
       WAcc<KC> a;
       // NV interleaved row vectors per thread and token decode: vector u of lane l is vector q + 32 u of the tile
@@ -923,7 +932,9 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
         for (unsigned long long rest = tmask; rest != 0ull; rest &= rest - 1ull) {
           const int i = __ffsll((long long)rest) - 1;
           const size_t wi = (size_t)c * W + i;
-          careful_tile<KC>(wv.tok + wi * BSR_MAXN, wv.pa + wi * BSR_MAXN, wv.pb + wi * BSR_MAXN, wv.nn[wi], wc.X32, wc.X64, wc.ld, wc.n, K, i, t_lo, tile_rows,
+          careful_tile<KC>(wv.tok + wi * BSR_MAXN, wv.pa + wi * BSR_MAXN, wv.pb + wi * BSR_MAXN, wv.nn[wi], wc.X32, wc.X64,
+                           MULTI ? (uint32_t)*s_ds * wc.ds_stride : 0u, wc.ld,
+                           wc.n, K, i, t_lo, tile_rows,
                            s_live, s_tok0, s_part, s_acc, s_dead, (KC > 5 && ((pre >> i) & 1ull)) ? s_bm + i * 8 : nullptr);
         }
         wide_mask |= tmask;
@@ -974,6 +985,7 @@ static __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_bad(ChainSta
   const int K = st.K;
   const uint32_t r_lo = blockIdx.y * wc.rows_per_split;
   const uint32_t r_hi = min(wc.n, r_lo + wc.rows_per_split);
+  const uint32_t xbase = (uint32_t)st.ds[c] * wc.ds_stride;
   for (int j = 0; j < K; ++j) {
     const int g = c * K + j;
     const int w = st.which[g];
@@ -981,7 +993,7 @@ static __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_bad(ChainSta
     const size_t slot = (size_t)g * BSR_MAXN;
     __syncthreads();
     if (threadIdx.x == 0) s_bad = 0;
-    stage_tokens<float>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, wc.ld, s_tok, threadIdx.x, blockDim.x);
+    stage_tokens<float>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, xbase, wc.ld, s_tok, threadIdx.x, blockDim.x);
     __syncthreads();
     bool bad = false;
     for (uint32_t row0 = r_lo + threadIdx.x * 4; row0 < r_hi; row0 += blockDim.x * 4) {
@@ -1047,8 +1059,9 @@ static __global__ void k_wrefit(ChainState st, WinCtx wc, int S, int c0, int cn)
   int il[BSR_MAXK];
   double bl[BSR_LDA];
   for (int j = 0; j < K; ++j) il[j] = j;
-  st.sse[c] = ridge_sse<BSR_LDA, false>(gl, il, K, wc.n_total, wc.sum_y, wc.yy, bl);
-  (void)ridge_sse<BSR_LDA, true>(gl, il, K, wc.n_total, wc.sum_y, wc.yy, bl);
+  const double* ys = wc.ystats + 2 * (size_t)st.ds[c];
+  st.sse[c] = ridge_sse<BSR_LDA, false>(gl, il, K, wc.n_total, ys[0], ys[1], bl);
+  (void)ridge_sse<BSR_LDA, true>(gl, il, K, wc.n_total, ys[0], ys[1], bl);
   for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = bl[j];
 }
 
@@ -1066,13 +1079,14 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
   double* s_red = reinterpret_cast<double*>(smem_raw + L.total);      // [NW][sgn], behind the layout k_weval uses
   EvTok<T>* s_ltok = reinterpret_cast<EvTok<T>*>(smem_raw + L.ltok);
   int* s_lm = reinterpret_cast<int*>(smem_raw + L.lm);
+  const uint32_t ds = (uint32_t)st.ds[c];
   for (int j = 0; j < K; ++j) {
     const int g = c * K + j;
     const int w = st.which[g];
     const int m = st.nn[w][g];
     if (threadIdx.x == 0) s_lm[j] = m;
     const size_t slot = (size_t)g * BSR_MAXN;
-    stage_tokens<T>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, wc.ld, s_ltok + j * BSR_MAXN, threadIdx.x, blockDim.x);
+    stage_tokens<T>(st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, m, ds * wc.ds_stride, wc.ld, s_ltok + j * BSR_MAXN, threadIdx.x, blockDim.x);
   }
   double g_[NG], by[KC], cs[KC], mx[KC];
 #pragma unroll
@@ -1085,7 +1099,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
   for (uint32_t t_lo = r_lo; t_lo < r_hi; t_lo += wc.TR) {
     const uint32_t tile_rows = min(wc.TR, r_hi - t_lo);
     __syncthreads();
-    live_tile<T>(st, wc, c, K, s_ltok, s_lm, t_lo, tile_rows, s_live);
+    live_tile<T>(st, wc, c, K, ds, s_ltok, s_lm, t_lo, tile_rows, s_live);
     __syncthreads();
     const uint32_t tv = (tile_rows + R - 1) / R;
 #pragma unroll 1
@@ -1150,7 +1164,8 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
 #ifndef BSR_WRES_MINB
 #define BSR_WRES_MINB 4
 #endif
-template <int KT>
+// MULTI: as for k_weval -- the chain's sum(y), y'y come from its data set's entry of wc.ystats, else from wc.sum_y, wc.yy.
+template <int KT, bool MULTI>
 __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(ChainState st, WinState ws, WinCtx wc) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int LD = (KT > 0) ? KT + 1 : BSR_LDA;
@@ -1253,7 +1268,8 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
     if (!finite_cols || rank_deficient<LD>(gv, idx, K, wc.n_total, wc.pivot_tol, dg)) {
       rank_rej = true;                                                         // funcs.py:1226-1228: no accept draw
     } else {
-      sse_new = ridge_sse<LD, false>(gv, idx, K, wc.n_total, wc.sum_y, wc.yy, beta);
+      sse_new = MULTI ? ridge_sse<LD, false>(gv, idx, K, wc.n_total, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
+                      : ridge_sse<LD, false>(gv, idx, K, wc.n_total, wc.sum_y, wc.yy, beta);
       const double ns = pi.new_sigma;
       const double yll_new = -sse_new / (2 * ns * ns) - 0.5 * wc.n_total * log(2 * 3.141592653589793 * ns * ns);
       const double yll_old = -sse_old / (2 * sigma * sigma) - 0.5 * wc.n_total * log(2 * 3.141592653589793 * sigma * sigma);
@@ -1272,7 +1288,7 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
         }
       } else {
         Draws<0> dr;
-        dr.init_philox(wc.seed, (uint64_t)(wc.chain_offset + c), (uint32_t)p, 2u);
+        dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)p, 2u);
         u = dr.u01();
       }
       accepted = !(log(u) >= alpha);                                           // funcs.py:1300
@@ -1390,7 +1406,8 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
       store_live_gram(gv, cur, K, st.sg + (size_t)c * sgn);
       // intercept refit + RMSE (bsr_class.py:211-233)
       double beta[BSR_LDA];
-      const double sse_i = ridge_sse<LD, true>(gv, cur, K, wc.n_total, wc.sum_y, wc.yy, beta);
+      const double sse_i = MULTI ? ridge_sse<LD, true>(gv, cur, K, wc.n_total, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
+                                 : ridge_sse<LD, true>(gv, cur, K, wc.n_total, wc.sum_y, wc.yy, beta);
       for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = beta[j];
       const double rmse = sqrt(sse_i / wc.n_total);
       int nerr = st.nerr[c];

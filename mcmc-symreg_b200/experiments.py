@@ -80,15 +80,34 @@ def run_experiment(func="sim", K=3, MM=50, n_train=100, n_test=30, val=100, seed
     return out, est, data
 
 
-def run_suite(funcs=("f1", "f2", "f3", "f4", "f5", "f6"), repeats=1, **kw):
-    """The whole benchmark suite (the paper's Table 1 recipe: every function, ``repeats`` independent data sets)."""
+def run_suite(funcs=("f1", "f2", "f3", "f4", "f5", "f6"), repeats=1, batched=False, **kw):
+    """The whole benchmark suite (the paper's Table 1 recipe: every function, ``repeats`` independent data sets).
+
+    batched=True fits all (function, repeat) data sets in one GPU run (``BSR.fit_many``) with the seeds the loop uses; the rows
+    are the loop's rows, except that ``fit_seconds`` is the batch's wall clock (fit and summaries) divided by the number of data
+    sets, and ``batch_seconds`` is that wall clock."""
     rows = []
     seed0 = kw.pop("seed", 0)
-    for f in funcs:
-        for r in range(repeats):
-            out, _, _ = run_experiment(f, seed=seed0 + r, **kw)
-            out["repeat"] = r
-            rows.append(out)
+    if not batched:
+        for f in funcs:
+            for r in range(repeats):
+                out, _, _ = run_experiment(f, seed=seed0 + r, **kw)
+                out["repeat"] = r
+                rows.append(out)
+        return rows
+    from .bsr_class import BSR
+    K, MM, n_train, n_test, val = kw.pop("K", 3), kw.pop("MM", 50), kw.pop("n_train", 100), kw.pop("n_test", 30), kw.pop("val", 100)
+    data_seed = kw.pop("data_seed", None)
+    jobs = [(f, r) for f in funcs for r in range(repeats)]
+    data = [make_dataset(f, n_train, n_test, seed=seed0 + r if data_seed is None else data_seed) for f, r in jobs]
+    t0 = time.perf_counter()
+    fits = BSR(K, MM, val=val, **kw).fit_many([(d["X"], d["y"]) for d in data], seeds=[seed0 + r for _, r in jobs])
+    rows = [summarize(est, d) for est, d in zip(fits, data)]
+    batch = time.perf_counter() - t0
+    for o, (_, r) in zip(rows, jobs):
+        o["fit_seconds"] = batch / len(jobs)
+        o["batch_seconds"] = batch
+        o["repeat"] = r
     return rows
 
 
@@ -112,9 +131,11 @@ def main(argv=None):
     ap.add_argument("--repeats", type=int, default=1)
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp64"])
     ap.add_argument("--json", action="store_true", help="one JSON object per experiment instead of the table")
+    ap.add_argument("--batched", action="store_true", help="fit all (function, repeat) data sets in one GPU run (BSR.fit_many)")
     a = ap.parse_args(argv)
     funcs = ("f1", "f2", "f3", "f4", "f5", "f6") if a.func == "all" else (a.func,)
-    rows = run_suite(funcs, a.repeats, K=a.K, MM=a.MM, n_train=a.n_train, n_test=a.n_test, val=a.val, seed=a.seed, precision=a.precision)
+    rows = run_suite(funcs, a.repeats, batched=a.batched, K=a.K, MM=a.MM, n_train=a.n_train, n_test=a.n_test, val=a.val, seed=a.seed,
+                     precision=a.precision)
     for o in rows:
         if a.json:
             print(json.dumps(o))

@@ -41,6 +41,33 @@ def collect(eng):
                 sse=st["sse"], counters=st["counters"], done=st["done"], nerr=st["nerr"], err=eng.get_err_trace())
 
 
+def split_results(res, n_datasets, MM):
+    """The gathered results of ``BSR.fit_many`` (chains b * MM ... (b + 1) * MM - 1 fit data set b) as one result dict per data
+    set, each shaped as ``collect`` / ``gather_results`` shape the results of one fit of MM chains."""
+    nn = np.asarray(res["nn"])
+    assert nn.shape[0] == n_datasets * MM
+    node_off = np.zeros(nn.shape[0] + 1, dtype=np.int64)
+    np.cumsum(nn.sum(axis=1), out=node_off[1:])
+    lt_off = np.zeros(res["ptok"].size + 1, dtype=np.int64)         # lt nodes before every node of the packed token stream
+    np.cumsum((res["ptok"] & 0xFF) == 2, out=lt_off[1:])
+    out = []
+    for b in range(n_datasets):
+        c0, c1 = b * MM, (b + 1) * MM
+        n0, n1 = node_off[c0], node_off[c1]
+        part = {}
+        for key, v in res.items():
+            if key == "ptok":
+                part[key] = v[n0:n1].copy()
+            elif key == "pab":
+                part[key] = v[lt_off[n0]:lt_off[n1]].copy()
+            elif key == "sweeps":
+                part[key] = v
+            else:
+                part[key] = v[c0:c1].copy()
+        out.append(part)
+    return out
+
+
 class _Local:
     rank, world = 0, 1
 

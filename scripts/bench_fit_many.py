@@ -1,0 +1,126 @@
+"""Measures what fitting many small data sets in one GPU run (BSR.fit_many) saves; prints one JSON line.
+
+1. The suite of the paper's Table 1 at the reference's own size: f1 ... f6 x R repeats, BSR(3, 50, val=100) on n = 100 rows.
+   Wall clock of the loop of BSR.fit calls against one BSR.fit_many over the same data sets and seeds, alternated, each timing
+   ending in a device synchronise; the two must give equal results (checked in the same run).
+2. Engine throughput: D data sets x 50 chains on n = 100 rows, fixed sweeps, device-timed (CUDA events) proposals per second.
+
+    python scripts/bench_fit_many.py [--repeats 50] [--rounds 3] [--sweeps 300] [--datasets 1,16,128,1024]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def gpu_info():
+    import torch
+    name = torch.cuda.get_device_name(0)
+    try:
+        power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True,
+                               text=True, timeout=60).stdout.strip()
+    except Exception as e:  # the name still identifies the card
+        power = "unknown (%s)" % type(e).__name__
+    return name, power
+
+
+def suite_data(repeats, n):
+    from mcmc_symreg_b200.experiments import make_dataset
+    jobs = [(f, r) for f in ("f1", "f2", "f3", "f4", "f5", "f6") for r in range(repeats)]
+    return jobs, [make_dataset(f, n, 30, seed=r) for f, r in jobs]
+
+
+def fingerprint(est):
+    return (est.model(), [b.ravel().tolist() for b in est.betas_], est.train_err_, est.counters_.tolist(), est.done_.tolist())
+
+
+def bench_suite(repeats, rounds, n):
+    import torch
+    from sklearn.base import clone
+    from mcmc_symreg_b200 import BSR
+    jobs, data = suite_data(repeats, n)
+    est = BSR(3, 50, val=100)
+    seeds = [r for _, r in jobs]
+    pairs = [(d["X"], d["y"]) for d in data]
+
+    def loop():
+        out = []
+        for (X, y), s in zip(pairs, seeds):
+            e = clone(est).set_params(seed=s)
+            e.fit(X, y)
+            out.append(e)
+        torch.cuda.synchronize()
+        return out
+
+    def batch():
+        out = est.fit_many(pairs, seeds=seeds)
+        torch.cuda.synchronize()
+        return out
+
+    loop(); batch()                               # module loads, allocations
+    t_loop, t_batch, equal = [], [], True
+    for _ in range(rounds):
+        t0 = time.perf_counter(); a = loop(); t_loop.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); b = batch(); t_batch.append(time.perf_counter() - t0)
+        equal = equal and all(fingerprint(x) == fingerprint(y) for x, y in zip(a, b))
+    assert equal, "fit_many and the loop of fits disagree"
+    return dict(datasets=len(jobs), chains_per_fit=50, rows=n, loop_seconds=t_loop, fit_many_seconds=t_batch,
+                loop_ms_per_fit=1e3 * float(np.median(t_loop)) / len(jobs), fit_many_ms_per_fit=1e3 * float(np.median(t_batch)) / len(jobs),
+                speedup_median=float(np.median(t_loop) / np.median(t_batch)), results_equal=equal)
+
+
+def bench_engine(D, sweeps, n, C=50, K=3):
+    import torch
+    from mcmc_symreg_b200 import capi
+    from mcmc_symreg_b200.experiments import TARGETS
+    rng = np.random.default_rng(D)
+    X = rng.uniform(-3, 3, (D, n, 2))
+    y = np.stack([TARGETS["f%d" % (1 + b % 6)][0](X[b]) for b in range(D)])
+    eng = capi.Engine(K, D * C, list(range(1, 11)), [0.1] * 10, val=0, plateau_rule=False)
+    try:
+        eng.set_datasets(X, y, np.repeat(np.arange(D), C))
+        eng.init_chains_keyed(np.repeat(np.arange(D) + 1000, C), np.tile(np.arange(C), D))
+        stream = torch.cuda.current_stream()
+        eng.run(20, stream.cuda_stream)                      # warm-up: allocations, module loads
+        p0 = int(eng.get_stats()["counters"][:, capi.CNT["proposals"]].sum())
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record(stream)
+        eng.run(sweeps, stream.cuda_stream)
+        b.record(stream)
+        b.synchronize()
+        ms = a.elapsed_time(b)
+        p1 = int(eng.get_stats()["counters"][:, capi.CNT["proposals"]].sum())
+    finally:
+        eng.close()
+    return dict(datasets=D, chains=D * C, rows=n, sweeps=sweeps, device_ms=ms, proposals=p1 - p0, proposals_per_s=(p1 - p0) / (ms * 1e-3))
+
+
+def main(argv=None):
+    ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
+    ap.add_argument("--repeats", type=int, default=50)
+    ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--rows", type=int, default=100)
+    ap.add_argument("--sweeps", type=int, default=300)
+    ap.add_argument("--datasets", default="1,16,128,1024")
+    a = ap.parse_args(argv)
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_fit_many: needs a CUDA device")
+    import __graft_entry__ as g
+    g.build()
+    name, power = gpu_info()
+    out = dict(gpu=name, power_limit=power)
+    out["suite"] = bench_suite(a.repeats, a.rounds, a.rows)
+    out["engine"] = [bench_engine(int(D), a.sweeps, a.rows) for D in a.datasets.split(",")]
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
