@@ -113,6 +113,17 @@ int bsr_set_data_device(bsr_handle* h, const float* X_colmajor, const float* y, 
  * features. */
 int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, int64_t n, int32_t d,
                           const int32_t* chain_dataset);
+/* Same, for data sets of different row counts (the same d): data set b has n_rows[b] >= 1 rows, X_rowmajor holds the rows of the
+ * data sets one after another (sum(n_rows) x d, row-major) and y their values (sum(n_rows)).  The handle keeps the layout of equal
+ * row counts with n the largest row count (rows past a data set's own are zeros) and the window geometry of that n
+ * (bsr_get_window_geometry); n_datasets * d * n (rounded up to 4) below 2^32 elements, checked before any data is read.  Every chain
+ * works on its own data set's rows alone.  With rps the rows per split of the geometry, the chains of data set b end bit for bit where
+ * the chains of a handle holding only data set b end (keyed alike) when n_rows[b] <= rps and that handle runs one split -- always below
+ * 16384 rows; with n_rows[b] > rps the two agree up to the fp64 summation order of the splits.  The same refusals and the same failure
+ * behaviour as bsr_set_datasets_host, which is the case of equal row counts.  Fits learning curves, cross-validation folds or groups
+ * of different sizes in one run. */
+int bsr_set_datasets_ragged_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, const int64_t* n_rows,
+                                 int32_t d, const int32_t* chain_dataset);
 
 /* Prior initialisation of every chain: sigma ~ IG(1), per tree sigma_a, sigma_b ~ IG(1) and grow()
  * (codes/bsr_class.py:123-142, codes/funcs.py:74-119), then the initial intercept OLS (bsr_class.py:147-163). */

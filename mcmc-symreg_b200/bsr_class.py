@@ -110,24 +110,28 @@ class BSR(BaseEstimator, RegressorMixin):
             print("chains: %d  proposals: %d  accepts: %d  rank-rejects: %d" % (MM, c[:, 0].sum(), c[:, 1].sum(), c[:, 2].sum()))
         return
 
-    def fit_many(self, datasets, seeds=None):
+    def fit_many(self, datasets, seeds=None, *, ragged=False):
         """Fit this estimator to each of several data sets in one GPU run; returns one fitted ``BSR`` per data set.
 
-        ``datasets``: a sequence of (X, y) pairs of the same shape (n rows, d features).  The ``itrNum`` restarts of every data
-        set run as chains of one handle (chains never interact), so the B fits share one upload, one sequence of launches
-        and one result read.  Estimator b is identical -- ``roots_`` / ``model()``, ``betas_``, ``train_err_``,
-        ``train_err_truncated_``, ``counters_``, ``done_``, ``final_rmse_`` and every ``predict*`` -- to
+        ``datasets``: a sequence of (X, y) pairs of the same shape (n rows, d features); with ``ragged=True`` the row counts may
+        differ (a learning curve, cross-validation folds, groups of different sizes), the number of features may not.  The
+        ``itrNum`` restarts of every data set run as chains of one handle (chains never interact), so the B fits share one upload,
+        one sequence of launches and one result read.  Estimator b is identical -- ``roots_`` / ``model()``, ``betas_``,
+        ``train_err_``, ``train_err_truncated_``, ``counters_``, ``done_``, ``final_rmse_`` and every ``predict*`` -- to
         ``clone(self).set_params(seed=seeds[b]).fit(*datasets[b])``: its chains draw from Philox under the keys
         (seeds[b], 0 ... itrNum - 1) that fit gives them.  This holds whenever the window geometry of the batch equals that of
         a single fit, which it always does below 16384 rows; above, with few chains, the row-split count depends on the chain
-        count and the results agree up to the fp64 summation order of the splits.  ``n_sweeps_`` reports the sweeps of the
+        count and the results agree up to the fp64 summation order of the splits.  With ``ragged=True`` the batch takes the
+        geometry of its largest data set, and data set b is identical to its fit when its n_b rows fit in the batch's first row
+        split and its own fit runs one split (always below 16384 rows), else equal up to the fp64 summation order of the splits.
+        With equal row counts ``ragged=True`` gives the estimators ``ragged=False`` gives.  ``n_sweeps_`` reports the sweeps of the
         whole batch (the stop rules are checked for all chains together), not the count a single fit would have needed.
 
         ``seeds``: one seed per data set; None gives every data set ``self.seed``, or, when that is None, draws one seed per
         data set from numpy's global state, in order, exactly as a loop of ``fit`` calls would.  The returned estimators
         carry the parameters of ``self``."""
         data = [(_as_matrix(X), np.asarray(y, dtype=np.float64).ravel()) for X, y in datasets]
-        check_datasets(data)
+        check_datasets(data, ragged)
         B = len(data)
         seeds = dataset_seeds(self.seed, B, seeds)
         MM, K = int(self.itrNum), int(self.treeNum)
@@ -144,7 +148,10 @@ class BSR(BaseEstimator, RegressorMixin):
             try:
                 g = np.arange(lo, hi)
                 ds, ids = g // MM, g % MM
-                eng.set_datasets(np.stack([X for X, _ in data]), np.stack([y for _, y in data]), ds)
+                if ragged:
+                    eng.set_datasets_ragged([X for X, _ in data], [y for _, y in data], ds)
+                else:
+                    eng.set_datasets(np.stack([X for X, _ in data]), np.stack([y for _, y in data]), ds)
                 eng.init_chains_keyed(np.asarray(seeds, dtype=object)[ds], ids)
                 if fixed:
                     eng.run(int(self.fixed_sweeps))
@@ -294,17 +301,21 @@ class _LazyRoots:
         return dict(_pk=self._pk, _cache={})
 
 
-def check_datasets(data):
-    """``fit_many``'s data sets, as (X (n, d), y) pairs, must share n and d, and each X must agree with its y: else ValueError."""
+def check_datasets(data, ragged=False):
+    """``fit_many``'s data sets, as (X (n, d), y) pairs, must share n (unless ``ragged``) and d, and each X must agree with its y:
+    else ValueError."""
     if len(data) == 0:
         raise ValueError("fit_many: no data sets")
     n, d = data[0][0].shape
     for b, (X, y) in enumerate(data):
         if X.shape[0] != y.shape[0]:
             raise ValueError("fit_many: data set %d: train_data and train_y disagree on the number of rows" % b)
-        if X.shape != (n, d):
-            raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape"
-                             % (b, X.shape[0], X.shape[1], n, d))
+        if ragged and X.shape[1] != d:
+            raise ValueError("fit_many: data set %d has %d features, data set 0 has %d: all data sets must have the same number of features"
+                             % (b, X.shape[1], d))
+        if not ragged and X.shape != (n, d):
+            raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape%s"
+                             % (b, X.shape[0], X.shape[1], n, d, " (ragged=True accepts different row counts)" if X.shape[1] == d else ""))
 
 
 def dataset_seeds(seed, n_datasets, seeds=None):

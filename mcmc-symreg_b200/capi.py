@@ -34,6 +34,7 @@ _SIGS = {
     "bsr_set_data_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int64]),
     "bsr_set_data_device": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int64, C.c_int64]),
     "bsr_set_datasets_host": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, C.c_int32, _P]),
+    "bsr_set_datasets_ragged_host": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P]),
     "bsr_init_chains": (C.c_int, [_P, C.c_uint64]),
     "bsr_init_chains_keyed": (C.c_int, [_P, _P, _P]),
     "bsr_set_state": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_uint64]),
@@ -267,6 +268,27 @@ class Engine:
             raise ValueError("chain_dataset must hold one data set index per chain")
         _ck(self._lib.bsr_set_datasets_host(self._h, X.shape[0], _ptr(X), _ptr(y), X.shape[1], X.shape[2], _ptr(cd)))
         self.n, self.d = X.shape[1], X.shape[2]
+
+    def set_datasets_ragged(self, Xs, ys, chain_dataset):
+        """D data sets of the same number of features and any row counts: Xs a sequence of (n_b, d) arrays, ys of (n_b,) arrays; chain
+        c fits data set ``chain_dataset[c]``.  ``n`` becomes the largest row count."""
+        Xs = [np.asarray(X, dtype=np.float64) for X in Xs]
+        ys = [np.asarray(y, dtype=np.float64).ravel() for y in ys]
+        if len(Xs) == 0 or len(Xs) != len(ys):
+            raise ValueError("set_datasets_ragged: one y per X, and at least one data set")
+        if any(X.ndim != 2 or X.shape[0] != y.shape[0] for X, y in zip(Xs, ys)):
+            raise ValueError("set_datasets_ragged: every X must be (n_b, d) and its y (n_b,)")
+        d = Xs[0].shape[1]
+        if any(X.shape[1] != d for X in Xs):
+            raise ValueError("set_datasets_ragged: all data sets must have the same number of features")
+        cd = np.ascontiguousarray(chain_dataset, dtype=np.int32).ravel()
+        if cd.size != self.C:
+            raise ValueError("chain_dataset must hold one data set index per chain")
+        n_rows = np.array([X.shape[0] for X in Xs], dtype=np.int64)
+        X = np.ascontiguousarray(np.concatenate(Xs, axis=0))
+        y = np.ascontiguousarray(np.concatenate(ys))
+        _ck(self._lib.bsr_set_datasets_ragged_host(self._h, len(Xs), _ptr(X), _ptr(y), _ptr(n_rows), d, _ptr(cd)))
+        self.n, self.d = int(n_rows.max()), d
 
     def set_data_device(self, x_ptr, y_ptr, n, d, ld, n_total=0):
         self.n, self.d = int(n), int(d)

@@ -99,6 +99,7 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
   rc |= dalloc(h, &h->split_cnt, (size_t)C);
   rc |= dalloc(h, &h->d_count, 2);      // [1]: abort flag of the peer-memory exchange (k_wwait)
   rc |= dalloc(h, &h->ystats, 2);
+  rc |= dalloc(h, &h->ds_n, 1);
   if (rc) { bsr_destroy(h); return 1; }
   for (int i = 0; i < 8; ++i) cudaEventCreate(&h->ev[i]);
   if (const char* e = getenv("BSR_SEQ_PIPELINE")) h->seq_pipeline = atoi(e) != 0;
@@ -179,7 +180,7 @@ static int finish_data(bsr_handle* h) {
   if (setup_col_cache(h)) return 1;
   if (h->initialised) h->needs_refit = true;
   // y statistics over the local rows of every data set; in row-sharded mode the caller replaces them with the global values
-  k_y_stats<<<h->n_ds, 1024>>>(h->y64, h->n, h->ld, h->ystats);
+  k_y_stats<<<h->n_ds, 1024>>>(h->y64, h->ds_n, h->ld, h->ystats);
   double s[2];
   CK(cudaMemcpy(s, h->ystats, sizeof s, cudaMemcpyDeviceToHost));
   h->sum_y = s[0]; h->yy = s[1];
@@ -192,24 +193,33 @@ static void free_data(bsr_handle* h) {
   h->X32 = nullptr; h->y32 = nullptr; h->X64 = nullptr; h->y64 = nullptr;
 }
 
-// Number of data sets and the data set of every chain (nullptr: all chains on data set 0), committed once the data of the D data
-// sets is in place.  On failure the caller drops the data (free_data): no entry point then runs on chains that name data sets the
-// handle does not hold.
-static int set_chain_datasets(bsr_handle* h, int D, const int32_t* chain_dataset) {
+// Number of data sets, their row counts (nullptr: all of h->n rows) and the data set of every chain (nullptr: all chains on data set
+// 0), committed once the data of the D data sets is in place.  On failure the caller drops the data (free_data): no entry point then
+// runs on chains that name data sets the handle does not hold.
+static int set_chain_datasets(bsr_handle* h, int D, const int64_t* n_rows, const int32_t* chain_dataset) {
   if (D != h->n_ds) {
     double* ys = nullptr;
-    if (dalloc(h, &ys, 2 * (size_t)D)) return 1;
-    dfree(h, h->ystats);
-    h->ystats = ys;
+    uint32_t* dn = nullptr;
+    if (dalloc(h, &ys, 2 * (size_t)D) || dalloc(h, &dn, (size_t)D)) { dfree(h, ys); return 1; }
+    dfree(h, h->ystats); dfree(h, h->ds_n);
+    h->ystats = ys; h->ds_n = dn;
     h->n_ds = D;
   }
+  std::vector<uint32_t> dn((size_t)D, (uint32_t)h->n);
+  if (n_rows) for (int b = 0; b < D; ++b) dn[(size_t)b] = (uint32_t)n_rows[b];
+  CK(cudaMemcpy(h->ds_n, dn.data(), (size_t)D * sizeof(uint32_t), cudaMemcpyHostToDevice));
   if (chain_dataset) CK(cudaMemcpy(h->st.ds, chain_dataset, (size_t)h->st.C * sizeof(int), cudaMemcpyHostToDevice));
   else CK(cudaMemset(h->st.ds, 0, (size_t)h->st.C * sizeof(int)));
   return 0;
 }
 
-// D data sets of n rows x d features from host memory (X row-major [D][n][d], y [D][n]) into the handle's buffers.
-static int upload_host(bsr_handle* h, int D, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
+// D data sets of n_rows[b] rows x d features from host memory (X row-major, the data sets' rows one after another; y likewise) into
+// the handle's buffers: X [D][d][ld], y [D][ld] with ld the largest row count rounded up to 4, zeros past a data set's own rows.
+static int upload_host(bsr_handle* h, int D, const double* X, const double* y, const int64_t* n_rows, int32_t d, int64_t n_total) {
+  std::vector<int64_t> off((size_t)D + 1, 0);       // first row of every data set in X / y, then the total
+  int64_t n = 0;
+  for (int b = 0; b < D; ++b) { off[(size_t)b + 1] = off[(size_t)b] + n_rows[b]; n = std::max(n, n_rows[b]); }
+  const int64_t rows = off[(size_t)D];
   const bool same_shape = h->own_x32 && h->X32 != nullptr && h->n == n && h->d == d && h->n_ds == D;
   const size_t ld = (size_t)(n + 3) / 4 * 4;
   if (!same_shape) {
@@ -218,31 +228,45 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, i
     h->n = n; h->d = d; h->ld = (int64_t)ld;
     h->own_x32 = true;
     if (dalloc(h, &h->X32, D * ld * d) || dalloc(h, &h->X64, D * ld * d) || dalloc(h, &h->y32, D * ld) || dalloc(h, &h->y64, D * ld)) return 1;
-    if (h->stage) cudaFree(h->stage);
-    h->stage = nullptr;
-    CK(cudaMalloc((void**)&h->stage, (size_t)D * n * d * sizeof(double)));
   }
+  // staging: X, then y, then the row offsets
+  const size_t xs = (size_t)rows * d, bytes = (xs + (size_t)rows) * sizeof(double) + off.size() * sizeof(int64_t);
+  if (bytes > h->stage_bytes) {
+    CK(cudaDeviceSynchronize());
+    if (h->stage) cudaFree(h->stage);
+    h->stage = nullptr; h->stage_bytes = 0;
+    CK(cudaMalloc((void**)&h->stage, bytes));
+    h->stage_bytes = bytes;
+  }
+  double* ystage = h->stage + xs;
+  int64_t* d_off = reinterpret_cast<int64_t*>(ystage + rows);
   h->n_total = n_total > 0 ? n_total : n;
   // stream-ordered after any sweep still in flight on the default stream; the copies from pageable memory are synchronous
-  CK(cudaMemcpy(h->stage, X, (size_t)D * n * d * sizeof(double), cudaMemcpyHostToDevice));
-  const dim3 blocks((unsigned)std::min<int64_t>(((int64_t)n * d + 255) / 256, 148 * 16), (unsigned)D);
-  k_transpose_in<float><<<blocks, 256>>>(h->stage, h->X32, n, d, h->ld);
-  k_transpose_in<double><<<blocks, 256>>>(h->stage, h->X64, n, d, h->ld);
-  // y [D][n] -> [D][ld]: the padding rows stay the zeros of the allocation
-  CK(cudaMemcpy2D(h->y64, ld * sizeof(double), y, (size_t)n * sizeof(double), (size_t)n * sizeof(double), (size_t)D, cudaMemcpyHostToDevice));
-  k_convert<double, float><<<blocks.x, 256>>>(h->y64, h->y32, (int64_t)(D * ld));
+  CK(cudaMemcpy(h->stage, X, xs * sizeof(double), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(ystage, y, (size_t)rows * sizeof(double), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(d_off, off.data(), off.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
+  // one launch per buffer for all D data sets (blockIdx.y); y is the one-column case
+  const dim3 blocks((unsigned)std::min<int64_t>(((int64_t)ld * d + 255) / 256, 148 * 16), (unsigned)D);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(h->stage, d_off, h->X32, d, h->ld);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(h->stage, d_off, h->X64, d, h->ld);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(ystage, d_off, h->y32, 1, h->ld);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(ystage, d_off, h->y64, 1, h->ld);
   CK(cudaGetLastError());
   return 0;
 }
 
-static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total,
-                         const int32_t* chain_dataset) {
+// The checks every host upload makes before it reads any data, then the upload.  n_rows: D row counts (the caller checked them >= 1).
+static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, const double* y, const int64_t* n_rows, int32_t d,
+                         int64_t n_total, const int32_t* chain_dataset) {
   const std::string f(fn);
-  if (n < 1 || d < 1 || d > 65535) return fail(f + ": need n >= 1 and 1 <= d <= 65535");
+  if (d < 1 || d > 65535) return fail(f + ": need n >= 1 and 1 <= d <= 65535");
+  int64_t n = 0;
+  for (int b = 0; b < D; ++b) n = std::max(n, n_rows[b]);
   if ((n + 3) / 4 * 4 * (int64_t)d * D >= (int64_t)1 << 32)
-    return fail(f + ": n_datasets * d * n must stay below 2^32 elements per device (shard the rows, or fit fewer data sets per handle)");
+    return fail(f + ": n_datasets * d * n (the largest row count) must stay below 2^32 elements per device (shard the rows, or fit fewer data "
+                "sets per handle)");
   CK(cudaSetDevice(h->cfg.device));
-  if (upload_host(h, D, X, y, n, d, n_total) || set_chain_datasets(h, D, chain_dataset)) {
+  if (upload_host(h, D, X, y, n_rows, d, n_total) || set_chain_datasets(h, D, n_rows, chain_dataset)) {
     free_data(h);
     return 1;
   }
@@ -251,24 +275,47 @@ static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, 
 
 int bsr_set_data_host(bsr_handle* h, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
   if (!h || !X || !y) return fail("bsr_set_data_host: null argument");
-  return set_data_host(h, "bsr_set_data_host", 1, X, y, n, d, n_total, nullptr);
+  if (n < 1) return fail("bsr_set_data_host: need n >= 1 and 1 <= d <= 65535");
+  return set_data_host(h, "bsr_set_data_host", 1, X, y, &n, d, n_total, nullptr);
+}
+
+// the refusals of every call that loads several data sets
+static int check_datasets(bsr_handle* h, const char* fn, int32_t n_datasets, const int32_t* chain_dataset) {
+  const std::string f(fn);
+  if (n_datasets < 1 || n_datasets > 65535) return fail(f + ": n_datasets must be in [1, 65535]");
+  for (int c = 0; c < h->st.C; ++c)
+    if (chain_dataset[c] < 0 || chain_dataset[c] >= n_datasets) {
+      char msg[200];
+      snprintf(msg, sizeof msg, "%s: chain_dataset[%d] = %d is outside [0, %d)", fn, c, (int)chain_dataset[c], (int)n_datasets);
+      return fail(msg);
+    }
+  // (a row-sharded handle holds a slice of the rows of one data set: bsr_set_data_* with the global row count)
+  if (h->cfg.row_sharded) return fail(f + ": not available on row-sharded handles (use bsr_set_data_host)");
+  if (n_datasets > 1 && h->seq_pipeline)
+    return fail(f + ": several data sets need the window path of bsr_run (this handle uses the proposal-by-proposal pipeline)");
+  return 0;
 }
 
 int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X, const double* y, int64_t n, int32_t d,
                           const int32_t* chain_dataset) {
   if (!h || !X || !y || !chain_dataset) return fail("bsr_set_datasets_host: null argument");
-  if (n_datasets < 1 || n_datasets > 65535) return fail("bsr_set_datasets_host: n_datasets must be in [1, 65535]");
-  for (int c = 0; c < h->st.C; ++c)
-    if (chain_dataset[c] < 0 || chain_dataset[c] >= n_datasets) {
+  if (check_datasets(h, "bsr_set_datasets_host", n_datasets, chain_dataset)) return 1;
+  if (n < 1) return fail("bsr_set_datasets_host: need n >= 1 and 1 <= d <= 65535");
+  const std::vector<int64_t> n_rows((size_t)n_datasets, n);
+  return set_data_host(h, "bsr_set_datasets_host", n_datasets, X, y, n_rows.data(), d, 0, chain_dataset);
+}
+
+int bsr_set_datasets_ragged_host(bsr_handle* h, int32_t n_datasets, const double* X, const double* y, const int64_t* n_rows, int32_t d,
+                                 const int32_t* chain_dataset) {
+  if (!h || !X || !y || !n_rows || !chain_dataset) return fail("bsr_set_datasets_ragged_host: null argument");
+  if (check_datasets(h, "bsr_set_datasets_ragged_host", n_datasets, chain_dataset)) return 1;
+  for (int b = 0; b < n_datasets; ++b)
+    if (n_rows[b] < 1) {
       char msg[160];
-      snprintf(msg, sizeof msg, "bsr_set_datasets_host: chain_dataset[%d] = %d is outside [0, %d)", c, (int)chain_dataset[c], (int)n_datasets);
+      snprintf(msg, sizeof msg, "bsr_set_datasets_ragged_host: n_rows[%d] = %lld: every data set needs at least one row", b, (long long)n_rows[b]);
       return fail(msg);
     }
-  // (a row-sharded handle holds a slice of the rows of one data set: bsr_set_data_* with the global row count)
-  if (h->cfg.row_sharded) return fail("bsr_set_datasets_host: not available on row-sharded handles (use bsr_set_data_host)");
-  if (n_datasets > 1 && h->seq_pipeline)
-    return fail("bsr_set_datasets_host: several data sets need the window path of bsr_run (this handle uses the proposal-by-proposal pipeline)");
-  return set_data_host(h, "bsr_set_datasets_host", n_datasets, X, y, n, d, 0, chain_dataset);
+  return set_data_host(h, "bsr_set_datasets_ragged_host", n_datasets, X, y, n_rows, d, 0, chain_dataset);
 }
 
 int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n, int32_t d, int64_t ld, int64_t n_total) {
@@ -290,7 +337,7 @@ int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n
     CK(cudaDeviceSynchronize());
     return 0;
   };
-  if (upload() || set_chain_datasets(h, 1, nullptr)) {
+  if (upload() || set_chain_datasets(h, 1, nullptr, nullptr)) {
     free_data(h);
     return 1;
   }

@@ -11,11 +11,14 @@ struct bsr_handle {
   PriorTables* d_pt = nullptr;   // device copy (the kernels read the tables from global memory)
   ChainState st;
   std::vector<void*> allocs;
-  // data: n_ds data sets of the same shape, X column-major [n_ds][d][ld], y [n_ds][ld]
+  // data: n_ds data sets of d features, X column-major [n_ds][d][ld], y [n_ds][ld]; data set b holds ds_n[b] rows (n: the largest,
+  // ld: n rounded up to 4), zeros past them
   float* X32 = nullptr; double* X64 = nullptr; float* y32 = nullptr; double* y64 = nullptr;
   int n_ds = 1;
+  uint32_t* ds_n = nullptr;      // [n_ds] (device)
   bool own_x32 = false;
-  double* stage = nullptr;       // device staging of the row-major host X (bsr_set_data_host / bsr_set_datasets_host)
+  double* stage = nullptr;       // device staging of the host data and its row offsets (bsr_set_data_host / bsr_set_datasets_*host)
+  size_t stage_bytes = 0;
   void* gt_dev = nullptr; void* gt_host = nullptr; size_t gt_bytes = 0;   // gather staging of bsr_get_trees (device, pinned host)
   void* pk_head = nullptr; size_t pk_head_bytes = 0;   // packed results (bsr_pack_trees): counts / offsets / node counts / scan scratch
   void* pk_body = nullptr; size_t pk_body_bytes = 0;   //                                   lt parameter pairs, then tokens

@@ -117,11 +117,9 @@ __global__ void k_convert(const TI* in, TO* out, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = (TO)in[i];
 }
 
-// row-major float64 (n x d) -> column-major T (d x ld); blockIdx.y: data set ([D][n][d] -> [D][d][ld])
+// row-major float64 (n x d) -> column-major T (d x ld)
 template <typename TO>
 __global__ void k_transpose_in(const double* in, TO* out, int64_t n, int d, int64_t ld) {
-  in += (size_t)blockIdx.y * n * d;
-  out += (size_t)blockIdx.y * d * ld;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n * d; i += (int64_t)gridDim.x * blockDim.x) {
     int64_t row = i / d;
     int col = (int)(i % d);
@@ -129,9 +127,25 @@ __global__ void k_transpose_in(const double* in, TO* out, int64_t n, int d, int6
   }
 }
 
-// y statistics: sum(y), y'y in fp64 (one block per data set, deterministic order per launch geometry): y [D][ld] -> out2 [D][2]
-__global__ void k_y_stats(const double* y, int64_t n, int64_t ld, double* out2) {
+// The same for the data sets of a handle: data set b = blockIdx.y is rows row_off[b] .. row_off[b + 1] of the input and goes to
+// out + b * d * ld, with zeros on the rows past its own (up to ld)
+template <typename TO>
+__global__ void k_transpose_datasets_in(const double* in, const int64_t* row_off, TO* out, int d, int64_t ld) {
+  const int64_t r0 = row_off[blockIdx.y], n = row_off[blockIdx.y + 1] - r0;
+  in += (size_t)r0 * d;
+  out += (size_t)blockIdx.y * d * ld;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ld * d; i += (int64_t)gridDim.x * blockDim.x) {
+    int64_t row = i / d;
+    int col = (int)(i % d);
+    out[(int64_t)col * ld + row] = row < n ? (TO)in[i] : (TO)0;
+  }
+}
+
+// y statistics: sum(y), y'y in fp64 over the n_rows[b] rows of every data set b (one block each, deterministic order per launch
+// geometry): y [D][ld] -> out2 [D][2]
+__global__ void k_y_stats(const double* y, const uint32_t* n_rows, int64_t ld, double* out2) {
   __shared__ double s1[32], s2[32];
+  const int64_t n = n_rows[blockIdx.x];
   y += (size_t)blockIdx.x * ld;
   out2 += 2 * (size_t)blockIdx.x;
   double a = 0.0, b = 0.0;

@@ -176,7 +176,7 @@ static int ensure_window(bsr_handle* h, int S) {
 
 template <typename T, int KC, bool EXACT, bool MULTI>
 static int launch_weval_t(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc, int threads) {
-  const size_t smem = win_smem_layout<T>(h->cfg.K, ws.W, threads / 32, wc.TR).total;
+  const size_t smem = win_smem_layout<T>(h->cfg.K, ws.W, threads / 32, wc.TR, MULTI).total;
   CK(cudaFuncSetAttribute(k_weval<T, KC, EXACT, MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   {
     // leave the rest of the unified L1 / shared-memory array to L1: the interpreter's operand stack (local memory) and
@@ -314,6 +314,7 @@ static WinCtx make_wc(bsr_handle* h, long long p_start, long long p_target, uint
   for (int r = 0; r < BSR_MAX_PEERS; ++r) { wc.peer_rec[r] = nullptr; wc.peer_bad[r] = nullptr; wc.peer_lrec[r] = nullptr; }
   wc.peer_lrec[0] = h->lrec;
   wc.abort_flag = nullptr;
+  wc.ds_n = h->n_ds > 1 ? h->ds_n : nullptr;
   return wc;
 }
 

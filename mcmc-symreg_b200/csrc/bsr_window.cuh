@@ -72,6 +72,9 @@ struct WinCtx {
   // refit after (re)initialisation (k_wlive_bad, k_wlive_gram, k_wrefit): partial Grams of the live columns per split and rank
   const double* peer_lrec[BSR_MAX_PEERS];
   const int* abort_flag;     // set by k_wwait when a peer never signalled: the window is not resolved
+  // rows of every data set ([D]; n is the largest, and the geometry is that of n), nullptr on a handle of one data set (its n rows, n_total
+  // of them over all ranks).  Last member: the kernels of one data set address the members above exactly as they did without it.
+  const uint32_t* ds_n;
 };
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -282,8 +285,10 @@ struct WinSmem {
 };
 template <typename T>
 __host__ __device__ constexpr int win_live_stride(int K) { return ((K + 1) * (RowVec<T>::R / 2)) | 1; }
+// multi: k_weval of several data sets, which keeps the chain's row count beside its data set (one int more; the geometry is
+// chosen without it, see win_geometry)
 template <typename T>
-__host__ __device__ inline WinSmem win_smem_layout(int K, int W, int NW, uint32_t TR) {
+__host__ __device__ inline WinSmem win_smem_layout(int K, int W, int NW, uint32_t TR, bool multi = false) {
   WinSmem s;
   size_t o = 0;
   s.live = o; o += (size_t)(TR / RowVec<T>::R) * win_live_stride<T>(K) * sizeof(double2);
@@ -292,7 +297,7 @@ __host__ __device__ inline WinSmem win_smem_layout(int K, int W, int NW, uint32_
   s.ltok = o; o += (size_t)K * BSR_MAXN * sizeof(EvTok<T>);
   s.ptok = o; o += (size_t)NW * BSR_MAXN * sizeof(EvTok<T>);
   o = (o + 15) / 16 * 16;
-  s.lm = o; o += (size_t)(K + (K & 1) + 8) * sizeof(int);   // + three 64-bit slot masks (second pass needed / its vectors already known / column not finite), + the work counter, + the data set
+  s.lm = o; o += (size_t)(K + (K & 1) + 8 + (multi ? 1 : 0)) * sizeof(int);   // + three 64-bit slot masks (second pass needed / its vectors already known / column not finite), + the work counter, + the data set (+ its rows)
   o = (o + 15) / 16 * 16;
   s.dd = o; o += 320;                                                   // results of the duplicate search (sizeof(DedupSmem))
   s.bm = o; if (sizeof(T) == 4 && K > 5) o += (size_t)W * 8 * sizeof(unsigned);   // per slot: which of the tile's <= 256 vectors are out of range (large trees, see k_weval)
@@ -362,13 +367,13 @@ static __device__ BSR_WIDE_INLINE double2 eval_tree_wide2(const EvTok<float>* tk
 }
 
 // The K live columns and y on rows [row_lo, row_lo + tile_rows) -> shared memory (fp64).  Block-cooperative; the
-// caller synchronises before and after.  Rows >= n are written as zeros.  ds: the chain's data set (its y; the live tokens
-// were staged with its X offset).
+// caller synchronises before and after.  Rows >= n are written as zeros.  ds, n: the chain's data set (its y; the live tokens
+// were staged with its X offset) and its row count.
 // lcol (fp32 mode, k_weval only; nullptr otherwise): the cache of live columns (WinState::lcol ...).  A column whose flag is set is
 // loaded instead of interpreted -- the same fp32 values; an interpreted one is written to the cache, k_wresolve sets its flag when the
 // window is over (unless the tree was replaced or the column had an out-of-range vector: *wide_mask).
 template <typename T>
-__device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc, int c, int K, uint32_t ds, const EvTok<T>* s_ltok, const int* s_lm,
+__device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc, int c, int K, uint32_t ds, uint32_t n, const EvTok<T>* s_ltok, const int* s_lm,
                                           uint32_t row_lo, uint32_t tile_rows, double2* s_live, float* lcol = nullptr, long long lcol_ld = 0,
                                           const unsigned char* lcol_ok = nullptr, unsigned* wide_mask = nullptr) {
   constexpr int R = RowVec<T>::R, NP = R / 2;
@@ -413,8 +418,8 @@ __device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc
       for (int pl = 0; pl < NP; ++pl) {
         const uint32_t r0 = row_lo + q * R + 2 * pl;
         double2 o;
-        o.x = (r0 < wc.n) ? d[2 * pl] : 0.0;
-        o.y = (r0 + 1 < wc.n) ? d[2 * pl + 1] : 0.0;
+        o.x = (r0 < n) ? d[2 * pl] : 0.0;
+        o.y = (r0 + 1 < n) ? d[2 * pl + 1] : 0.0;
         s_live[q * LS + j * NP + pl] = o;
       }
     }
@@ -426,8 +431,8 @@ __device__ __forceinline__ void live_tile(const ChainState& st, const WinCtx& wc
     const uint32_t r0 = row_lo + q2 * 2;
     const double2 yv = *reinterpret_cast<const double2*>(wc.y64 + (size_t)ds * wc.ld + r0);
     double2 d;
-    d.x = (r0 < wc.n) ? yv.x : 0.0;
-    d.y = (r0 + 1 < wc.n) ? yv.y : 0.0;
+    d.x = (r0 < n) ? yv.x : 0.0;
+    d.y = (r0 + 1 < n) ? yv.y : 0.0;
     s_live[(NP == 2 ? (q2 >> 1) : q2) * LS + K * NP + (NP == 2 ? (q2 & 1) : 0)] = d;
   }
 }
@@ -767,16 +772,20 @@ static __device__ BSR_WIDE_INLINE void careful_tile(const uint32_t* __restrict__
 // MULTI: the handle holds several data sets and every chain reads its own (st.ds).  The instances of one data set (MULTI = false)
 // have no data-set term at all: whatever the term is written as, ptxas allocates the 80-register tile loop differently for it, with
 // more spills in some instances (DESIGN.md section 5), and a handle of one data set must not pay for that.
+// The data sets of a MULTI handle may differ in row count (wc.ds_n): the chain's rows end at its own n, and a (chain, split) block
+// whose split starts at or past it has nothing to do -- k_wresolve reads only the splits that hold rows of the chain's data set.
 template <typename T, int KC, bool EXACT, bool MULTI>
 __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 : (KC <= 5 ? 3 : 2))) k_weval(ChainState st, WinState ws, WinCtx wc) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int c = wc.c0 + blockIdx.x;
   if (st.done[c] || ws.pos[c] >= wc.p_target) return;
+  const uint32_t n_c = MULTI ? wc.ds_n[st.ds[c]] : wc.n;
+  if (MULTI && blockIdx.y * wc.rows_per_split >= n_c) return;
   const int K = EXACT ? KC : st.K;
   constexpr int R = RowVec<T>::R;
   const int W = ws.W, RECN = K + 4;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, NW = blockDim.x >> 5;
-  const WinSmem L = win_smem_layout<T>(K, W, NW, wc.TR);
+  const WinSmem L = win_smem_layout<T>(K, W, NW, wc.TR, MULTI);
   double2* s_live = reinterpret_cast<double2*>(smem_raw + L.live);
   double* s_acc = reinterpret_cast<double*>(smem_raw + L.acc);
   EvTok<T>* s_ltok = reinterpret_cast<EvTok<T>*>(smem_raw + L.ltok);
@@ -786,13 +795,14 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
   unsigned long long* s_dead = s_flag + 1;                                                  // slots whose column is not finite even in double range
   unsigned long long* s_pre = s_dead + 1;                                                   // slots of this tile whose out-of-range vectors the first pass listed (s_bm)
   int* s_next = reinterpret_cast<int*>(s_pre + 1);
-  int* s_ds = s_next + 1;                                                                   // (MULTI) the chain's data set: read where it is
-                                                                                            // used, so that the tile loop holds no register for it
+  int* s_ds = s_next + 1;                                                                   // (MULTI) the chain's data set and its row count: read
+  uint32_t* s_n = reinterpret_cast<uint32_t*>(s_ds + 1);                                    // where they are used, so that the tile loop holds no
+                                                                                            // register for them
   unsigned* s_bm = reinterpret_cast<unsigned*>(smem_raw + L.bm);
   const T* X = (sizeof(T) == 4) ? reinterpret_cast<const T*>(wc.X32) : reinterpret_cast<const T*>(wc.X64);
   DedupSmem& dd = *reinterpret_cast<DedupSmem*>(smem_raw + L.dd);
   const unsigned char* s_rep = dd.rep;
-  if (threadIdx.x == 0) { *s_flag = 0ull; *s_dead = 0ull; if (MULTI) *s_ds = st.ds[c]; }
+  if (threadIdx.x == 0) { *s_flag = 0ull; *s_dead = 0ull; if (MULTI) { *s_ds = st.ds[c]; *s_n = n_c; } }
   const int head = ws.chead[c];                   // ring index of the chain's last window (still valid for the live state), or -1
   const int nprev = (head >= 0 && wc.dedup >= 2) ? (int)ws.cvalid[c] : 0;
   const WinState wv = win_half(ws, head >= 0 ? ((head + 1) % ws.R) : 0, K);     // this window's slots (win_parity)
@@ -819,7 +829,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
   const unsigned char* s_order = dd.order;
 
   const uint32_t r_lo = blockIdx.y * wc.rows_per_split;
-  const uint32_t r_hi = min(wc.n, r_lo + wc.rows_per_split);
+  const uint32_t r_hi = min(n_c, r_lo + wc.rows_per_split);
   unsigned long long wide_mask = 0ull;             // slots that needed the second pass on some tile of this block (block-uniform)
   for (uint32_t t_lo = r_lo; t_lo < r_hi; t_lo += wc.TR) {
     const uint32_t tile_rows = min(wc.TR, r_hi - t_lo);
@@ -828,8 +838,8 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
     if (n_eval == 0) continue;                     // every tree of this window has its record already (block-uniform)
     // (the cache of live columns and the checked first pass belong to the K > 5 kernels: the 80-register kernels of K <= 5 pay for the
     // extra paths in spills -- measured: C4 -3 %, C5 -7 % -- what the cache gives their 4-node trees)
-    if (KC > 5) live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, s_ltok, s_lm, t_lo, tile_rows, s_live, ws.lcol, ws.lcol_ld, ws.lcol_ok, ws.lcol_wide);
-    else live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, s_ltok, s_lm, t_lo, tile_rows, s_live);
+    if (KC > 5) live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, MULTI ? *s_n : wc.n, s_ltok, s_lm, t_lo, tile_rows, s_live, ws.lcol, ws.lcol_ld, ws.lcol_ok, ws.lcol_wide);
+    else live_tile<T>(st, wc, c, K, MULTI ? (uint32_t)*s_ds : 0u, MULTI ? *s_n : wc.n, s_ltok, s_lm, t_lo, tile_rows, s_live);
     __syncthreads();
     const uint32_t tv = (tile_rows + R - 1) / R;
     const unsigned long long dead = *s_dead;      // columns found non-finite on an earlier tile: their record is settled (reject)
@@ -854,7 +864,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
       constexpr int NV = (sizeof(T) == 4) ? BSR_WEVAL_NV : 1;
       constexpr int NP = R / 2;
       const int LS = win_live_stride<T>(K);
-      const bool tail_tile = t_lo + tv * R > wc.n;      // only the last vector of the last tile can be ragged
+      const bool tail_tile = t_lo + tv * R > (MULTI ? *s_n : wc.n);      // only the last vector of the last tile can be ragged
       a.zero();
       // Large trees (fp32 mode): the pass tells finite from out-of-range vectors as it goes (4 FFMA per vector: nothing beside a
       // 12+-node tree, 5 % beside the average 4-node tree of C2) -- it keeps the sums of the finite vectors and leaves a bitmap of the
@@ -877,7 +887,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
 #pragma unroll
             for (int r = 0; r < 4; ++r) vf[r] = (float)v[u][r < R ? r : 0];
             const bool fin = vec_finite(vf);
-            if (valid && fin) wacc_rows<T, KC, NP, true>(a, K, v[u], s_live + (size_t)(q + 32 * u) * LS, rowoff[u], wc.n);
+            if (valid && fin) wacc_rows<T, KC, NP, true>(a, K, v[u], s_live + (size_t)(q + 32 * u) * LS, rowoff[u], MULTI ? *s_n : wc.n);
             const unsigned bal = __ballot_sync(0xffffffffu, valid && !fin);
             if (lane == 0) s_bm[i * 8 + (q0 >> 5) + u] = bal;
             anyb |= bal;
@@ -900,7 +910,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
 #pragma unroll
         for (int u = 0; u < NV; ++u) {
           if (u == 0 || q + 32 * u < tv) {
-            if (tail_tile && rowoff[u] + R > wc.n) wacc_rows<T, KC, NP, true>(a, K, v[u], lv + 32 * u * LS, rowoff[u], wc.n);
+            if (tail_tile && rowoff[u] + R > (MULTI ? *s_n : wc.n)) wacc_rows<T, KC, NP, true>(a, K, v[u], lv + 32 * u * LS, rowoff[u], MULTI ? *s_n : wc.n);
             else wacc_rows<T, KC, NP, false>(a, K, v[u], lv + 32 * u * LS, rowoff[u], wc.n);
           }
         }
@@ -934,7 +944,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS, (KC <= 3 ? BSR_WEVAL_MINB3 
           const size_t wi = (size_t)c * W + i;
           careful_tile<KC>(wv.tok + wi * BSR_MAXN, wv.pa + wi * BSR_MAXN, wv.pb + wi * BSR_MAXN, wv.nn[wi], wc.X32, wc.X64,
                            MULTI ? (uint32_t)*s_ds * wc.ds_stride : 0u, wc.ld,
-                           wc.n, K, i, t_lo, tile_rows,
+                           MULTI ? *s_n : wc.n, K, i, t_lo, tile_rows,
                            s_live, s_tok0, s_part, s_acc, s_dead, (KC > 5 && ((pre >> i) & 1ull)) ? s_bm + i * 8 : nullptr);
         }
         wide_mask |= tmask;
@@ -983,8 +993,9 @@ static __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_bad(ChainSta
   __shared__ int s_bad;
   const int c = wc.c0 + blockIdx.x;
   const int K = st.K;
+  const uint32_t n = wc.ds_n != nullptr ? wc.ds_n[st.ds[c]] : wc.n;
   const uint32_t r_lo = blockIdx.y * wc.rows_per_split;
-  const uint32_t r_hi = min(wc.n, r_lo + wc.rows_per_split);
+  const uint32_t r_hi = min(n, r_lo + wc.rows_per_split);
   const uint32_t xbase = (uint32_t)st.ds[c] * wc.ds_stride;
   for (int j = 0; j < K; ++j) {
     const int g = c * K + j;
@@ -1000,7 +1011,7 @@ static __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_bad(ChainSta
       float v[4];
       eval_tree_rows<float, 4>(s_tok, m, wc.X32, row0, v);
 #pragma unroll
-      for (int r = 0; r < 4; ++r) bad = bad || (row0 + r < wc.n && !(fabsf(v[r]) <= FLT_MAX));
+      for (int r = 0; r < 4; ++r) bad = bad || (row0 + r < n && !(fabsf(v[r]) <= FLT_MAX));
     }
     if (bad) s_bad = 1;
     __syncthreads();
@@ -1042,10 +1053,14 @@ static __global__ void k_wrefit(ChainState st, WinCtx wc, int S, int c0, int cn)
   const int sgn = sg_size(K);
   double* sg = st.sg + (size_t)c * sgn;
   const int n_src = wc.n_peers > 0 ? wc.n_peers : 1;
+  // several data sets: the chain's own rows and the splits that hold them; one data set: all rows of all ranks, every split
+  const int ds = st.ds[c];
+  const double n_rows = wc.ds_n != nullptr ? (double)wc.ds_n[ds] : wc.n_total;
+  const int S_c = wc.ds_n != nullptr ? (int)((wc.ds_n[ds] + wc.rows_per_split - 1) / wc.rows_per_split) : S;
   for (int e = 0; e < sgn; ++e) {
     double v = 0.0;
     for (int pr = 0; pr < n_src; ++pr)
-      for (int sp = 0; sp < S; ++sp) {
+      for (int sp = 0; sp < S_c; ++sp) {
         const double x = wc.peer_lrec[pr][((size_t)c * S + sp) * sgn + e];
         v = (e < sgn - K) ? v + x : (v > x ? v : x);
       }
@@ -1059,9 +1074,9 @@ static __global__ void k_wrefit(ChainState st, WinCtx wc, int S, int c0, int cn)
   int il[BSR_MAXK];
   double bl[BSR_LDA];
   for (int j = 0; j < K; ++j) il[j] = j;
-  const double* ys = wc.ystats + 2 * (size_t)st.ds[c];
-  st.sse[c] = ridge_sse<BSR_LDA, false>(gl, il, K, wc.n_total, ys[0], ys[1], bl);
-  (void)ridge_sse<BSR_LDA, true>(gl, il, K, wc.n_total, ys[0], ys[1], bl);
+  const double* ys = wc.ystats + 2 * (size_t)ds;
+  st.sse[c] = ridge_sse<BSR_LDA, false>(gl, il, K, n_rows, ys[0], ys[1], bl);
+  (void)ridge_sse<BSR_LDA, true>(gl, il, K, n_rows, ys[0], ys[1], bl);
   for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = bl[j];
 }
 
@@ -1080,6 +1095,7 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
   EvTok<T>* s_ltok = reinterpret_cast<EvTok<T>*>(smem_raw + L.ltok);
   int* s_lm = reinterpret_cast<int*>(smem_raw + L.lm);
   const uint32_t ds = (uint32_t)st.ds[c];
+  const uint32_t n = wc.ds_n != nullptr ? wc.ds_n[ds] : wc.n;
   for (int j = 0; j < K; ++j) {
     const int g = c * K + j;
     const int w = st.which[g];
@@ -1095,11 +1111,11 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
   for (int j = 0; j < KC; ++j) { by[j] = 0.0; cs[j] = 0.0; mx[j] = 0.0; }
   const int LS = win_live_stride<T>(K);
   const uint32_t r_lo = blockIdx.y * wc.rows_per_split;
-  const uint32_t r_hi = min(wc.n, r_lo + wc.rows_per_split);
+  const uint32_t r_hi = min(n, r_lo + wc.rows_per_split);
   for (uint32_t t_lo = r_lo; t_lo < r_hi; t_lo += wc.TR) {
     const uint32_t tile_rows = min(wc.TR, r_hi - t_lo);
     __syncthreads();
-    live_tile<T>(st, wc, c, K, ds, s_ltok, s_lm, t_lo, tile_rows, s_live);
+    live_tile<T>(st, wc, c, K, ds, n, s_ltok, s_lm, t_lo, tile_rows, s_live);
     __syncthreads();
     const uint32_t tv = (tile_rows + R - 1) / R;
 #pragma unroll 1
@@ -1164,7 +1180,9 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
 #ifndef BSR_WRES_MINB
 #define BSR_WRES_MINB 4
 #endif
-// MULTI: as for k_weval -- the chain's sum(y), y'y come from its data set's entry of wc.ystats, else from wc.sum_y, wc.yy.
+// MULTI: as for k_weval -- the chain's sum(y), y'y come from its data set's entry of wc.ystats, else from wc.sum_y, wc.yy; its row
+// count from wc.ds_n (else wc.n_total, wc.n_local: a handle of several data sets is never row-sharded, so the two are one number),
+// and its records from the splits that hold its rows.
 template <int KT, bool MULTI>
 __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(ChainState st, WinState ws, WinCtx wc) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1219,6 +1237,7 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
   dg.pivot_min = nan(""); dg.sv_ratio = -1.0; dg.path = 0;
   const double sigma = st.sigma[c];
   const double sse_old = st.sse[c];
+  const uint32_t n_c = MULTI ? wc.ds_n[st.ds[c]] : 0u;     // (MULTI only)
   int msum = 0;
   for (int j = 0; j < K; ++j) msum += st.nn[st.which[c * K + j]][c * K + j];
   const int m_old_k = st.nn[st.which[c * K + k]][c * K + k];
@@ -1244,7 +1263,7 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
     for (int pr = 0; pr < n_src; ++pr) {
       const double* base = wc.n_peers > 0 ? wc.peer_rec[pr] : wv.rec;
 #pragma unroll 1
-      for (int s = 0; s < ws.S; ++s) {
+      for (int s = 0; s < (MULTI ? (int)((n_c + wc.rows_per_split - 1) / wc.rows_per_split) : ws.S); ++s) {
         const double* src = base + (((size_t)c * ws.S + s) * W + sl) * RECN;
 #pragma unroll
         for (int q = 0; q < RECN; ++q) {
@@ -1265,14 +1284,14 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
     double beta[BSR_LDA];
     bool finite_cols = true;
     for (int j = 0; j < K; ++j) { idx[j] = (j == k) ? K : j; finite_cols = finite_cols && (gv.mx(idx[j]) <= DBL_MAX); }
-    if (!finite_cols || rank_deficient<LD>(gv, idx, K, wc.n_total, wc.pivot_tol, dg)) {
+    if (!finite_cols || rank_deficient<LD>(gv, idx, K, MULTI ? (double)n_c : wc.n_total, wc.pivot_tol, dg)) {
       rank_rej = true;                                                         // funcs.py:1226-1228: no accept draw
     } else {
-      sse_new = MULTI ? ridge_sse<LD, false>(gv, idx, K, wc.n_total, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
+      sse_new = MULTI ? ridge_sse<LD, false>(gv, idx, K, (double)n_c, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
                       : ridge_sse<LD, false>(gv, idx, K, wc.n_total, wc.sum_y, wc.yy, beta);
       const double ns = pi.new_sigma;
-      const double yll_new = -sse_new / (2 * ns * ns) - 0.5 * wc.n_total * log(2 * 3.141592653589793 * ns * ns);
-      const double yll_old = -sse_old / (2 * sigma * sigma) - 0.5 * wc.n_total * log(2 * 3.141592653589793 * sigma * sigma);
+      const double yll_new = -sse_new / (2 * ns * ns) - 0.5 * (MULTI ? (double)n_c : wc.n_total) * log(2 * 3.141592653589793 * ns * ns);
+      const double yll_old = -sse_old / (2 * sigma * sigma) - 0.5 * (MULTI ? (double)n_c : wc.n_total) * log(2 * 3.141592653589793 * sigma * sigma);
       const double qr = pi.Qinv / pi.Q;
       logR = (yll_new - yll_old) + (pi.fs_old - prop_fs_new(pi)) + log(qr > 1e-5 ? qr : 1e-5);
       if (pi.change != CH_NONE)
@@ -1371,8 +1390,8 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
   long long* cnt = st.counters + (size_t)c * BSR_N_COUNTERS;
   if (lane == 0) {
     if (half == 0) ev_exec += msum;                 // the live columns, once per window
-    atomicAdd(reinterpret_cast<unsigned long long*>(cnt + BSR_CNT_NODE_EVALS_REF), (unsigned long long)(ev_ref * (long long)wc.n_local));
-    atomicAdd(reinterpret_cast<unsigned long long*>(cnt + BSR_CNT_NODE_EVALS_EXEC), (unsigned long long)(ev_exec * (long long)wc.n_local));
+    atomicAdd(reinterpret_cast<unsigned long long*>(cnt + BSR_CNT_NODE_EVALS_REF), (unsigned long long)(ev_ref * (MULTI ? (long long)n_c : (long long)wc.n_local)));
+    atomicAdd(reinterpret_cast<unsigned long long*>(cnt + BSR_CNT_NODE_EVALS_EXEC), (unsigned long long)(ev_exec * (MULTI ? (long long)n_c : (long long)wc.n_local)));
   }
 
   // everything else is written by the warp that holds the accepting slot (or by the chain's first warp)
@@ -1406,10 +1425,10 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
       store_live_gram(gv, cur, K, st.sg + (size_t)c * sgn);
       // intercept refit + RMSE (bsr_class.py:211-233)
       double beta[BSR_LDA];
-      const double sse_i = MULTI ? ridge_sse<LD, true>(gv, cur, K, wc.n_total, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
+      const double sse_i = MULTI ? ridge_sse<LD, true>(gv, cur, K, (double)n_c, wc.ystats[2 * (size_t)st.ds[c]], wc.ystats[2 * (size_t)st.ds[c] + 1], beta)
                                  : ridge_sse<LD, true>(gv, cur, K, wc.n_total, wc.sum_y, wc.yy, beta);
       for (int j = 0; j <= K; ++j) st.beta[(size_t)c * (K + 1) + j] = beta[j];
-      const double rmse = sqrt(sse_i / wc.n_total);
+      const double rmse = sqrt(sse_i / (MULTI ? (double)n_c : wc.n_total));
       int nerr = st.nerr[c];
       double* e = st.err + (size_t)c * st.err_cap;
       if (nerr < st.err_cap) e[nerr] = rmse;

@@ -80,33 +80,47 @@ def run_experiment(func="sim", K=3, MM=50, n_train=100, n_test=30, val=100, seed
     return out, est, data
 
 
+def suite_jobs(funcs, repeats, n_train=100, seed=0):
+    """The data sets of ``run_suite`` as (function, n_train, repeat, seed), function by function, then training size (``n_train``: one
+    size or a sequence of sizes), then repeat.  Repeat r draws its data and its chains from seed + r at every size, so the training
+    sets of a learning curve share their draws."""
+    sizes = [int(n_train)] if np.isscalar(n_train) else [int(n) for n in n_train]
+    return [(f, n, r, seed + r) for f in funcs for n in sizes for r in range(repeats)]
+
+
 def run_suite(funcs=("f1", "f2", "f3", "f4", "f5", "f6"), repeats=1, batched=False, **kw):
     """The whole benchmark suite (the paper's Table 1 recipe: every function, ``repeats`` independent data sets).
 
-    batched=True fits all (function, repeat) data sets in one GPU run (``BSR.fit_many``) with the seeds the loop uses; the rows
-    are the loop's rows, except that ``fit_seconds`` is the batch's wall clock (fit and summaries) divided by the number of data
-    sets, and ``batch_seconds`` is that wall clock."""
+    ``n_train`` may be a sequence of training sizes: the suite then runs every function at every size (a learning curve), and every
+    row carries its ``n_train``.  batched=True fits all data sets in one GPU run (``BSR.fit_many``, ``ragged=True`` for several
+    sizes) with the seeds the loop uses; the rows are the loop's rows, except that ``fit_seconds`` is the batch's wall clock (fit and
+    summaries) divided by the number of data sets, and ``batch_seconds`` is that wall clock."""
     rows = []
     seed0 = kw.pop("seed", 0)
+    n_train = kw.pop("n_train", 100)
+    grid = not np.isscalar(n_train)
+    jobs = suite_jobs(funcs, repeats, n_train, seed0)
     if not batched:
-        for f in funcs:
-            for r in range(repeats):
-                out, _, _ = run_experiment(f, seed=seed0 + r, **kw)
-                out["repeat"] = r
-                rows.append(out)
+        for f, n, r, s in jobs:
+            out, _, _ = run_experiment(f, n_train=n, seed=s, **kw)
+            if grid:
+                out["n_train"] = n
+            out["repeat"] = r
+            rows.append(out)
         return rows
     from .bsr_class import BSR
-    K, MM, n_train, n_test, val = kw.pop("K", 3), kw.pop("MM", 50), kw.pop("n_train", 100), kw.pop("n_test", 30), kw.pop("val", 100)
+    K, MM, n_test, val = kw.pop("K", 3), kw.pop("MM", 50), kw.pop("n_test", 30), kw.pop("val", 100)
     data_seed = kw.pop("data_seed", None)
-    jobs = [(f, r) for f in funcs for r in range(repeats)]
-    data = [make_dataset(f, n_train, n_test, seed=seed0 + r if data_seed is None else data_seed) for f, r in jobs]
+    data = [make_dataset(f, n, n_test, seed=s if data_seed is None else data_seed) for f, n, _, s in jobs]
     t0 = time.perf_counter()
-    fits = BSR(K, MM, val=val, **kw).fit_many([(d["X"], d["y"]) for d in data], seeds=[seed0 + r for _, r in jobs])
+    fits = BSR(K, MM, val=val, **kw).fit_many([(d["X"], d["y"]) for d in data], seeds=[s for _, _, _, s in jobs], ragged=grid)
     rows = [summarize(est, d) for est, d in zip(fits, data)]
     batch = time.perf_counter() - t0
-    for o, (_, r) in zip(rows, jobs):
+    for o, (_, n, r, _) in zip(rows, jobs):
         o["fit_seconds"] = batch / len(jobs)
         o["batch_seconds"] = batch
+        if grid:
+            o["n_train"] = n
         o["repeat"] = r
     return rows
 
@@ -119,19 +133,25 @@ def format_row(o):
              o["complexity_last"], o["complexity_best"], o["complexity_mean"], 100 * o["accept_rate"], o["fit_seconds"]))
 
 
+def _sizes(text):
+    """--n-train: one size (an int), or a comma list of sizes (a tuple)"""
+    parts = [int(v) for v in text.split(",") if v.strip()]
+    return tuple(parts) if "," in text else parts[0]
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="BSR benchmark-function experiments on the GPU (codes/simulations.py recipe)")
     ap.add_argument("--func", default="sim", help="one of %s, or 'all'" % ", ".join(sorted(TARGETS)))
     ap.add_argument("--K", type=int, default=3)
     ap.add_argument("--MM", type=int, default=50, help="restarts (chains on the GPU)")
-    ap.add_argument("--n-train", type=int, default=100)
+    ap.add_argument("--n-train", type=_sizes, default=100, help="training rows, or a comma list of sizes (a learning curve: 30,100,300)")
     ap.add_argument("--n-test", type=int, default=30)
     ap.add_argument("--val", type=int, default=100)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--repeats", type=int, default=1)
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp64"])
     ap.add_argument("--json", action="store_true", help="one JSON object per experiment instead of the table")
-    ap.add_argument("--batched", action="store_true", help="fit all (function, repeat) data sets in one GPU run (BSR.fit_many)")
+    ap.add_argument("--batched", action="store_true", help="fit all (function, size, repeat) data sets in one GPU run (BSR.fit_many)")
     a = ap.parse_args(argv)
     funcs = ("f1", "f2", "f3", "f4", "f5", "f6") if a.func == "all" else (a.func,)
     rows = run_suite(funcs, a.repeats, batched=a.batched, K=a.K, MM=a.MM, n_train=a.n_train, n_test=a.n_test, val=a.val, seed=a.seed,

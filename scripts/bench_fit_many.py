@@ -3,9 +3,12 @@
 1. The suite of the paper's Table 1 at the reference's own size: f1 ... f6 x R repeats, BSR(3, 50, val=100) on n = 100 rows.
    Wall clock of the loop of BSR.fit calls against one BSR.fit_many over the same data sets and seeds, alternated, each timing
    ending in a device synchronise; the two must give equal results (checked in the same run).
-2. Engine throughput: D data sets x 50 chains on n = 100 rows, fixed sweeps, device-timed (CUDA events) proposals per second.
+   With several sizes (--rows 30,100,300,1000) the suite is f1 ... f6 x those sizes x R repeats, and fit_many runs with ragged=True.
+2. Engine throughput: D data sets x 50 chains on n = 100 rows (the first of --rows), fixed sweeps, device-timed (CUDA events)
+   proposals per second.  With several sizes, one more line: the largest D with the data sets cycling through the sizes (a ragged
+   batch, every chain on its own rows) against the same chains on data sets of the largest size.
 
-    python scripts/bench_fit_many.py [--repeats 50] [--rounds 3] [--sweeps 300] [--datasets 1,16,128,1024]
+    python scripts/bench_fit_many.py [--repeats 50] [--rounds 3] [--sweeps 300] [--datasets 1,16,128,1024] [--rows 100 | 30,100,300,1000]
 """
 import argparse
 import json
@@ -31,23 +34,24 @@ def gpu_info():
     return name, power
 
 
-def suite_data(repeats, n):
-    from mcmc_symreg_b200.experiments import make_dataset
-    jobs = [(f, r) for f in ("f1", "f2", "f3", "f4", "f5", "f6") for r in range(repeats)]
-    return jobs, [make_dataset(f, n, 30, seed=r) for f, r in jobs]
+def suite_data(repeats, sizes):
+    from mcmc_symreg_b200.experiments import make_dataset, suite_jobs
+    jobs = suite_jobs(("f1", "f2", "f3", "f4", "f5", "f6"), repeats, sizes[0] if len(sizes) == 1 else sizes)
+    return jobs, [make_dataset(f, n, 30, seed=s) for f, n, _, s in jobs]
 
 
 def fingerprint(est):
     return (est.model(), [b.ravel().tolist() for b in est.betas_], est.train_err_, est.counters_.tolist(), est.done_.tolist())
 
 
-def bench_suite(repeats, rounds, n):
+def bench_suite(repeats, rounds, sizes):
     import torch
     from sklearn.base import clone
     from mcmc_symreg_b200 import BSR
-    jobs, data = suite_data(repeats, n)
+    jobs, data = suite_data(repeats, sizes)
+    ragged = len(sizes) > 1
     est = BSR(3, 50, val=100)
-    seeds = [r for _, r in jobs]
+    seeds = [s for _, _, _, s in jobs]
     pairs = [(d["X"], d["y"]) for d in data]
 
     def loop():
@@ -60,7 +64,7 @@ def bench_suite(repeats, rounds, n):
         return out
 
     def batch():
-        out = est.fit_many(pairs, seeds=seeds)
+        out = est.fit_many(pairs, seeds=seeds, ragged=ragged)
         torch.cuda.synchronize()
         return out
 
@@ -71,21 +75,26 @@ def bench_suite(repeats, rounds, n):
         t0 = time.perf_counter(); b = batch(); t_batch.append(time.perf_counter() - t0)
         equal = equal and all(fingerprint(x) == fingerprint(y) for x, y in zip(a, b))
     assert equal, "fit_many and the loop of fits disagree"
-    return dict(datasets=len(jobs), chains_per_fit=50, rows=n, loop_seconds=t_loop, fit_many_seconds=t_batch,
+    return dict(datasets=len(jobs), chains_per_fit=50, rows=sizes[0] if len(sizes) == 1 else list(sizes), ragged=ragged, loop_seconds=t_loop, fit_many_seconds=t_batch,
                 loop_ms_per_fit=1e3 * float(np.median(t_loop)) / len(jobs), fit_many_ms_per_fit=1e3 * float(np.median(t_batch)) / len(jobs),
                 speedup_median=float(np.median(t_loop) / np.median(t_batch)), results_equal=equal)
 
 
 def bench_engine(D, sweeps, n, C=50, K=3):
+    """n: the rows of every data set, or a sequence the data sets cycle through (a ragged batch)"""
     import torch
     from mcmc_symreg_b200 import capi
     from mcmc_symreg_b200.experiments import TARGETS
     rng = np.random.default_rng(D)
-    X = rng.uniform(-3, 3, (D, n, 2))
-    y = np.stack([TARGETS["f%d" % (1 + b % 6)][0](X[b]) for b in range(D)])
+    sizes = [n] * D if np.isscalar(n) else [n[b % len(n)] for b in range(D)]
+    X = [rng.uniform(-3, 3, (sizes[b], 2)) for b in range(D)]
+    y = [TARGETS["f%d" % (1 + b % 6)][0](X[b]) for b in range(D)]
     eng = capi.Engine(K, D * C, list(range(1, 11)), [0.1] * 10, val=0, plateau_rule=False)
     try:
-        eng.set_datasets(X, y, np.repeat(np.arange(D), C))
+        if np.isscalar(n):
+            eng.set_datasets(np.stack(X), np.stack(y), np.repeat(np.arange(D), C))
+        else:
+            eng.set_datasets_ragged(X, y, np.repeat(np.arange(D), C))
         eng.init_chains_keyed(np.repeat(np.arange(D) + 1000, C), np.tile(np.arange(C), D))
         stream = torch.cuda.current_stream()
         eng.run(20, stream.cuda_stream)                      # warm-up: allocations, module loads
@@ -99,14 +108,14 @@ def bench_engine(D, sweeps, n, C=50, K=3):
         p1 = int(eng.get_stats()["counters"][:, capi.CNT["proposals"]].sum())
     finally:
         eng.close()
-    return dict(datasets=D, chains=D * C, rows=n, sweeps=sweeps, device_ms=ms, proposals=p1 - p0, proposals_per_s=(p1 - p0) / (ms * 1e-3))
+    return dict(datasets=D, chains=D * C, rows=n if np.isscalar(n) else list(n), sweeps=sweeps, device_ms=ms, proposals=p1 - p0, proposals_per_s=(p1 - p0) / (ms * 1e-3))
 
 
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("--repeats", type=int, default=50)
     ap.add_argument("--rounds", type=int, default=3)
-    ap.add_argument("--rows", type=int, default=100)
+    ap.add_argument("--rows", default="100", help="rows per data set, or a comma list of sizes (30,100,300,1000)")
     ap.add_argument("--sweeps", type=int, default=300)
     ap.add_argument("--datasets", default="1,16,128,1024")
     a = ap.parse_args(argv)
@@ -117,8 +126,14 @@ def main(argv=None):
     g.build()
     name, power = gpu_info()
     out = dict(gpu=name, power_limit=power)
-    out["suite"] = bench_suite(a.repeats, a.rounds, a.rows)
-    out["engine"] = [bench_engine(int(D), a.sweeps, a.rows) for D in a.datasets.split(",")]
+    sizes = [int(v) for v in a.rows.split(",")]
+    Ds = [int(D) for D in a.datasets.split(",")]
+    out["suite"] = bench_suite(a.repeats, a.rounds, sizes)
+    out["engine"] = [bench_engine(D, a.sweeps, sizes[0]) for D in Ds]
+    if len(sizes) > 1:
+        # the same chains on the ragged batch and on data sets of the largest size: what rows a chain does not hold cost nothing
+        r, p = bench_engine(max(Ds), a.sweeps, sizes), bench_engine(max(Ds), a.sweeps, max(sizes))
+        out["engine_ragged"] = dict(ragged=r, padded=p, throughput_ratio=r["proposals_per_s"] / p["proposals_per_s"])
     print(json.dumps(out))
 
 
