@@ -260,6 +260,24 @@ int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, 
                      const double* beta, const double* X_rowmajor, int64_t n_test, int32_t d, int32_t reduce, double* out,
                      int32_t* n_used);
 
+/* Many models on many test sets in one call -- the fits of BSR.fit_many, each on its own test set.
+ * Models, in the packed layout of bsr_read_packed: nn [M][K] node counts; tok the n_tok tokens of tree after tree (tree m * K + k
+ * holds nn[m][k]); ab [n_lt][2] the (a, b) pairs of the lt nodes in node order; beta [M][K+1].
+ * Test sets: X_rowmajor holds the rows of S sets of d features one after another, set s is rows set_off[s] .. set_off[s+1].
+ * Groups: group g evaluates the models grp_models[grp_off[g] .. grp_off[g+1]) on set grp_set[g].
+ * out holds the groups' blocks in group order: [n_models_g][n_rows_s] predictions, or, when grp_reduce[g] != 0, [2][n_rows_s]: the
+ * mean over the group's models and their standard deviation, reduced on the device in model order with the arithmetic of
+ * bsr_predict_many.  n_used[g] is the smallest number of models any row of group g used (its model count without reduce).
+ * Every value equals what bsr_predict_many returns for the same models on the same set.  Refused before anything is read on the
+ * device: null pointers, K outside 1 .. BSR_MAX_TREES, a tree of 0 or more than 64 nodes or whose tokens are not a pre-order tree,
+ * node counts that do not cover tok, lt nodes that do not match n_lt, a leaf feature >= d, set_off or grp_off that do not start at
+ * 0 or decrease, a set without rows, a group without models, a model index outside [0, M) or a set index outside [0, S).
+ * Restores the caller's device. */
+int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok, const double* ab,
+                       int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X_rowmajor, const int64_t* set_off,
+                       int32_t G, const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce,
+                       double* out, int32_t* n_used);
+
 /* Timing helper for bench.py: accumulated device time (ms) and launch counts of the sweeps run while enabled, per
  * stage (0 propose, 1 evaluation stage as a whole, 2 resolve, 3 k_trees alone, 4 Gram kernel alone), measured with
  * CUDA events on the run's stream.  While enabled, bsr_run uses a single chain group and synchronises every sweep. */

@@ -175,6 +175,44 @@ class BSR(BaseEstimator, RegressorMixin):
                           "their roots_ / betas_ hold the current states (see done_)" % (open_sets, int(self.max_sweeps)), RuntimeWarning)
         return fits
 
+    @staticmethod
+    def predict_many(fits, test_data, method="last", last_ind=1, return_std=False):
+        """Predict many fitted estimators, each on its own test set, in one GPU call; returns one result per fit.
+
+        ``fits``: fitted estimators of one ``treeNum`` and device (``fit_many``'s result, cross-validation folds, ...);
+        ``test_data``: one X per fit, row counts may differ.  ``method="last"`` gives ``fit.predict(X, last_ind=last_ind)``,
+        ``"best"`` ``fit.predict_best(X)``, ``"mean"`` ``fit.predict_mean(X, return_std=return_std)`` (and sets each fit's
+        ``n_used_`` as that does): (n_b, 1) arrays, or (mean, std) pairs, bit for bit what those methods return.  All models go up
+        in one upload and are evaluated in one launch (``bsr_predict_groups``)."""
+        fits, test_data = list(fits), list(test_data)
+        if len(fits) != len(test_data):
+            raise ValueError("predict_many: %d fits and %d test sets" % (len(fits), len(test_data)))
+        if method not in ("last", "best", "mean"):
+            raise ValueError("predict_many: method must be 'last', 'best' or 'mean', not %r" % (method,))
+        if not fits:
+            return []
+        check_same_engine(fits)
+        Xs = [_as_matrix(X) for X in test_data]
+        if method == "last":
+            sel = []
+            for b, f in enumerate(fits):
+                m = len(f.betas_) - last_ind
+                if not 0 <= m < len(f.betas_):
+                    raise ValueError("predict_many: last_ind = %r is outside 1 .. %d for fit %d" % (last_ind, len(f.betas_), b))
+                sel.append([m])
+        elif method == "best":
+            sel = [[f.best_chain()] for f in fits]
+        else:
+            sel = [np.arange(len(f.betas_)) for f in fits]
+        blocks, used = predict_fit_groups(fits, Xs, [(b, b, idx, method == "mean") for b, idx in enumerate(sel)])
+        if method != "mean":
+            return [blk[0].reshape(-1, 1) for blk in blocks]
+        out = []
+        for f, blk, u in zip(fits, blocks, used):
+            f.n_used_ = int(u)
+            out.append((blk[0].reshape(-1, 1), blk[1].reshape(-1, 1)) if return_std else blk[0].reshape(-1, 1))
+        return out
+
     # ---- beyond the reference: what a batch of restarts allows (SURVEY.md 8f 1, 3) ----------------------
     def best_chain(self):
         """Index of the restart with the lowest training RMSE at its last accept (codes/simulations.py:127-128 picks restarts
@@ -316,6 +354,33 @@ def check_datasets(data, ragged=False):
         if not ragged and X.shape != (n, d):
             raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape%s"
                              % (b, X.shape[0], X.shape[1], n, d, " (ragged=True accepts different row counts)" if X.shape[1] == d else ""))
+
+
+def check_same_engine(fits):
+    """The fits one grouped prediction serves must share ``treeNum`` and device (else ValueError) and be fitted (else the
+    AttributeError ``predict`` raises on an unfitted estimator)."""
+    K, dev = int(fits[0].treeNum), fits[0]._device_index()
+    for b, f in enumerate(fits):
+        if int(f.treeNum) != K:
+            raise ValueError("predict_many: fit %d has treeNum = %d, fit 0 has %d" % (b, int(f.treeNum), K))
+        if f._device_index() != dev:
+            raise ValueError("predict_many: fit %d is on device %d, fit 0 on device %d" % (b, f._device_index(), dev))
+    for f in fits:
+        len(f.betas_)                 # an unfitted estimator: AttributeError, as from predict
+
+
+def predict_fit_groups(fits, test_sets, groups):
+    """The models of several fits on several test sets in one ``capi.predict_groups`` call.  ``groups``: (fit b, test set s, model
+    indices within fit b, reduce) tuples.  The fits' packed trees are concatenated as they are (no per-tree work on the host).
+    Returns (blocks, n_used) of ``capi.predict_groups``."""
+    check_same_engine(fits)
+    K = int(fits[0].treeNum)
+    pk = capi.PackedTrees.concat([f._packed_ for f in fits])
+    first = np.zeros(len(fits) + 1, dtype=np.int64)
+    np.cumsum([f._packed_.nn.shape[0] for f in fits], out=first[1:])
+    beta = np.concatenate([np.asarray(f.betas_, dtype=np.float64).reshape(-1, K + 1) for f in fits])
+    return capi.predict_groups(fits[0]._device_index(), pk.nn, pk.tok, pk.ab, beta, test_sets, [s for _, s, _, _ in groups],
+                               [first[b] + np.asarray(idx, dtype=np.int64) for b, _, idx, _ in groups], [r for _, _, _, r in groups])
 
 
 def dataset_seeds(seed, n_datasets, seeds=None):

@@ -73,6 +73,8 @@ _SIGS = {
     "bsr_predict_trees": (C.c_int, [C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int32, _P]),
     "bsr_predict_many": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P,
                                    C.POINTER(C.c_int32)]),
+    "bsr_predict_groups": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int32, C.c_int32, _P, _P,
+                                     C.c_int32, _P, _P, _P, _P, _P, _P]),
     "bsr_peer_export": (C.c_int, [_P, C.c_int32, _P]),
     "bsr_peer_import": (C.c_int, [_P, C.c_int32, C.c_int32, _P]),
     "bsr_set_window": (C.c_int, [_P, C.c_int32]),
@@ -152,6 +154,44 @@ def predict_many(device, tok, pa, pb, nn, beta, X, reduce=False):
     return out
 
 
+def predict_groups(device, nn, tok, ab, beta, test_sets, grp_set, grp_models, grp_reduce):
+    """Many models on many test sets in one call (``bsr_predict_groups``).  Models packed as ``PackedTrees`` holds them: nn [M][K],
+    tok the tokens of tree after tree, ab [n_lt][2]; beta [M][K+1].  ``test_sets``: S arrays (n_s, d), one d.  Group g evaluates the
+    model indices ``grp_models[g]`` on ``test_sets[grp_set[g]]``.  Returns (blocks, n_used): blocks[g] is (n_models_g, n_s), or, for
+    ``grp_reduce[g]``, (2, n_s) with the mean over the models and their standard deviation (what ``predict_many`` returns for
+    reduce=False / True); n_used [G] the smallest number of models any row of a group used."""
+    lib = load()
+    nn = np.ascontiguousarray(nn, dtype=np.int32)
+    M, K = nn.shape
+    tok = np.ascontiguousarray(tok, dtype=np.uint32).ravel()
+    ab = np.ascontiguousarray(ab, dtype=np.float64).reshape(-1, 2)
+    beta = np.ascontiguousarray(beta, dtype=np.float64).reshape(M, K + 1)
+    Xs = [np.asarray(X, dtype=np.float64) for X in test_sets]
+    if not Xs or any(X.ndim != 2 or X.shape[1] != Xs[0].shape[1] for X in Xs):
+        raise ValueError("predict_groups: test_sets must be one or more (n_s, d) arrays of the same d")
+    set_off = np.zeros(len(Xs) + 1, dtype=np.int64)
+    np.cumsum([X.shape[0] for X in Xs], out=set_off[1:])
+    X = np.ascontiguousarray(np.concatenate(Xs, axis=0))
+    models = [np.asarray(m, dtype=np.int32).ravel() for m in grp_models]
+    G = len(models)
+    grp_set = np.ascontiguousarray(grp_set, dtype=np.int32).ravel()
+    grp_reduce = np.ascontiguousarray([int(bool(r)) for r in grp_reduce], dtype=np.int32)
+    if grp_set.size != G or grp_reduce.size != G or G == 0:
+        raise ValueError("predict_groups: grp_set, grp_models and grp_reduce must describe the same one or more groups")
+    grp_off = np.zeros(G + 1, dtype=np.int64)
+    np.cumsum([m.size for m in models], out=grp_off[1:])
+    flat = np.ascontiguousarray(np.concatenate(models))
+    rows = np.array([Xs[s].shape[0] if 0 <= s < len(Xs) else 0 for s in grp_set], dtype=np.int64)
+    sizes = np.where(grp_reduce != 0, 2, grp_off[1:] - grp_off[:-1]) * rows
+    out = np.zeros(int(sizes.sum()))
+    used = np.zeros(G, dtype=np.int32)
+    _ck(lib.bsr_predict_groups(int(device), M, K, _ptr(nn), _ptr(tok), tok.size, _ptr(ab), ab.shape[0], _ptr(beta), len(Xs), X.shape[1],
+                               _ptr(X), _ptr(set_off), G, _ptr(grp_set), _ptr(grp_off), _ptr(flat), _ptr(grp_reduce), _ptr(out), _ptr(used)))
+    ends = np.cumsum(sizes)
+    blocks = [out[e - z:e].reshape(-1, int(r)) for e, z, r in zip(ends, sizes, rows)]
+    return blocks, used
+
+
 class PackedTrees:
     """Trees without the padding of their device slots (``bsr_pack_trees``): ``nn`` [C][K] node counts, ``tok`` the tokens of
     tree after tree, ``ab`` the (a, b) pairs of the lt nodes in node order.  ``tree(c, k)`` / ``dense()`` give the fixed-capacity
@@ -160,6 +200,13 @@ class PackedTrees:
     def __init__(self, nn, tok, ab):
         self.nn, self.tok, self.ab = nn, tok, ab
         self._off = None
+
+    @staticmethod
+    def concat(packs):
+        """The models of several PackedTrees of the same K, one table after another: model m of packs[i] becomes model
+        sum(models of packs[:i]) + m (its nodes and lt pairs follow those of the packs before it)."""
+        return PackedTrees(np.concatenate([p.nn for p in packs]), np.concatenate([p.tok for p in packs]),
+                           np.concatenate([np.asarray(p.ab, dtype=np.float64).reshape(-1, 2) for p in packs]))
 
     @property
     def nbytes(self):

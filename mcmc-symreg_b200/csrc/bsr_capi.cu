@@ -1,4 +1,5 @@
 // C-ABI of libbsr_b200.so (see include/bsr_b200.h): host-side handle, memory, launches.
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -33,6 +34,16 @@ static void dfree(bsr_handle* h, void* p) {
     if (h->allocs[i] == p) { h->allocs.erase(h->allocs.begin() + i); break; }
   cudaFree(p);
 }
+
+// One device buffer carved into 256-byte aligned sections (bsr_predict_groups).
+struct Carve {
+  size_t bytes = 0;
+  template <typename T> size_t take(size_t count) {
+    const size_t at = bytes;
+    bytes += (count * sizeof(T) + 255) / 256 * 256;
+    return at;
+  }
+};
 
 extern "C" {
 
@@ -229,7 +240,9 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, c
     h->own_x32 = true;
     if (dalloc(h, &h->X32, D * ld * d) || dalloc(h, &h->X64, D * ld * d) || dalloc(h, &h->y32, D * ld) || dalloc(h, &h->y64, D * ld)) return 1;
   }
-  // staging: X, then y, then the row offsets
+  off.resize(2 * ((size_t)D + 1));                   // then the first column element of every data set: b * ld (one ld for all)
+  for (int b = 0; b <= D; ++b) off[(size_t)D + 1 + b] = (int64_t)b * (int64_t)ld;
+  // staging: X, then y, then the row and column offsets
   const size_t xs = (size_t)rows * d, bytes = (xs + (size_t)rows) * sizeof(double) + off.size() * sizeof(int64_t);
   if (bytes > h->stage_bytes) {
     CK(cudaDeviceSynchronize());
@@ -240,6 +253,7 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, c
   }
   double* ystage = h->stage + xs;
   int64_t* d_off = reinterpret_cast<int64_t*>(ystage + rows);
+  int64_t* d_col = d_off + D + 1;
   h->n_total = n_total > 0 ? n_total : n;
   // stream-ordered after any sweep still in flight on the default stream; the copies from pageable memory are synchronous
   CK(cudaMemcpy(h->stage, X, xs * sizeof(double), cudaMemcpyHostToDevice));
@@ -247,10 +261,10 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, c
   CK(cudaMemcpy(d_off, off.data(), off.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
   // one launch per buffer for all D data sets (blockIdx.y); y is the one-column case
   const dim3 blocks((unsigned)std::min<int64_t>(((int64_t)ld * d + 255) / 256, 148 * 16), (unsigned)D);
-  k_transpose_datasets_in<float><<<blocks, 256>>>(h->stage, d_off, h->X32, d, h->ld);
-  k_transpose_datasets_in<double><<<blocks, 256>>>(h->stage, d_off, h->X64, d, h->ld);
-  k_transpose_datasets_in<float><<<blocks, 256>>>(ystage, d_off, h->y32, 1, h->ld);
-  k_transpose_datasets_in<double><<<blocks, 256>>>(ystage, d_off, h->y64, 1, h->ld);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(h->stage, d_off, d_col, h->X32, d);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(h->stage, d_off, d_col, h->X64, d);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(ystage, d_off, d_col, h->y32, 1);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(ystage, d_off, d_col, h->y64, 1);
   CK(cudaGetLastError());
   return 0;
 }
@@ -1124,6 +1138,157 @@ int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, 
   rc = body();
   cudaFree(d_tok); cudaFree(d_a); cudaFree(d_b); cudaFree(d_nn); cudaFree(d_beta); cudaFree(d_x); cudaFree(d_xc); cudaFree(d_pred);
   cudaFree(d_ms); cudaFree(d_used);
+  cudaSetDevice(prev);
+  return rc;
+}
+
+int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok, const double* ab,
+                       int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X, const int64_t* set_off, int32_t G,
+                       const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce, double* out,
+                       int32_t* n_used) {
+  const std::string f = "bsr_predict_groups: ";
+  if (!nn || !tok || !ab || !beta || !X || !set_off || !grp_set || !grp_off || !grp_models || !grp_reduce || !out || !n_used)
+    return fail(f + "null argument");
+  if (M < 1 || K < 1 || K > BSR_MAXK || S < 1 || G < 1 || d < 1 || n_tok < 0 || n_lt < 0)
+    return fail(f + "bad shape (need M, S, G, d >= 1, 1 <= K <= 16, n_tok, n_lt >= 0)");
+  // models: every tree a well-formed pre-order token sequence of 1 .. 64 nodes reading features < d; the node counts cover tok and
+  // the lt nodes cover ab exactly
+  const size_t NT = (size_t)M * K;
+  std::vector<int64_t> node_off(NT + 1, 0), lt_off(NT + 1, 0);
+  for (size_t t = 0; t < NT; ++t) {
+    if (nn[t] < 1 || nn[t] > BSR_MAXN) return fail(f + "tree size out of range (1 .. 64 nodes)");
+    node_off[t + 1] = node_off[t] + nn[t];
+    if (node_off[t + 1] > n_tok) return fail(f + "the node counts nn add up to more tokens than tok holds");
+    int64_t lts = 0;
+    int depth = 0;                                  // subtrees the right-to-left scan holds
+    for (int64_t i = node_off[t + 1] - 1; i >= node_off[t]; --i) {
+      const int op = tok_op(tok[i]);
+      if (op > OP_MUL) return fail(f + "unknown opcode in tok");
+      if (op == OP_LEAF && tok_ft(tok[i]) >= d) return fail(f + "a tree reads a feature the data does not have");
+      const int ar = op_arity(op);
+      if (depth < ar) return fail(f + "a token sequence is not a pre-order tree");
+      depth += 1 - ar;
+      lts += op == OP_LT;
+    }
+    if (depth != 1) return fail(f + "a token sequence is not a pre-order tree");
+    lt_off[t + 1] = lt_off[t] + lts;
+  }
+  if (node_off[NT] != n_tok) return fail(f + "the node counts nn add up to fewer tokens than tok holds");
+  if (lt_off[NT] != n_lt) return fail(f + "the lt nodes of tok and the (a, b) pairs of ab differ in number");
+  // test sets: each its own ld (rows rounded up to 4, so every column starts 32-byte aligned)
+  if (set_off[0] != 0) return fail(f + "set_off[0] must be 0");
+  std::vector<int64_t> col_off((size_t)S + 1, 0), n_rows((size_t)S);
+  int64_t max_n = 0;
+  for (int s = 0; s < S; ++s) {
+    const int64_t n = set_off[s + 1] - set_off[s];
+    if (n < 0) return fail(f + "set_off decreases");
+    if (n == 0) return fail(f + "test set " + std::to_string(s) + " has no rows");
+    const int64_t ld = (n + 3) / 4 * 4;
+    if (ld * (int64_t)d >= (int64_t)1 << 32) return fail(f + "a test set of d * n >= 2^32 elements");
+    n_rows[(size_t)s] = n;
+    col_off[(size_t)s + 1] = col_off[(size_t)s] + ld;
+    max_n = std::max(max_n, n);
+  }
+  // groups and their tasks
+  if (grp_off[0] != 0) return fail(f + "grp_off[0] must be 0");
+  std::vector<int64_t> grp_out((size_t)G), grp_scr((size_t)G, -1);
+  std::vector<int32_t> red_grp, used((size_t)G);
+  int64_t out_total = 0, red_models = 0;
+  for (int g = 0; g < G; ++g) {
+    const int64_t cnt = grp_off[g + 1] - grp_off[g];
+    if (cnt < 0) return fail(f + "grp_off decreases");
+    if (cnt == 0) return fail(f + "group " + std::to_string(g) + " has no models");
+    if (grp_set[g] < 0 || grp_set[g] >= S) return fail(f + "grp_set[" + std::to_string(g) + "] is outside [0, S)");
+    if (grp_off[g + 1] > INT32_MAX) return fail(f + "more than 2^31 - 1 (group, model) tasks");
+    const int64_t n = n_rows[(size_t)grp_set[g]];
+    grp_out[(size_t)g] = out_total;
+    out_total += (grp_reduce[g] ? 2 : cnt) * n;
+    used[(size_t)g] = (int32_t)cnt;
+    if (grp_reduce[g]) { red_grp.push_back(g); grp_scr[(size_t)g] = red_models; red_models += cnt; }
+  }
+  const int64_t T = grp_off[G];
+  std::vector<int32_t> task_grp((size_t)T);
+  for (int g = 0; g < G; ++g)
+    for (int64_t t = grp_off[g]; t < grp_off[g + 1]; ++t) {
+      if (grp_models[t] < 0 || grp_models[t] >= M) return fail(f + "grp_models[" + std::to_string(t) + "] is outside [0, M)");
+      task_grp[(size_t)t] = g;
+    }
+  // rows in chunks so that the predictions of the reducing groups ([models][chunk]) stay near 256 MB; one chunk without them
+  int64_t chunk = (max_n + 1) / 2 * 2;
+  if (red_models) chunk = std::min(chunk, std::max<int64_t>(256, ((int64_t)32 << 20) / red_models) / 2 * 2);
+  for (int64_t& o : grp_scr) if (o >= 0) o *= chunk;
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(f + "no CUDA device (no CPU fallback)");
+  // one device buffer: the uploaded sections first (one copy), then used and out (read back), the transposed sets and the scratch
+  Carve c;
+  const int64_t rows_total = set_off[S];
+  const size_t o_X = c.take<double>((size_t)rows_total * d), o_tok = c.take<uint32_t>((size_t)n_tok), o_ab = c.take<double>(2 * (size_t)n_lt);
+  const size_t o_beta = c.take<double>(NT + M), o_node = c.take<int64_t>(NT + 1), o_lt = c.take<int64_t>(NT + 1);
+  const size_t o_soff = c.take<int64_t>((size_t)S + 1), o_col = c.take<int64_t>((size_t)S + 1), o_nrows = c.take<int64_t>((size_t)S);
+  const size_t o_tmod = c.take<int32_t>((size_t)T), o_tgrp = c.take<int32_t>((size_t)T), o_gset = c.take<int32_t>((size_t)G);
+  const size_t o_goff = c.take<int64_t>((size_t)G + 1), o_gout = c.take<int64_t>((size_t)G), o_gscr = c.take<int64_t>((size_t)G);
+  const size_t o_red = c.take<int32_t>(red_grp.size()), o_used = c.take<int32_t>((size_t)G);
+  const size_t up_bytes = c.bytes;
+  const size_t o_out = c.take<double>((size_t)out_total), o_xc = c.take<double>((size_t)col_off[(size_t)S] * d);
+  const size_t o_scr = c.take<double>((size_t)red_models * chunk);
+  std::vector<unsigned char> up(up_bytes);
+  auto put = [&](size_t at, const void* src, size_t bytes) { if (bytes) memcpy(up.data() + at, src, bytes); };
+  put(o_X, X, (size_t)rows_total * d * sizeof(double));
+  put(o_tok, tok, (size_t)n_tok * sizeof(uint32_t));
+  put(o_ab, ab, 2 * (size_t)n_lt * sizeof(double));
+  put(o_beta, beta, (NT + M) * sizeof(double));
+  put(o_node, node_off.data(), (NT + 1) * sizeof(int64_t));
+  put(o_lt, lt_off.data(), (NT + 1) * sizeof(int64_t));
+  put(o_soff, set_off, ((size_t)S + 1) * sizeof(int64_t));
+  put(o_col, col_off.data(), ((size_t)S + 1) * sizeof(int64_t));
+  put(o_nrows, n_rows.data(), (size_t)S * sizeof(int64_t));
+  put(o_tmod, grp_models, (size_t)T * sizeof(int32_t));
+  put(o_tgrp, task_grp.data(), (size_t)T * sizeof(int32_t));
+  put(o_gset, grp_set, (size_t)G * sizeof(int32_t));
+  put(o_goff, grp_off, ((size_t)G + 1) * sizeof(int64_t));
+  put(o_gout, grp_out.data(), (size_t)G * sizeof(int64_t));
+  put(o_gscr, grp_scr.data(), (size_t)G * sizeof(int64_t));
+  put(o_red, red_grp.data(), red_grp.size() * sizeof(int32_t));
+  put(o_used, used.data(), (size_t)G * sizeof(int32_t));
+  int prev = 0;
+  cudaGetDevice(&prev);
+  unsigned char* buf = nullptr;
+  auto body = [&]() -> int {
+    CK(cudaSetDevice(device));
+    CK(cudaMalloc((void**)&buf, c.bytes));
+    CK(cudaMemcpy(buf, up.data(), up_bytes, cudaMemcpyHostToDevice));
+    GroupTables p;
+    p.tok = (const uint32_t*)(buf + o_tok); p.ab = (const double*)(buf + o_ab);
+    p.node_off = (const int64_t*)(buf + o_node); p.lt_off = (const int64_t*)(buf + o_lt); p.beta = (const double*)(buf + o_beta);
+    p.X = (const double*)(buf + o_xc); p.col_off = (const int64_t*)(buf + o_col); p.n_rows = (const int64_t*)(buf + o_nrows);
+    p.task_model = (const int*)(buf + o_tmod); p.task_grp = (const int*)(buf + o_tgrp); p.grp_set = (const int*)(buf + o_gset);
+    p.grp_off = (const int64_t*)(buf + o_goff); p.grp_out = (const int64_t*)(buf + o_gout); p.grp_scr = (const int64_t*)(buf + o_gscr);
+    p.red_grp = (const int*)(buf + o_red);
+    p.out = (double*)(buf + o_out); p.scr = (double*)(buf + o_scr); p.used = (int*)(buf + o_used);
+    p.K = K; p.d = d;
+    // all test sets in one launch (blockIdx.y = set; 65535 sets per launch)
+    const unsigned tx = (unsigned)std::min<int64_t>(((max_n + 3) / 4 * 4 * d + 255) / 256, 148 * 16);
+    for (int s0 = 0; s0 < S; s0 += 65535)
+      k_transpose_datasets_in<double><<<dim3(tx, (unsigned)std::min(65535, S - s0)), 256>>>(
+          (const double*)(buf + o_X), (const int64_t*)(buf + o_soff) + s0, p.col_off + s0, (double*)(buf + o_xc), d);
+    CK(cudaGetLastError());
+    const size_t smem = (size_t)K * BSR_MAXN * sizeof(EvTok<double>);
+    const unsigned by = (unsigned)std::max<int64_t>(1, std::min<int64_t>(((chunk + 1) / 2 + 127) / 128, 64));
+    const unsigned ry = (unsigned)std::max<int64_t>(1, std::min<int64_t>((chunk + 127) / 128, 64));
+    for (int64_t r0 = 0; r0 < max_n; r0 += chunk) {
+      k_predict_groups<<<dim3((unsigned)T, by), 128, smem>>>(p, r0, chunk);
+      CK(cudaGetLastError());
+      if (!red_grp.empty()) {
+        k_predict_groups_reduce<<<dim3((unsigned)red_grp.size(), ry), 128>>>(p, r0, chunk);
+        CK(cudaGetLastError());
+      }
+    }
+    CK(cudaMemcpy(n_used, buf + o_used, (size_t)G * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    if (out_total) CK(cudaMemcpy(out, buf + o_out, (size_t)out_total * sizeof(double), cudaMemcpyDeviceToHost));
+    return 0;
+  };
+  const int rc = body();
+  if (buf) cudaFree(buf);
   cudaSetDevice(prev);
   return rc;
 }

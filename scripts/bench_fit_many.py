@@ -4,7 +4,11 @@
    Wall clock of the loop of BSR.fit calls against one BSR.fit_many over the same data sets and seeds, alternated, each timing
    ending in a device synchronise; the two must give equal results (checked in the same run).
    With several sizes (--rows 30,100,300,1000) the suite is f1 ... f6 x those sizes x R repeats, and fit_many runs with ragged=True.
-2. Engine throughput: D data sets x 50 chains on n = 100 rows (the first of --rows), fixed sweeps, device-timed (CUDA events)
+2. The summaries of those fits (experiments.summarize: RMSE of the last, best and mean prediction on the training, test and
+   extrapolation sets, 9 predictions per fit): the summarize loop against summarize_many (one grouped prediction call), alternated,
+   each timing ending in a device synchronise, rows compared; and per method the 3 x (data sets) single-estimator prediction calls
+   against one BSR.predict_many per set.
+3. Engine throughput: D data sets x 50 chains on n = 100 rows (the first of --rows), fixed sweeps, device-timed (CUDA events)
    proposals per second.  With several sizes, one more line: the largest D with the data sets cycling through the sizes (a ragged
    batch, every chain on its own rows) against the same chains on data sets of the largest size.
 
@@ -80,6 +84,54 @@ def bench_suite(repeats, rounds, sizes):
                 speedup_median=float(np.median(t_loop) / np.median(t_batch)), results_equal=equal)
 
 
+def bench_summaries(repeats, rounds, sizes):
+    """The summaries of the suite's fits: the per-estimator summarize loop (9 prediction calls per fit) against summarize_many (one
+    grouped call), alternated, each timing ending in a device synchronise, rows compared as JSON.  Then the predictions alone: per
+    method, one call per (fit, set) against one BSR.predict_many per set."""
+    import torch
+    from mcmc_symreg_b200 import BSR
+    from mcmc_symreg_b200.experiments import SETS, summarize, summarize_many
+    jobs, data = suite_data(repeats, sizes)
+    fits = BSR(3, 50, val=100).fit_many([(d["X"], d["y"]) for d in data], seeds=[s for _, _, _, s in jobs], ragged=len(sizes) > 1)
+    dump = lambda rows: [json.dumps(o, sort_keys=True, default=str) for o in rows]
+
+    def timed(fn):
+        t0 = time.perf_counter()
+        out = fn()
+        torch.cuda.synchronize()
+        return time.perf_counter() - t0, out
+
+    loop = lambda: [summarize(e, d) for e, d in zip(fits, data)]
+    many = lambda: summarize_many(fits, data)
+    loop(); many()                                # module loads, allocations
+    t_loop, t_many, equal = [], [], True
+    for _ in range(rounds):
+        ta, a = timed(loop)
+        tb, b = timed(many)
+        t_loop.append(ta); t_many.append(tb)
+        equal = equal and dump(a) == dump(b)
+    assert equal, "summarize_many and the summarize loop disagree"
+    single = dict(last=lambda e, X: e.predict(X), best=lambda e, X: e.predict_best(X), mean=lambda e, X: e.predict_mean(X))
+    per_method = {}
+    for method, call in single.items():
+        singles = lambda: [call(e, d[Xk]) for _, Xk, _ in SETS for e, d in zip(fits, data)]
+        grouped = lambda: [BSR.predict_many(fits, [d[Xk] for d in data], method=method) for _, Xk, _ in SETS]
+        singles(); grouped()
+        ts, tg, same = [], [], True
+        for _ in range(rounds):
+            t, a = timed(singles)
+            ts.append(t)
+            t, b = timed(grouped)
+            tg.append(t)
+            same = same and all(np.array_equal(x, y) for x, y in zip(a, [p for per_set in b for p in per_set]))
+        assert same, "predict_many(method=%r) and the single calls disagree" % method
+        per_method[method] = dict(single_calls=len(fits) * len(SETS), single_seconds=ts, predict_many_calls=len(SETS),
+                                  predict_many_seconds=tg, speedup_median=float(np.median(ts) / np.median(tg)))
+    return dict(fits=len(fits), loop_seconds=t_loop, summarize_many_seconds=t_many,
+                loop_ms_per_fit=1e3 * float(np.median(t_loop)) / len(fits), summarize_many_ms_per_fit=1e3 * float(np.median(t_many)) / len(fits),
+                speedup_median=float(np.median(t_loop) / np.median(t_many)), results_equal=equal, predictions=per_method)
+
+
 def bench_engine(D, sweeps, n, C=50, K=3):
     """n: the rows of every data set, or a sequence the data sets cycle through (a ragged batch)"""
     import torch
@@ -129,6 +181,7 @@ def main(argv=None):
     sizes = [int(v) for v in a.rows.split(",")]
     Ds = [int(D) for D in a.datasets.split(",")]
     out["suite"] = bench_suite(a.repeats, a.rounds, sizes)
+    out["summaries"] = bench_summaries(a.repeats, a.rounds, sizes)
     out["engine"] = [bench_engine(D, a.sweeps, sizes[0]) for D in Ds]
     if len(sizes) > 1:
         # the same chains on the ragged batch and on data sets of the largest size: what rows a chain does not hold cost nothing
