@@ -241,21 +241,30 @@ int bsr_count_done(bsr_handle* h, int32_t* n_done);
  * precision as in bsr_config. */
 int bsr_eval_trees(bsr_handle* h, int32_t n_trees, const uint32_t* tok, const double* pa, const double* pb,
                    const int32_t* nn, int32_t precision, double* out);
-/* BSR.predict (codes/bsr_class.py:53-68) for one chain: out[i] = beta0 + sum_k beta_k * tree_k(X[i]).
- * reported != 0 uses the roots_ snapshot, else the live state. */
+/* Prediction: BSR.predict (codes/bsr_class.py:53-68) of model m on row i, evaluated in float64 on `device` (all but bsr_predict
+ * need no handle, so a fitted or un-pickled estimator predicts without chain state on the device):
+ *   pred_m(X[i]) = beta_m[0] + sum_k beta_m[k+1] * tree_mk(X[i]),  k in order.
+ * A reducing call returns instead, row by row, the posterior-predictive mean over its models and their sample standard deviation,
+ * reduced on the device in model order; a model whose prediction at a row is not finite is left out of that row, and n_used
+ * returns the smallest number of models any row used (the model count without reduce).  This extends codes/bsr_class.py:53-68,
+ * which reads one restart (SURVEY.md 8f 1).  All four entry points run the same kernels, so a model predicts the same bits through
+ * each.  Refused on the host, before the device reads anything: null pointers; K outside 1 .. BSR_MAX_TREES; a tree of 0 or more
+ * than 64 nodes, with an unknown opcode, whose tokens are not a pre-order tree or with a leaf feature >= d; a test set without rows
+ * or of ld * d >= 2^32 elements (ld = its rows rounded up to 4).  The model count has no limit of its own.  The caller's device is
+ * restored and every device buffer freed on every path, failures included.  On the device a call holds its inputs and its whole
+ * output (a non-reducing call [M][n_test] of them), plus, for the models of reducing groups, a [models][chunk] scratch: rows go in
+ * chunks that keep it near 256 MB (at least 256 rows a chunk).
+ *
+ * bsr_predict: one chain of a handle; reported != 0 uses the roots_ snapshot, else the live state. */
 int bsr_predict(bsr_handle* h, int32_t chain, int32_t reported, const double* X_rowmajor, int64_t n_test, int32_t d,
                 double* out);
 
-/* Same for K explicit trees (host arrays [K][BSR_MAX_NODES], beta [K+1]); needs no handle, so a fitted (or
- * un-pickled) estimator can predict without keeping chain state on the device. */
+/* K explicit trees (host arrays [K][BSR_MAX_NODES], beta [K+1]): out [n_test]. */
 int bsr_predict_trees(int32_t device, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
                       const double* beta, const double* X_rowmajor, int64_t n_test, int32_t d, double* out);
 
-/* The same for M models at once -- the restarts of one fit (host arrays [M][K][BSR_MAX_NODES], nn [M][K], beta [M][K+1]).
- * reduce == 0: out is [M][n_test], every model's predictions.  reduce != 0: out is [2][n_test], the posterior-predictive
- * mean over the models and the standard deviation across them, reduced on the device in model order; a model whose
- * prediction at a row is not finite is left out of that row and *n_used returns the smallest number of models any row
- * used.  Extends codes/bsr_class.py:53-68, which reads one restart (SURVEY.md 8f 1). */
+/* M models at once -- the restarts of one fit (host arrays [M][K][BSR_MAX_NODES], nn [M][K], beta [M][K+1]).  reduce == 0: out is
+ * [M][n_test]; reduce != 0: out is [2][n_test] (mean, then std).  n_used may be NULL. */
 int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
                      const double* beta, const double* X_rowmajor, int64_t n_test, int32_t d, int32_t reduce, double* out,
                      int32_t* n_used);
@@ -265,14 +274,9 @@ int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, 
  * holds nn[m][k]); ab [n_lt][2] the (a, b) pairs of the lt nodes in node order; beta [M][K+1].
  * Test sets: X_rowmajor holds the rows of S sets of d features one after another, set s is rows set_off[s] .. set_off[s+1].
  * Groups: group g evaluates the models grp_models[grp_off[g] .. grp_off[g+1]) on set grp_set[g].
- * out holds the groups' blocks in group order: [n_models_g][n_rows_s] predictions, or, when grp_reduce[g] != 0, [2][n_rows_s]: the
- * mean over the group's models and their standard deviation, reduced on the device in model order with the arithmetic of
- * bsr_predict_many.  n_used[g] is the smallest number of models any row of group g used (its model count without reduce).
- * Every value equals what bsr_predict_many returns for the same models on the same set.  Refused before anything is read on the
- * device: null pointers, K outside 1 .. BSR_MAX_TREES, a tree of 0 or more than 64 nodes or whose tokens are not a pre-order tree,
- * node counts that do not cover tok, lt nodes that do not match n_lt, a leaf feature >= d, set_off or grp_off that do not start at
- * 0 or decrease, a set without rows, a group without models, a model index outside [0, M) or a set index outside [0, S).
- * Restores the caller's device. */
+ * out holds the groups' blocks in group order: [n_models_g][n_rows_s] predictions, or, when grp_reduce[g] != 0, [2][n_rows_s] (mean,
+ * then std); n_used [G].  Also refused: node counts that do not cover tok, lt nodes that do not match n_lt, set_off or grp_off that
+ * do not start at 0 or decrease, a group without models, a model index outside [0, M) or a set index outside [0, S). */
 int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok, const double* ab,
                        int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X_rowmajor, const int64_t* set_off,
                        int32_t G, const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce,

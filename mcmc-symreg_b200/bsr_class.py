@@ -268,16 +268,19 @@ class BSR(BaseEstimator, RegressorMixin):
         return parallel.default_device()
 
     def _predict_chains(self, idx, X, reduce=False):
-        pk = self._packed_
-        idx = np.asarray(idx, dtype=np.int64)
-        K = pk.nn.shape[1]
-        tok = np.zeros((len(idx), K, capi.MAX_NODES), dtype=np.uint32); pa = np.zeros((len(idx), K, capi.MAX_NODES)); pb = np.zeros_like(pa)
-        nn = np.zeros((len(idx), K), dtype=np.int32)
-        for j, m in enumerate(idx):
-            for k in range(K):
-                tok[j, k], pa[j, k], pb[j, k], nn[j, k] = pk.tree(int(m), k)
-        beta = np.stack([np.asarray(self.betas_[int(m)]).ravel() for m in idx])
-        return capi.predict_many(self._device_index(), tok, pa, pb, nn, beta, X, reduce=reduce)
+        """The restarts ``idx`` on X as one group of one ``capi.predict_groups`` call: their (len(idx), n) predictions, or, with
+        ``reduce``, (mean, std, n_used) over them.  Only their rows of the packed table go to the device (a large fit's whole table
+        would cost predict() of one restart more than the prediction).  An index outside [0, len(betas_)) raises IndexError."""
+        idx = np.asarray(idx, dtype=np.int64).ravel()
+        bad = idx[(idx < 0) | (idx >= len(self.betas_))]
+        if bad.size:
+            raise IndexError("restart index %d is outside 0 .. %d" % (int(bad[0]), len(self.betas_) - 1))
+        pk = self._packed_.select(idx)
+        beta = np.stack([np.asarray(self.betas_[m], dtype=np.float64).ravel() for m in idx])
+        blocks, used = capi.predict_groups(self._device_index(), pk.nn, pk.tok, pk.ab, beta, [X], [0], [np.arange(idx.size)], [reduce])
+        if reduce:
+            return blocks[0][0], blocks[0][1], int(used[0])
+        return blocks[0]
 
     def _set_results(self, res):
         self._packed_ = capi.PackedTrees(res["nn"], res["ptok"], res["pab"])

@@ -117,22 +117,6 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
-def predict_trees(device, tok, pa, pb, nn, beta, X):
-    """BSR.predict for K explicit trees (codes/bsr_class.py:53-68) on `device`; returns (n_test,) float64."""
-    lib = load()
-    tok = np.ascontiguousarray(tok, dtype=np.uint32).reshape(-1, MAX_NODES)
-    K = tok.shape[0]
-    pa = np.ascontiguousarray(pa, dtype=np.float64).reshape(K, MAX_NODES)
-    pb = np.ascontiguousarray(pb, dtype=np.float64).reshape(K, MAX_NODES)
-    nn = np.ascontiguousarray(nn, dtype=np.int32).reshape(K)
-    beta = np.ascontiguousarray(beta, dtype=np.float64).reshape(K + 1)
-    X = np.ascontiguousarray(X, dtype=np.float64)
-    out = np.zeros(X.shape[0])
-    _ck(lib.bsr_predict_trees(int(device), K, _ptr(tok), _ptr(pa), _ptr(pb), _ptr(nn), _ptr(beta), _ptr(X), X.shape[0],
-                              X.shape[1], _ptr(out)))
-    return out
-
-
 def predict_many(device, tok, pa, pb, nn, beta, X, reduce=False):
     """BSR.predict for M models at once (codes/bsr_class.py:53-68 per model).  tok / pa / pb: [M][K][MAX_NODES], nn [M][K],
     beta [M][K+1].  reduce=False: (M, n_test) predictions.  reduce=True: (mean, std, n_used) over the models, reduced on the
@@ -207,6 +191,16 @@ class PackedTrees:
         sum(models of packs[:i]) + m (its nodes and lt pairs follow those of the packs before it)."""
         return PackedTrees(np.concatenate([p.nn for p in packs]), np.concatenate([p.tok for p in packs]),
                            np.concatenate([np.asarray(p.ab, dtype=np.float64).reshape(-1, 2) for p in packs]))
+
+    def select(self, models):
+        """The models ``models`` (indices, in that order) as a table of their own: model j of the result is model models[j]."""
+        off, lt_before, is_lt = self._offsets()
+        models = np.asarray(models, dtype=np.int64).ravel()
+        trees = (models[:, None] * self.nn.shape[1] + np.arange(self.nn.shape[1])).ravel()
+        lens = off[trees + 1] - off[trees]
+        node = np.repeat(off[trees] - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+        ab = np.asarray(self.ab, dtype=np.float64).reshape(-1, 2)
+        return PackedTrees(self.nn[models], self.tok[node], ab[lt_before[node][is_lt[node]]])
 
     @property
     def nbytes(self):

@@ -1023,130 +1023,13 @@ int bsr_eval_trees(bsr_handle* h, int32_t n_trees, const uint32_t* tok, const do
   return 0;
 }
 
-int bsr_predict_trees(int32_t device, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
-                      const double* beta, const double* X, int64_t n_test, int32_t d, double* out) {
-  if (!tok || !pa || !pb || !nn || !beta || !X || !out) return fail("bsr_predict_trees: null argument");
-  if (K < 1 || K > BSR_MAXK || n_test < 1 || d < 1) return fail("bsr_predict_trees: bad shape");
-  for (int k = 0; k < K; ++k) {
-    if (nn[k] < 1 || nn[k] > BSR_MAXN) return fail("bsr_predict_trees: tree size out of range");
-    for (int j = 0; j < nn[k]; ++j)
-      if (tok_op(tok[k * BSR_MAXN + j]) == OP_LEAF && tok_ft(tok[k * BSR_MAXN + j]) >= d)
-        return fail("bsr_predict_trees: a tree reads a feature the data does not have");
-  }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("bsr_predict_trees: no CUDA device (no CPU fallback)");
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
-  CK(cudaSetDevice(device));
-  uint32_t* d_tok; double *d_a, *d_b, *d_x, *d_xc, *d_out, *d_beta; int* d_nn;
-  const size_t KN = (size_t)K * BSR_MAXN;
-  const int64_t ld = (n_test + 3) / 4 * 4;
-  CK(cudaMalloc((void**)&d_tok, KN * sizeof(uint32_t)));
-  CK(cudaMalloc((void**)&d_a, KN * sizeof(double)));
-  CK(cudaMalloc((void**)&d_b, KN * sizeof(double)));
-  CK(cudaMalloc((void**)&d_nn, K * sizeof(int)));
-  CK(cudaMalloc((void**)&d_beta, (K + 1) * sizeof(double)));
-  CK(cudaMalloc((void**)&d_x, (size_t)n_test * d * sizeof(double)));
-  CK(cudaMalloc((void**)&d_xc, (size_t)ld * d * sizeof(double)));
-  CK(cudaMalloc((void**)&d_out, (size_t)n_test * sizeof(double)));
-  CK(cudaMemcpy(d_tok, tok, KN * sizeof(uint32_t), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(d_a, pa, KN * sizeof(double), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(d_b, pb, KN * sizeof(double), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(d_nn, nn, K * sizeof(int), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(d_beta, beta, (K + 1) * sizeof(double), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(d_x, X, (size_t)n_test * d * sizeof(double), cudaMemcpyHostToDevice));
-  int blocks = (int)std::min<int64_t>((n_test * d + 255) / 256, 148 * 16);
-  k_transpose_in<double><<<blocks, 256>>>(d_x, d_xc, n_test, d, ld);
-  size_t smem = KN * sizeof(EvTok<double>);
-  CK(cudaFuncSetAttribute(k_predict, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int pb_ = (int)std::min<int64_t>((n_test + 127) / 128, 148 * 8);
-  k_predict<<<pb_, 128, smem>>>(d_tok, d_a, d_b, d_nn, K, d_beta, d_xc, (uint32_t)n_test, (uint32_t)ld, d_out);
-  CK(cudaGetLastError());
-  CK(cudaMemcpy(out, d_out, (size_t)n_test * sizeof(double), cudaMemcpyDeviceToHost));
-  cudaFree(d_tok); cudaFree(d_a); cudaFree(d_b); cudaFree(d_nn); cudaFree(d_beta); cudaFree(d_x); cudaFree(d_xc); cudaFree(d_out);
-  cudaSetDevice(prev_dev);     // a handle on another device may be in use by this thread
-  return 0;
-}
-
-int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
-                     const double* beta, const double* X, int64_t n_test, int32_t d, int32_t reduce, double* out, int32_t* n_used) {
-  if (!tok || !pa || !pb || !nn || !beta || !X || !out) return fail("bsr_predict_many: null argument");
-  if (M < 1 || K < 1 || K > BSR_MAXK || n_test < 1 || d < 1) return fail("bsr_predict_many: bad shape");
-  for (int g = 0; g < M * K; ++g) {
-    if (nn[g] < 1 || nn[g] > BSR_MAXN) return fail("bsr_predict_many: tree size out of range");
-    for (int j = 0; j < nn[g]; ++j)
-      if (tok_op(tok[(size_t)g * BSR_MAXN + j]) == OP_LEAF && tok_ft(tok[(size_t)g * BSR_MAXN + j]) >= d)
-        return fail("bsr_predict_many: a tree reads a feature the data does not have");
-  }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("bsr_predict_many: no CUDA device (no CPU fallback)");
-  int prev = 0;
-  cudaGetDevice(&prev);
-  CK(cudaSetDevice(device));
-  const size_t TN = (size_t)M * K * BSR_MAXN;
-  const int64_t ld = (n_test + 3) / 4 * 4;
-  // rows are processed in chunks so that the [M][chunk] prediction block stays below 256 MB
-  int64_t chunk = std::max<int64_t>(2048, ((int64_t)32 << 20) / M) / 2 * 2;
-  chunk = std::min<int64_t>(chunk, (n_test + 1) / 2 * 2);
-  uint32_t* d_tok = nullptr; double *d_a = nullptr, *d_b = nullptr, *d_x = nullptr, *d_xc = nullptr, *d_pred = nullptr, *d_beta = nullptr, *d_ms = nullptr;
-  int *d_nn = nullptr, *d_used = nullptr;
-  int rc = 0;
-  auto body = [&]() -> int {
-    CK(cudaMalloc((void**)&d_tok, TN * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&d_a, TN * sizeof(double)));
-    CK(cudaMalloc((void**)&d_b, TN * sizeof(double)));
-    CK(cudaMalloc((void**)&d_nn, (size_t)M * K * sizeof(int)));
-    CK(cudaMalloc((void**)&d_beta, (size_t)M * (K + 1) * sizeof(double)));
-    CK(cudaMalloc((void**)&d_x, (size_t)n_test * d * sizeof(double)));
-    CK(cudaMalloc((void**)&d_xc, (size_t)ld * d * sizeof(double)));
-    CK(cudaMalloc((void**)&d_pred, (size_t)M * chunk * sizeof(double)));
-    CK(cudaMalloc((void**)&d_ms, (size_t)2 * chunk * sizeof(double)));
-    CK(cudaMalloc((void**)&d_used, (size_t)chunk * sizeof(int)));
-    CK(cudaMemcpy(d_tok, tok, TN * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_a, pa, TN * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_b, pb, TN * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_nn, nn, (size_t)M * K * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_beta, beta, (size_t)M * (K + 1) * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_x, X, (size_t)n_test * d * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemset(d_xc, 0, (size_t)ld * d * sizeof(double)));
-    int blocks = (int)std::min<int64_t>((n_test * d + 255) / 256, 148 * 16);
-    k_transpose_in<double><<<blocks, 256>>>(d_x, d_xc, n_test, d, ld);
-    const size_t smem = (size_t)K * BSR_MAXN * sizeof(EvTok<double>);
-    CK(cudaFuncSetAttribute(k_predict_many, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int min_used = M;
-    std::vector<int> used_h((size_t)chunk);
-    for (int64_t r0 = 0; r0 < n_test; r0 += chunk) {
-      const int64_t rows = std::min<int64_t>(chunk, n_test - r0);
-      const int bx = (int)std::max<int64_t>(1, std::min<int64_t>(((rows + 1) / 2 + 127) / 128, 64));
-      k_predict_many<<<dim3(bx, M), 128, smem>>>(d_tok, d_a, d_b, d_nn, K, d_beta, d_xc, (uint32_t)ld, (uint32_t)r0, (uint32_t)rows, d_pred, (uint32_t)chunk);
-      CK(cudaGetLastError());
-      if (!reduce) {
-        CK(cudaMemcpy2D(out + r0, (size_t)n_test * sizeof(double), d_pred, (size_t)chunk * sizeof(double), (size_t)rows * sizeof(double), M,
-                        cudaMemcpyDeviceToHost));
-      } else {
-        k_predict_reduce<<<(unsigned)((rows + 127) / 128), 128>>>(d_pred, (uint32_t)chunk, M, (uint32_t)rows, d_ms, d_ms + chunk, d_used);
-        CK(cudaGetLastError());
-        CK(cudaMemcpy(out + r0, d_ms, (size_t)rows * sizeof(double), cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(out + n_test + r0, d_ms + chunk, (size_t)rows * sizeof(double), cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(used_h.data(), d_used, (size_t)rows * sizeof(int), cudaMemcpyDeviceToHost));
-        for (int64_t i = 0; i < rows; ++i) min_used = std::min(min_used, used_h[(size_t)i]);
-      }
-    }
-    if (n_used) *n_used = min_used;
-    return 0;
-  };
-  rc = body();
-  cudaFree(d_tok); cudaFree(d_a); cudaFree(d_b); cudaFree(d_nn); cudaFree(d_beta); cudaFree(d_x); cudaFree(d_xc); cudaFree(d_pred);
-  cudaFree(d_ms); cudaFree(d_used);
-  cudaSetDevice(prev);
-  return rc;
-}
-
-int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok, const double* ab,
-                       int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X, const int64_t* set_off, int32_t G,
-                       const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce, double* out,
-                       int32_t* n_used) {
-  const std::string f = "bsr_predict_groups: ";
+// The body of every prediction entry point: bsr_predict_groups (include/bsr_b200.h) and, through predict_dense, the dense ones;
+// `name` heads the error messages.
+static int predict_groups(const char* name, int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok,
+                          const double* ab, int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X, const int64_t* set_off,
+                          int32_t G, const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce,
+                          double* out, int32_t* n_used) {
+  const std::string f = std::string(name) + ": ";
   if (!nn || !tok || !ab || !beta || !X || !set_off || !grp_set || !grp_off || !grp_models || !grp_reduce || !out || !n_used)
     return fail(f + "null argument");
   if (M < 1 || K < 1 || K > BSR_MAXK || S < 1 || G < 1 || d < 1 || n_tok < 0 || n_lt < 0)
@@ -1291,6 +1174,53 @@ int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, 
   if (buf) cudaFree(buf);
   cudaSetDevice(prev);
   return rc;
+}
+
+int bsr_predict_groups(int32_t device, int32_t M, int32_t K, const int32_t* nn, const uint32_t* tok, int64_t n_tok, const double* ab,
+                       int64_t n_lt, const double* beta, int32_t S, int32_t d, const double* X, const int64_t* set_off, int32_t G,
+                       const int32_t* grp_set, const int64_t* grp_off, const int32_t* grp_models, const int32_t* grp_reduce, double* out,
+                       int32_t* n_used) {
+  return predict_groups("bsr_predict_groups", device, M, K, nn, tok, n_tok, ab, n_lt, beta, S, d, X, set_off, G, grp_set, grp_off,
+                        grp_models, grp_reduce, out, n_used);
+}
+
+// M dense models ([M][K][BSR_MAXN] slots) on one test set: packed into the layout of bsr_predict_groups and predicted as one group
+// of all M models.  nn is checked first, so the packing never reads past a tree's 64 slots.
+static int predict_dense(const char* name, int32_t device, int32_t M, int32_t K, const uint32_t* tok, const double* pa, const double* pb,
+                         const int32_t* nn, const double* beta, const double* X, int64_t n_test, int32_t d, int32_t reduce, double* out,
+                         int32_t* n_used) {
+  const std::string f = std::string(name) + ": ";
+  if (!tok || !pa || !pb || !nn || !beta || !X || !out) return fail(f + "null argument");
+  if (M < 1 || K < 1 || K > BSR_MAXK || n_test < 1 || d < 1) return fail(f + "bad shape");
+  std::vector<uint32_t> ptok;
+  std::vector<double> ab;
+  for (size_t t = 0; t < (size_t)M * K; ++t) {
+    if (nn[t] < 1 || nn[t] > BSR_MAXN) return fail(f + "tree size out of range (1 .. 64 nodes)");
+    for (size_t i = t * BSR_MAXN; i < t * BSR_MAXN + nn[t]; ++i) {
+      ptok.push_back(tok[i]);
+      if (tok_op(tok[i]) == OP_LT) { ab.push_back(pa[i]); ab.push_back(pb[i]); }
+    }
+  }
+  const double no_lt = 0.0;                         // a non-null ab when no tree has an lt node
+  const int64_t set_off[2] = {0, n_test}, grp_off[2] = {0, M};
+  std::vector<int32_t> models((size_t)M);
+  for (int32_t m = 0; m < M; ++m) models[(size_t)m] = m;
+  const int32_t grp_set = 0, grp_reduce = reduce != 0;
+  int32_t used = 0;
+  const int rc = predict_groups(name, device, M, K, nn, ptok.data(), (int64_t)ptok.size(), ab.empty() ? &no_lt : ab.data(),
+                                (int64_t)ab.size() / 2, beta, 1, d, X, set_off, 1, &grp_set, grp_off, models.data(), &grp_reduce, out, &used);
+  if (!rc && n_used) *n_used = used;
+  return rc;
+}
+
+int bsr_predict_trees(int32_t device, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
+                      const double* beta, const double* X, int64_t n_test, int32_t d, double* out) {
+  return predict_dense("bsr_predict_trees", device, 1, K, tok, pa, pb, nn, beta, X, n_test, d, 0, out, nullptr);
+}
+
+int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, const double* pa, const double* pb, const int32_t* nn,
+                     const double* beta, const double* X, int64_t n_test, int32_t d, int32_t reduce, double* out, int32_t* n_used) {
+  return predict_dense("bsr_predict_many", device, M, K, tok, pa, pb, nn, beta, X, n_test, d, reduce, out, n_used);
 }
 
 int bsr_predict(bsr_handle* h, int32_t chain, int32_t reported, const double* X, int64_t n_test, int32_t d, double* out) {

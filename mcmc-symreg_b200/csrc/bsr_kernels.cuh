@@ -3,7 +3,7 @@
 //   k_propose      Prop + auxProp + fStruc for K trees/chain    codes/funcs.py:1188-1210
 //   k_eval         allcal of the 2K columns + Gram reductions   codes/funcs.py:1212-1224, 1147-1157
 //   k_resolve      rank test, ylogLike, logR, accept, refit     codes/funcs.py:1226-1306, bsr_class.py:195-252
-//   k_eval_trees / k_predict   allcal / BSR.predict for arbitrary trees
+// (allcal / BSR.predict for arbitrary trees, k_eval_trees / k_predict_groups, are in bsr_misc_kernels.cuh)
 #pragma once
 #include "bsr_common.cuh"
 #include "bsr_eval.cuh"

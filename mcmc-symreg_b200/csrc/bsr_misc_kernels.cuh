@@ -1,4 +1,4 @@
-// Small utility kernels used by the host API (bsr_capi.cu): allcal / predict for explicit trees, layout
+// Small utility kernels used by the host API (bsr_capi.cu): allcal for explicit trees, prediction, layout
 // conversion, y statistics.
 #pragma once
 #include "bsr_common.cuh"
@@ -28,88 +28,6 @@ __global__ void k_eval_trees(const uint32_t* tok, const double* pa, const double
     for (int r = 0; r < R; ++r)
       if (q * R + r < n) out[(size_t)t * n + q * R + r] = (double)acc[r];
   }
-}
-
-// BSR.predict (bsr_class.py:53-68): out[row] = beta0 + sum_k beta_k * tree_k(X[row]), float64 evaluation.
-__global__ void k_predict(const uint32_t* tok, const double* pa, const double* pb, const int* nn, int K, const double* beta,
-                          const double* X, uint32_t n, uint32_t ld, double* out) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  EvTok<double>* s_tok = reinterpret_cast<EvTok<double>*>(smem_raw);
-  for (int j = threadIdx.x; j < K * BSR_MAXN; j += blockDim.x) {
-    int k = j / BSR_MAXN, i = j % BSR_MAXN;
-    if (i < nn[k]) {
-      EvTok<double> e;
-      e.op = tok_op(tok[j]); e.off = (uint32_t)tok_ft(tok[j]) * ld; e.a = pa[j]; e.b = pb[j];
-      s_tok[j] = e;
-    }
-  }
-  __syncthreads();
-  const uint32_t n_vec = (n + 1) / 2;
-  for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < n_vec; q += gridDim.x * blockDim.x) {
-    double v[2] = {beta[0], beta[0]};
-    for (int k = 0; k < K; ++k) {
-      double acc[2];
-      eval_tree_rows<double, 2>(s_tok + k * BSR_MAXN, nn[k], X, q * 2, acc);
-      v[0] += beta[k + 1] * acc[0];
-      v[1] += beta[k + 1] * acc[1];
-    }
-    if (q * 2 < n) out[q * 2] = v[0];
-    if (q * 2 + 1 < n) out[q * 2 + 1] = v[1];
-  }
-}
-
-// BSR.predict for M models at once (the restarts of one fit): blockIdx.y = model, pred[m][row] over rows [row0, row0 + rows).
-__global__ void k_predict_many(const uint32_t* tok, const double* pa, const double* pb, const int* nn, int K, const double* beta,
-                               const double* X, uint32_t ld, uint32_t row0, uint32_t rows, double* pred, uint32_t pred_ld) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  EvTok<double>* s_tok = reinterpret_cast<EvTok<double>*>(smem_raw);
-  const int m = blockIdx.y;
-  const size_t base = (size_t)m * K * BSR_MAXN;
-  for (int j = threadIdx.x; j < K * BSR_MAXN; j += blockDim.x) {
-    const int k = j / BSR_MAXN, i = j % BSR_MAXN;
-    if (i < nn[m * K + k]) {
-      EvTok<double> e;
-      const uint32_t t = tok[base + j];
-      e.op = tok_op(t); e.off = (uint32_t)tok_ft(t) * ld; e.a = pa[base + j]; e.b = pb[base + j];
-      s_tok[j] = e;
-    }
-  }
-  __syncthreads();
-  const double* b = beta + (size_t)m * (K + 1);
-  const uint32_t n_vec = (rows + 1) / 2;
-  for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < n_vec; q += gridDim.x * blockDim.x) {
-    double v[2] = {b[0], b[0]};
-    for (int k = 0; k < K; ++k) {
-      double acc[2];
-      eval_tree_rows<double, 2>(s_tok + k * BSR_MAXN, nn[m * K + k], X, row0 + q * 2, acc);
-      v[0] += b[k + 1] * acc[0];
-      v[1] += b[k + 1] * acc[1];
-    }
-    if (q * 2 < rows) pred[(size_t)m * pred_ld + q * 2] = v[0];
-    if (q * 2 + 1 < rows) pred[(size_t)m * pred_ld + q * 2 + 1] = v[1];
-  }
-}
-
-// Posterior-predictive mean and standard deviation over the M models, row by row, models in index order (deterministic);
-// a model whose prediction at a row is not finite is left out of that row.  used[row] = models that entered.
-__global__ void k_predict_reduce(const double* pred, uint32_t pred_ld, int M, uint32_t rows, double* mean, double* sd, int* used) {
-  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= rows) return;
-  double s = 0.0;
-  int cnt = 0;
-  for (int m = 0; m < M; ++m) {
-    const double v = pred[(size_t)m * pred_ld + r];
-    if (fabs(v) <= DBL_MAX) { s += v; ++cnt; }
-  }
-  const double mu = cnt ? s / cnt : nan("");
-  double q = 0.0;
-  for (int m = 0; m < M; ++m) {
-    const double v = pred[(size_t)m * pred_ld + r];
-    if (fabs(v) <= DBL_MAX) q += (v - mu) * (v - mu);
-  }
-  mean[r] = mu;
-  sd[r] = cnt > 1 ? sqrt(q / (cnt - 1)) : 0.0;
-  used[r] = cnt;
 }
 
 // The device tables of bsr_predict_groups (bsr_capi.cu).
@@ -142,9 +60,9 @@ struct GroupTables {
   int K, d;
 };
 
-// BSR.predict of many models, each on its own test set: rows [r0, r0 + chunk) of task blockIdx.x, blockIdx.y splits the rows.
-// The trees are staged from the packed layout (one warp per tree, the lt pairs located by a ballot over the node's lt flags); the
-// evaluation and the accumulation v = beta0 + beta_k * tree_k, k in order, are those of k_predict_many, so every value is its value.
+// BSR.predict (bsr_class.py:53-68) of many models, each on its own test set: rows [r0, r0 + chunk) of task blockIdx.x, blockIdx.y
+// splits the rows.  The trees are staged from the packed layout (one warp per tree, the lt pairs located by a ballot over the node's
+// lt flags) and evaluated in float64, two rows per thread: v = beta0 + beta_k * tree_k, accumulated over k in order.
 __global__ void k_predict_groups(GroupTables p, int64_t r0, int64_t chunk) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   EvTok<double>* s_tok = reinterpret_cast<EvTok<double>*>(smem_raw);
@@ -200,8 +118,9 @@ __global__ void k_predict_groups(GroupTables p, int64_t r0, int64_t chunk) {
   }
 }
 
-// Mean, sample standard deviation and used count over the models of reducing group red_grp[blockIdx.x], rows [r0, r0 + chunk) of its
-// set: the order, the two-pass formula and the finiteness test of k_predict_reduce.  mean goes to out + grp_out[g], std n rows later.
+// Posterior-predictive mean, sample standard deviation and used count over the models of reducing group red_grp[blockIdx.x], rows
+// [r0, r0 + chunk) of its set, row by row, models in index order (deterministic), two-pass; a model whose prediction at a row is not
+// finite is left out of that row.  mean goes to out + grp_out[g], std n rows later.
 __global__ void k_predict_groups_reduce(GroupTables p, int64_t r0, int64_t chunk) {
   const int g = p.red_grp[blockIdx.x];
   const int64_t n = p.n_rows[p.grp_set[g]];
@@ -237,18 +156,9 @@ __global__ void k_convert(const TI* in, TO* out, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = (TO)in[i];
 }
 
-// row-major float64 (n x d) -> column-major T (d x ld)
-template <typename TO>
-__global__ void k_transpose_in(const double* in, TO* out, int64_t n, int d, int64_t ld) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n * d; i += (int64_t)gridDim.x * blockDim.x) {
-    int64_t row = i / d;
-    int col = (int)(i % d);
-    out[(int64_t)col * ld + row] = (TO)in[i];
-  }
-}
-
-// The same for several data sets: data set b = blockIdx.y is rows row_off[b] .. row_off[b + 1] of the input and goes to
-// out + col_off[b] * d with leading dimension ld = col_off[b + 1] - col_off[b], with zeros on the rows past its own (up to ld).
+// row-major float64 -> column-major T for several data sets: data set b = blockIdx.y is rows row_off[b] .. row_off[b + 1] of the
+// input and goes to out + col_off[b] * d with leading dimension ld = col_off[b + 1] - col_off[b], with zeros on the rows past its own
+// (up to ld).
 // A handle's data sets share one ld (col_off[b] = b * ld); the test sets of bsr_predict_groups each have their own.
 template <typename TO>
 __global__ void k_transpose_datasets_in(const double* in, const int64_t* row_off, const int64_t* col_off, TO* out, int d) {

@@ -1,6 +1,7 @@
 """GPU tests of grouped prediction (bsr_predict_groups, capi.predict_groups, BSR.predict_many, experiments.summarize_many): every
-value is bit for bit what the single-estimator methods (bsr_predict_many) return, across row chunks, non-finite models and more
-models than one launch dimension of bsr_predict_many holds; malformed tables are refused before the device reads them."""
+value of the multi-fit route is bit for bit what the single-fit route returns (the single-estimator methods, and bsr_predict_many
+on dense models), across grouping, set offsets, row chunks, packing, non-finite models and more models than one launch dimension
+holds; malformed tables are refused before the device reads them."""
 import numpy as np
 import pytest
 
@@ -116,7 +117,8 @@ def _tiled(fits, M, seed):
 
 def test_more_models_than_one_launch_dimension(fits):
     """70000 models in one plain and one reducing group, on enough rows that the reduction runs in several chunks: the plain block
-    equals capi.predict_many over slices of at most 65535 models bit for bit, the reduction a float64 numpy mean / std to 1e-12"""
+    equals capi.predict_many over all the models and over slices of at most 65535 models bit for bit, the reduction a float64 numpy
+    mean / std to 1e-12"""
     from mcmc_symreg_b200 import capi
     M = 70000
     nn, tok, ab, beta = _tiled(fits, M, 54)
@@ -129,6 +131,7 @@ def test_more_models_than_one_launch_dimension(fits):
     assert [b.shape for b in blocks] == [(M, rows), (2, rows), (small.size, 3)]
     assert list(used) == [M, M, small.size]
     dense = capi.PackedTrees(nn, tok, ab).dense()
+    np.testing.assert_array_equal(blocks[0], capi.predict_many(0, *dense, beta, X))
     for lo in range(0, M, 65535):
         hi = min(M, lo + 65535)
         want = capi.predict_many(0, dense[0][lo:hi], dense[1][lo:hi], dense[2][lo:hi], dense[3][lo:hi], beta[lo:hi], X)

@@ -1,10 +1,14 @@
-"""Host logic of BSR.predict_many that needs no GPU: the argument errors it raises before any library call, the concatenated
-packed table it uploads, and the group tables it hands to capi.predict_groups."""
+"""Host logic of prediction that needs no GPU: the argument errors BSR.predict_many and the single-estimator methods raise before
+any library call, the concatenated packed table they upload, the group tables they hand to capi.predict_groups, and the malformed
+dense models bsr_predict_many and bsr_predict_trees refuse before they look for a device."""
+import ctypes
+
 import numpy as np
 import pytest
 
 from mcmc_symreg_b200 import BSR, capi
 from mcmc_symreg_b200 import experiments
+from mcmc_symreg_b200.trees import OP_ADD, OP_LT
 
 
 @pytest.fixture
@@ -78,6 +82,37 @@ def test_concatenated_table_decodes_to_each_fits_trees():
             np.testing.assert_array_equal(x[first[i]:first[i + 1]], y)
 
 
+def test_selected_models_decode_to_their_trees():
+    """PackedTrees.select: model j of the selection is model idx[j] of the table, in any order and with repeats"""
+    pk = _fake_fit(9, 4, np.random.default_rng(5))._packed_
+    for idx in ([3], [8, 0, 5], [2, 2, 7], list(range(9))):
+        for x, y in zip(pk.select(idx).dense(), pk.dense()):
+            np.testing.assert_array_equal(x, y[idx])
+
+
+def test_single_fit_predictions_upload_only_the_selected_models(monkeypatch):
+    """predict, predict_best and predict_mean hand capi.predict_groups one group over the selected restarts' own table"""
+    est = _fake_fit(6, 3, np.random.default_rng(6))
+    X = np.zeros((4, 2))
+    calls = []
+
+    def fake(device, nn, tok, ab, beta, sets, grp_set, grp_models, grp_reduce):
+        calls.append(dict(pk=capi.PackedTrees(nn, tok, ab), beta=beta, grp_models=[list(m) for m in grp_models], grp_reduce=grp_reduce))
+        n = sets[0].shape[0]
+        return [np.full((2, n), 7.0) if grp_reduce[0] else np.full((len(grp_models[0]), n), 5.0)], np.array([4], np.int32)
+
+    monkeypatch.setattr(capi, "predict_groups", fake)
+    assert est.predict(X, last_ind=2).shape == (4, 1)
+    m, s = est.predict_mean(X, chains=[4, 1], return_std=True)
+    assert m.shape == s.shape == (4, 1) and est.n_used_ == 4
+    for c, idx in zip(calls, ([4], [4, 1])):
+        assert c["grp_models"] == [list(range(len(idx)))]
+        np.testing.assert_array_equal(c["beta"], np.stack(est.betas_)[idx, :, 0])
+        for x, y in zip(c["pk"].dense(), est._packed_.dense()):
+            np.testing.assert_array_equal(x, y[idx])
+    assert [c["grp_reduce"] for c in calls] == [[False], [True]]
+
+
 def test_group_tables(monkeypatch):
     """what predict_many and summarize_many hand to capi.predict_groups: the concatenated models and betas, one group per fit (per
     fit and set for summarize_many) with global model indices, and the per-group results back in the methods' shapes"""
@@ -114,3 +149,69 @@ def test_group_tables(monkeypatch):
     assert c["grp_reduce"] == [False, False, True] * 9
     assert [f.n_used_ for f in fits] == [108, 117, 126]
     assert [float(rows[1]["test"][j][0]) for j in range(3)] == [12.0, 13.0, 140.0]
+
+
+def test_restart_index_out_of_range_before_any_library_call(no_library):
+    est = _fake_fit(4, 3, np.random.default_rng(4))
+    X = np.zeros((3, 2))
+    for call in (lambda: est.predict(X, last_ind=0), lambda: est.predict(X, last_ind=5),
+                 lambda: est.predict_mean(X, chains=[-1]), lambda: est.predict_mean(X, chains=[0, 4])):
+        with pytest.raises(IndexError, match="outside 0 .. 3"):
+            call()
+
+
+def _dense(M, K):
+    """M models of K trees (+ (lt x1) x0) in dense [M][K][64] slots"""
+    tok = np.zeros((M, K, capi.MAX_NODES), np.uint32)
+    tok[:, :, :4] = [OP_ADD, OP_LT, 1 << 16, 0]
+    pa, pb = np.full(tok.shape, 2.0), np.full(tok.shape, 0.5)
+    return dict(tok=tok, pa=pa, pb=pb, nn=np.full((M, K), 4, np.int32), beta=np.ones((M, K + 1)))
+
+
+def _predict_dense(entry, a, X):
+    lib = capi.load()
+    M, K = a["nn"].shape
+    p = {k: None if v is None else capi._ptr(v) for k, v in a.items()}
+    out = np.zeros((M, X.shape[0]))
+    if entry == "bsr_predict_trees":
+        rc = lib.bsr_predict_trees(0, K, p["tok"], p["pa"], p["pb"], p["nn"], p["beta"], capi._ptr(X), X.shape[0], X.shape[1],
+                                   capi._ptr(out))
+    else:
+        rc = lib.bsr_predict_many(0, M, K, p["tok"], p["pa"], p["pb"], p["nn"], p["beta"], capi._ptr(X), X.shape[0], X.shape[1], 0,
+                                  capi._ptr(out), ctypes.byref(ctypes.c_int32()))
+    capi._ck(rc)
+
+
+@pytest.mark.parametrize("entry", ["bsr_predict_many", "bsr_predict_trees"])
+def test_dense_entry_points_refuse_malformed_models(entry):
+    """each malformed model is refused on the host under the entry point's own name, before the library looks for a device"""
+    M = 3 if entry == "bsr_predict_many" else 1
+    X = np.zeros((5, 2))
+
+    def changed(name, index, value):
+        a = _dense(M, 2)
+        if value is None:
+            a[name] = None
+        else:
+            a[name][index] = value
+        return a
+
+    cases = [("unknown opcode", changed("tok", (M - 1, 1, 2), 11)),
+             ("not a pre-order tree", changed("tok", (M - 1, 1, 3), OP_ADD)),                    # a leaf turned into +
+             ("reads a feature the data does not have", changed("tok", (0, 0, 2), 2 << 16)),
+             ("tree size out of range", changed("nn", (M - 1, 0), 0)),
+             ("tree size out of range", changed("nn", (0, 1), 65)),
+             ("null argument", changed("pa", None, None))]
+    for match, a in cases:
+        with pytest.raises(capi.BsrError, match=entry + ": .*" + match):
+            _predict_dense(entry, a, X)
+
+
+@pytest.mark.parametrize("entry", ["bsr_predict_many", "bsr_predict_trees"])
+def test_dense_entry_points_have_no_cpu_fallback(entry):
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("GPU present")
+    M = 3 if entry == "bsr_predict_many" else 1
+    with pytest.raises(capi.BsrError, match=entry + r": no CUDA device \(no CPU fallback\)"):
+        _predict_dense(entry, _dense(M, 2), np.zeros((5, 2)))
