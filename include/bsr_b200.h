@@ -124,6 +124,19 @@ int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X_row
  * of different sizes in one run. */
 int bsr_set_datasets_ragged_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, const int64_t* n_rows,
                                  int32_t d, const int32_t* chain_dataset);
+/* Same, for data sets of different row and feature counts: data set b is n_rows[b] >= 1 rows x n_features[b] features (1 .. 65535),
+ * X_rowmajor holds the data sets one after another (data set b row-major, sum(n_rows[b] * n_features[b]) values) and y their values
+ * (sum(n_rows)).  The handle keeps X as [n_datasets][d][ld] with d the largest feature count (columns past a data set's own are zeros
+ * that no chain of it reads), so it holds n_datasets * d * ld values per precision -- ld the largest row count rounded up to 4 -- which
+ * must stay below 2^32; a suite of mostly narrow data sets beside one wide one pays for the wide one's columns.  Every chain draws its
+ * leaf features and charges its tree prior (log n_features per leaf) with its own data set's feature count: data set b is fitted as a
+ * handle holding only data set b fits it, bit for bit under the row-split condition of bsr_set_datasets_ragged_host, which is the case
+ * of one feature count.  The same refusals, checked before any data is read, and the same failure behaviour.  Further refusals once
+ * the data sets differ in feature count: replacing the data so that an initialised chain gets fewer features than its trees were grown
+ * on (here and in every other bsr_set_data*), and a bsr_set_state tree with a leaf feature >= its chain's feature count; bsr_predict
+ * compares d with the chain's own feature count.  Fits a benchmark suite of problems with 1 to 9 inputs in one run. */
+int bsr_set_datasets_mixed_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, const int64_t* n_rows,
+                                const int32_t* n_features, const int32_t* chain_dataset);
 
 /* Prior initialisation of every chain: sigma ~ IG(1), per tree sigma_a, sigma_b ~ IG(1) and grow()
  * (codes/bsr_class.py:123-142, codes/funcs.py:74-119), then the initial intercept OLS (bsr_class.py:147-163). */

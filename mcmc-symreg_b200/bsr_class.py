@@ -110,7 +110,7 @@ class BSR(BaseEstimator, RegressorMixin):
             print("chains: %d  proposals: %d  accepts: %d  rank-rejects: %d" % (MM, c[:, 0].sum(), c[:, 1].sum(), c[:, 2].sum()))
         return
 
-    def fit_many(self, datasets, seeds=None, *, ragged=False):
+    def fit_many(self, datasets, seeds=None, *, ragged=False, mixed_features=False):
         """Fit this estimator to each of several data sets in one GPU run; returns one fitted ``BSR`` per data set.
 
         ``datasets``: a sequence of (X, y) pairs of the same shape (n rows, d features); with ``ragged=True`` the row counts may
@@ -124,14 +124,20 @@ class BSR(BaseEstimator, RegressorMixin):
         count and the results agree up to the fp64 summation order of the splits.  With ``ragged=True`` the batch takes the
         geometry of its largest data set, and data set b is identical to its fit when its n_b rows fit in the batch's first row
         split and its own fit runs one split (always below 16384 rows), else equal up to the fp64 summation order of the splits.
-        With equal row counts ``ragged=True`` gives the estimators ``ragged=False`` gives.  ``n_sweeps_`` reports the sweeps of the
+        With equal row counts ``ragged=True`` gives the estimators ``ragged=False`` gives.  With ``mixed_features=True`` the row counts
+        and the numbers of features may both differ (a benchmark suite of problems with 1 to 9 inputs): every data set's chains draw
+        their leaf features from its own d_b features and charge its own tree prior, so data set b is identical to its fit under the
+        condition ``ragged=True`` states (n_b in the batch's first row split, its own fit one split: always below 16384 rows), else
+        equal up to the fp64 summation order of the splits.  The device holds every data set with the columns of the widest (zeros
+        no chain reads), B * d_max * n_max values per precision.  With one feature count ``mixed_features=True`` gives the
+        estimators ``ragged=True`` gives.  ``n_sweeps_`` reports the sweeps of the
         whole batch (the stop rules are checked for all chains together), not the count a single fit would have needed.
 
         ``seeds``: one seed per data set; None gives every data set ``self.seed``, or, when that is None, draws one seed per
         data set from numpy's global state, in order, exactly as a loop of ``fit`` calls would.  The returned estimators
         carry the parameters of ``self``."""
         data = [(_as_matrix(X), np.asarray(y, dtype=np.float64).ravel()) for X, y in datasets]
-        check_datasets(data, ragged)
+        check_datasets(data, ragged, mixed_features)
         B = len(data)
         seeds = dataset_seeds(self.seed, B, seeds)
         MM, K = int(self.itrNum), int(self.treeNum)
@@ -148,7 +154,9 @@ class BSR(BaseEstimator, RegressorMixin):
             try:
                 g = np.arange(lo, hi)
                 ds, ids = g // MM, g % MM
-                if ragged:
+                if mixed_features:
+                    eng.set_datasets_mixed([X for X, _ in data], [y for _, y in data], ds)
+                elif ragged:
                     eng.set_datasets_ragged([X for X, _ in data], [y for _, y in data], ds)
                 else:
                     eng.set_datasets(np.stack([X for X, _ in data]), np.stack([y for _, y in data]), ds)
@@ -342,18 +350,22 @@ class _LazyRoots:
         return dict(_pk=self._pk, _cache={})
 
 
-def check_datasets(data, ragged=False):
-    """``fit_many``'s data sets, as (X (n, d), y) pairs, must share n (unless ``ragged``) and d, and each X must agree with its y:
-    else ValueError."""
+def check_datasets(data, ragged=False, mixed_features=False):
+    """``fit_many``'s data sets, as (X (n, d), y) pairs, must share n (unless ``ragged`` or ``mixed_features``) and d (unless
+    ``mixed_features``), and each X must agree with its y: else ValueError."""
     if len(data) == 0:
         raise ValueError("fit_many: no data sets")
     n, d = data[0][0].shape
     for b, (X, y) in enumerate(data):
         if X.shape[0] != y.shape[0]:
             raise ValueError("fit_many: data set %d: train_data and train_y disagree on the number of rows" % b)
+        if mixed_features:
+            if X.shape[1] < 1:
+                raise ValueError("fit_many: data set %d has no features" % b)
+            continue
         if ragged and X.shape[1] != d:
             raise ValueError("fit_many: data set %d has %d features, data set 0 has %d: all data sets must have the same number of features"
-                             % (b, X.shape[1], d))
+                             " (mixed_features=True accepts different feature counts)" % (b, X.shape[1], d))
         if not ragged and X.shape != (n, d):
             raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape%s"
                              % (b, X.shape[0], X.shape[1], n, d, " (ragged=True accepts different row counts)" if X.shape[1] == d else ""))

@@ -35,6 +35,7 @@ _SIGS = {
     "bsr_set_data_device": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, C.c_int64, C.c_int64]),
     "bsr_set_datasets_host": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, C.c_int32, _P]),
     "bsr_set_datasets_ragged_host": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P]),
+    "bsr_set_datasets_mixed_host": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "bsr_init_chains": (C.c_int, [_P, C.c_uint64]),
     "bsr_init_chains_keyed": (C.c_int, [_P, _P, _P]),
     "bsr_set_state": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_uint64]),
@@ -140,28 +141,36 @@ def predict_many(device, tok, pa, pb, nn, beta, X, reduce=False):
 
 def predict_groups(device, nn, tok, ab, beta, test_sets, grp_set, grp_models, grp_reduce):
     """Many models on many test sets in one call (``bsr_predict_groups``).  Models packed as ``PackedTrees`` holds them: nn [M][K],
-    tok the tokens of tree after tree, ab [n_lt][2]; beta [M][K+1].  ``test_sets``: S arrays (n_s, d), one d.  Group g evaluates the
+    tok the tokens of tree after tree, ab [n_lt][2]; beta [M][K+1].  ``test_sets``: S arrays (n_s, d_s).  Group g evaluates the
     model indices ``grp_models[g]`` on ``test_sets[grp_set[g]]``.  Returns (blocks, n_used): blocks[g] is (n_models_g, n_s), or, for
     ``grp_reduce[g]``, (2, n_s) with the mean over the models and their standard deviation (what ``predict_many`` returns for
-    reduce=False / True); n_used [G] the smallest number of models any row of a group used."""
-    lib = load()
+    reduce=False / True); n_used [G] the smallest number of models any row of a group used.
+
+    Test sets of different widths (the fits of ``fit_many(mixed_features=True)``) go to the library padded with zero columns to the
+    widest; first, every model of a group must read only features below the width of its own test set (else ValueError), the check
+    the library makes against the one width it is given."""
     nn = np.ascontiguousarray(nn, dtype=np.int32)
     M, K = nn.shape
     tok = np.ascontiguousarray(tok, dtype=np.uint32).ravel()
     ab = np.ascontiguousarray(ab, dtype=np.float64).reshape(-1, 2)
     beta = np.ascontiguousarray(beta, dtype=np.float64).reshape(M, K + 1)
     Xs = [np.asarray(X, dtype=np.float64) for X in test_sets]
-    if not Xs or any(X.ndim != 2 or X.shape[1] != Xs[0].shape[1] for X in Xs):
-        raise ValueError("predict_groups: test_sets must be one or more (n_s, d) arrays of the same d")
-    set_off = np.zeros(len(Xs) + 1, dtype=np.int64)
-    np.cumsum([X.shape[0] for X in Xs], out=set_off[1:])
-    X = np.ascontiguousarray(np.concatenate(Xs, axis=0))
+    if not Xs or any(X.ndim != 2 for X in Xs):
+        raise ValueError("predict_groups: test_sets must be one or more (n_s, d_s) arrays")
     models = [np.asarray(m, dtype=np.int32).ravel() for m in grp_models]
     G = len(models)
     grp_set = np.ascontiguousarray(grp_set, dtype=np.int32).ravel()
     grp_reduce = np.ascontiguousarray([int(bool(r)) for r in grp_reduce], dtype=np.int32)
     if grp_set.size != G or grp_reduce.size != G or G == 0:
         raise ValueError("predict_groups: grp_set, grp_models and grp_reduce must describe the same one or more groups")
+    widths = np.array([X.shape[1] for X in Xs], dtype=np.int64)
+    if np.any(widths != widths[0]):
+        _check_group_features(nn, tok, widths, grp_set, models)
+        d = int(widths.max())
+        Xs = [X if X.shape[1] == d else np.pad(X, ((0, 0), (0, d - X.shape[1]))) for X in Xs]
+    set_off = np.zeros(len(Xs) + 1, dtype=np.int64)
+    np.cumsum([X.shape[0] for X in Xs], out=set_off[1:])
+    X = np.ascontiguousarray(np.concatenate(Xs, axis=0))
     grp_off = np.zeros(G + 1, dtype=np.int64)
     np.cumsum([m.size for m in models], out=grp_off[1:])
     flat = np.ascontiguousarray(np.concatenate(models))
@@ -169,11 +178,33 @@ def predict_groups(device, nn, tok, ab, beta, test_sets, grp_set, grp_models, gr
     sizes = np.where(grp_reduce != 0, 2, grp_off[1:] - grp_off[:-1]) * rows
     out = np.zeros(int(sizes.sum()))
     used = np.zeros(G, dtype=np.int32)
+    lib = load()
     _ck(lib.bsr_predict_groups(int(device), M, K, _ptr(nn), _ptr(tok), tok.size, _ptr(ab), ab.shape[0], _ptr(beta), len(Xs), X.shape[1],
                                _ptr(X), _ptr(set_off), G, _ptr(grp_set), _ptr(grp_off), _ptr(flat), _ptr(grp_reduce), _ptr(out), _ptr(used)))
     ends = np.cumsum(sizes)
     blocks = [out[e - z:e].reshape(-1, int(r)) for e, z, r in zip(ends, sizes, rows)]
     return blocks, used
+
+
+def _check_group_features(nn, tok, widths, grp_set, models):
+    """Every model of group g reads only features below widths[grp_set[g]]: else ValueError.  Vectorised over the packed tokens; a
+    table whose node counts do not cover tok, or a group naming a model or test set that does not exist, is left to the library's
+    own refusals."""
+    M, K = nn.shape
+    if np.any(nn < 0) or int(nn.sum()) != tok.size:
+        return
+    model_of = np.repeat(np.arange(M * K) // K, nn.ravel())
+    leaf = (tok & 0xFF) == 0
+    widest = np.full(M, -1, dtype=np.int64)             # largest leaf feature of every model
+    np.maximum.at(widest, model_of[leaf], (tok[leaf] >> 16).astype(np.int64))
+    for g, (s, m) in enumerate(zip(grp_set, models)):
+        if not 0 <= s < widths.size:
+            continue
+        m = m[(m >= 0) & (m < M)]
+        over = m[widest[m] >= widths[s]]
+        if over.size:
+            raise ValueError("predict_groups: group %d: model %d reads feature %d, its test set %d has %d features"
+                             % (g, int(over[0]), int(widest[over[0]]), int(s), int(widths[s])))
 
 
 class PackedTrees:
@@ -330,6 +361,25 @@ class Engine:
         y = np.ascontiguousarray(np.concatenate(ys))
         _ck(self._lib.bsr_set_datasets_ragged_host(self._h, len(Xs), _ptr(X), _ptr(y), _ptr(n_rows), d, _ptr(cd)))
         self.n, self.d = int(n_rows.max()), d
+
+    def set_datasets_mixed(self, Xs, ys, chain_dataset):
+        """D data sets of any row and feature counts: Xs a sequence of (n_b, d_b) arrays, ys of (n_b,) arrays; chain c fits data set
+        ``chain_dataset[c]`` with its own d_b features.  ``n`` becomes the largest row count, ``d`` the largest feature count."""
+        Xs = [np.asarray(X, dtype=np.float64) for X in Xs]
+        ys = [np.asarray(y, dtype=np.float64).ravel() for y in ys]
+        if len(Xs) == 0 or len(Xs) != len(ys):
+            raise ValueError("set_datasets_mixed: one y per X, and at least one data set")
+        if any(X.ndim != 2 or X.shape[0] != y.shape[0] for X, y in zip(Xs, ys)):
+            raise ValueError("set_datasets_mixed: every X must be (n_b, d_b) and its y (n_b,)")
+        cd = np.ascontiguousarray(chain_dataset, dtype=np.int32).ravel()
+        if cd.size != self.C:
+            raise ValueError("chain_dataset must hold one data set index per chain")
+        n_rows = np.array([X.shape[0] for X in Xs], dtype=np.int64)
+        n_features = np.array([X.shape[1] for X in Xs], dtype=np.int32)
+        X = np.ascontiguousarray(np.concatenate([X.ravel() for X in Xs]))
+        y = np.ascontiguousarray(np.concatenate(ys))
+        _ck(self._lib.bsr_set_datasets_mixed_host(self._h, len(Xs), _ptr(X), _ptr(y), _ptr(n_rows), _ptr(n_features), _ptr(cd)))
+        self.n, self.d = int(n_rows.max()), int(n_features.max())
 
     def set_data_device(self, x_ptr, y_ptr, n, d, ld, n_total=0):
         self.n, self.d = int(n), int(d)

@@ -104,6 +104,7 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
   rc |= dalloc(h, &st.key_seed, (size_t)C);
   rc |= dalloc(h, &st.key_id, (size_t)C);
   rc |= dalloc(h, &st.ds, (size_t)C);
+  rc |= dalloc(h, &h->chain_pt, (size_t)C);
   const int P = 2 * K;
   rc |= dalloc(h, &h->gram, (size_t)2 * C * (gram_n_sum(P) + P));   // [sums | maxs | per-chain scratch records]
   rc |= dalloc(h, &h->need64, (size_t)C);
@@ -139,11 +140,11 @@ int bsr_destroy(bsr_handle* h) {
   return 0;
 }
 
-static int build_tables(bsr_handle* h) {
-  PriorTables& pt = h->pt;
+static PriorTables prior_tables(const bsr_handle* h, int n_feature) {
+  PriorTables pt;
   memset(&pt, 0, sizeof pt);
   pt.n_ops = h->cfg.n_ops;
-  pt.n_feature = h->d;
+  pt.n_feature = n_feature;
   pt.beta = h->cfg.beta;
   double acc = 0;
   for (int i = 0; i < pt.n_ops; ++i) {
@@ -159,10 +160,35 @@ static int build_tables(bsr_handle* h) {
     pt.logsplit[dpt] = log((double)(1 + dpt)) * h->cfg.beta;  // codes/funcs.py:370
     pt.log1m[dpt] = log(1.0 - ps);                            // codes/funcs.py:362-363 (-inf at depth 0)
   }
-  pt.lognf = log((double)h->d);
-  if (!h->d_pt && dalloc(h, &h->d_pt, 1)) return 1;
-  CK(cudaMemcpy(h->d_pt, &pt, sizeof pt, cudaMemcpyHostToDevice));
+  pt.lognf = log((double)n_feature);
+  return pt;
+}
+
+// One table per distinct feature count of the data sets (a table is ~2 KB; a handle may hold 65535 data sets), and the table
+// of every chain's data set (chain_pt).  A handle of one feature count has one table, entry 0, and every chain reads it.
+static int build_tables(bsr_handle* h) {
+  std::vector<int32_t> counts(h->ds_d);
+  std::sort(counts.begin(), counts.end());
+  counts.erase(std::unique(counts.begin(), counts.end()), counts.end());
+  std::vector<PriorTables> pt;
+  for (int32_t d : counts) pt.push_back(prior_tables(h, d));
+  if ((int)pt.size() != h->n_pt) {
+    dfree(h, h->d_pt);
+    h->d_pt = nullptr; h->n_pt = 0;
+    if (dalloc(h, &h->d_pt, pt.size())) return 1;
+    h->n_pt = (int)pt.size();
+  }
+  CK(cudaMemcpy(h->d_pt, pt.data(), pt.size() * sizeof(PriorTables), cudaMemcpyHostToDevice));
+  std::vector<int> idx((size_t)h->st.C);
+  for (int c = 0; c < h->st.C; ++c)
+    idx[(size_t)c] = (int)(std::lower_bound(counts.begin(), counts.end(), h->ds_d[(size_t)h->chain_ds[(size_t)c]]) - counts.begin());
+  CK(cudaMemcpy(h->chain_pt, idx.data(), idx.size() * sizeof(int), cudaMemcpyHostToDevice));
   return 0;
+}
+
+// feature count of chain c's data set
+static int32_t chain_features(const bsr_handle* h, int c) {
+  return h->chain_ds.empty() ? h->d : h->ds_d[(size_t)h->chain_ds[(size_t)c]];
 }
 
 static int setup_col_cache(bsr_handle* h) {
@@ -204,10 +230,10 @@ static void free_data(bsr_handle* h) {
   h->X32 = nullptr; h->y32 = nullptr; h->X64 = nullptr; h->y64 = nullptr;
 }
 
-// Number of data sets, their row counts (nullptr: all of h->n rows) and the data set of every chain (nullptr: all chains on data set
-// 0), committed once the data of the D data sets is in place.  On failure the caller drops the data (free_data): no entry point then
-// runs on chains that name data sets the handle does not hold.
-static int set_chain_datasets(bsr_handle* h, int D, const int64_t* n_rows, const int32_t* chain_dataset) {
+// Number of data sets, their row counts (nullptr: all of h->n rows), their feature counts and the data set of every chain (nullptr:
+// all chains on data set 0), committed once the data of the D data sets is in place.  On failure the caller drops the data
+// (free_data): no entry point then runs on chains that name data sets the handle does not hold.
+static int set_chain_datasets(bsr_handle* h, int D, const int64_t* n_rows, const int32_t* n_features, const int32_t* chain_dataset) {
   if (D != h->n_ds) {
     double* ys = nullptr;
     uint32_t* dn = nullptr;
@@ -221,15 +247,48 @@ static int set_chain_datasets(bsr_handle* h, int D, const int64_t* n_rows, const
   CK(cudaMemcpy(h->ds_n, dn.data(), (size_t)D * sizeof(uint32_t), cudaMemcpyHostToDevice));
   if (chain_dataset) CK(cudaMemcpy(h->st.ds, chain_dataset, (size_t)h->st.C * sizeof(int), cudaMemcpyHostToDevice));
   else CK(cudaMemset(h->st.ds, 0, (size_t)h->st.C * sizeof(int)));
+  h->ds_d.assign(n_features, n_features + D);
+  if (chain_dataset) h->chain_ds.assign(chain_dataset, chain_dataset + h->st.C);
+  else h->chain_ds.assign((size_t)h->st.C, 0);
+  h->mixed = std::any_of(h->ds_d.begin(), h->ds_d.end(), [&](int32_t v) { return v != h->ds_d[0]; });
   return 0;
 }
 
-// D data sets of n_rows[b] rows x d features from host memory (X row-major, the data sets' rows one after another; y likewise) into
-// the handle's buffers: X [D][d][ld], y [D][ld] with ld the largest row count rounded up to 4, zeros past a data set's own rows.
-static int upload_host(bsr_handle* h, int D, const double* X, const double* y, const int64_t* n_rows, int32_t d, int64_t n_total) {
-  std::vector<int64_t> off((size_t)D + 1, 0);       // first row of every data set in X / y, then the total
+// Replacing the data under initialised chains when the old or the new data sets differ in feature count: no chain may end up with
+// fewer features than its trees were grown on (a leaf would read a column of zeros).  n_features [D], chain_dataset [C].  (Handles of
+// one feature count keep their behaviour: the caller answers for the trees there, as bsr_set_state leaves it to them.)
+static int check_live_features(const bsr_handle* h, const char* fn, int D, const int32_t* n_features, const int32_t* chain_dataset) {
+  if (!h->initialised || !h->X32 || h->chain_ds.empty()) return 0;
+  if (!h->mixed && std::all_of(n_features, n_features + D, [&](int32_t v) { return v == n_features[0]; })) return 0;
+  for (int c = 0; c < h->st.C; ++c) {
+    const int32_t now = chain_features(h, c), next = n_features[chain_dataset[c]];
+    if (next < now) {
+      char msg[240];
+      snprintf(msg, sizeof msg, "%s: chain %d has trees over %d features and would get a data set of %d features (load it into a new "
+               "handle)", fn, c, (int)now, (int)next);
+      return fail(msg);
+    }
+  }
+  return 0;
+}
+
+// D data sets of n_rows[b] rows x n_features[b] features from host memory (X row-major, the data sets one after another; y likewise)
+// into the handle's buffers: X [D][d][ld], y [D][ld] with ld the largest row count rounded up to 4 and d the largest feature count,
+// zeros past a data set's own rows and columns.
+static int upload_host(bsr_handle* h, int D, const double* X, const double* y, const int64_t* n_rows, const int32_t* n_features,
+                       int64_t n_total) {
+  // staged tables: first row of every data set in y, then the first column element of every data set in the handle's X (b * ld), then
+  // the first element of every data set in X (each the totals at [D]), then the feature counts
+  const size_t D1 = (size_t)D + 1;
+  std::vector<int64_t> off(3 * D1, 0);
   int64_t n = 0;
-  for (int b = 0; b < D; ++b) { off[(size_t)b + 1] = off[(size_t)b] + n_rows[b]; n = std::max(n, n_rows[b]); }
+  int32_t d = 0;
+  for (int b = 0; b < D; ++b) {
+    off[(size_t)b + 1] = off[(size_t)b] + n_rows[b];
+    off[2 * D1 + b + 1] = off[2 * D1 + b] + n_rows[b] * n_features[b];
+    n = std::max(n, n_rows[b]);
+    d = std::max(d, n_features[b]);
+  }
   const int64_t rows = off[(size_t)D];
   const bool same_shape = h->own_x32 && h->X32 != nullptr && h->n == n && h->d == d && h->n_ds == D;
   const size_t ld = (size_t)(n + 3) / 4 * 4;
@@ -240,10 +299,10 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, c
     h->own_x32 = true;
     if (dalloc(h, &h->X32, D * ld * d) || dalloc(h, &h->X64, D * ld * d) || dalloc(h, &h->y32, D * ld) || dalloc(h, &h->y64, D * ld)) return 1;
   }
-  off.resize(2 * ((size_t)D + 1));                   // then the first column element of every data set: b * ld (one ld for all)
-  for (int b = 0; b <= D; ++b) off[(size_t)D + 1 + b] = (int64_t)b * (int64_t)ld;
-  // staging: X, then y, then the row and column offsets
-  const size_t xs = (size_t)rows * d, bytes = (xs + (size_t)rows) * sizeof(double) + off.size() * sizeof(int64_t);
+  for (int b = 0; b <= D; ++b) off[D1 + b] = (int64_t)b * (int64_t)ld;
+  // staging: X, then y, then the offsets, then the feature counts
+  const size_t xs = (size_t)off[3 * D1 - 1];
+  const size_t bytes = (xs + (size_t)rows) * sizeof(double) + off.size() * sizeof(int64_t) + (size_t)D * sizeof(int32_t);
   if (bytes > h->stage_bytes) {
     CK(cudaDeviceSynchronize());
     if (h->stage) cudaFree(h->stage);
@@ -253,34 +312,40 @@ static int upload_host(bsr_handle* h, int D, const double* X, const double* y, c
   }
   double* ystage = h->stage + xs;
   int64_t* d_off = reinterpret_cast<int64_t*>(ystage + rows);
-  int64_t* d_col = d_off + D + 1;
+  int32_t* d_nf = reinterpret_cast<int32_t*>(d_off + off.size());
   h->n_total = n_total > 0 ? n_total : n;
   // stream-ordered after any sweep still in flight on the default stream; the copies from pageable memory are synchronous
   CK(cudaMemcpy(h->stage, X, xs * sizeof(double), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(ystage, y, (size_t)rows * sizeof(double), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(d_off, off.data(), off.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(d_nf, n_features, (size_t)D * sizeof(int32_t), cudaMemcpyHostToDevice));
   // one launch per buffer for all D data sets (blockIdx.y); y is the one-column case
   const dim3 blocks((unsigned)std::min<int64_t>(((int64_t)ld * d + 255) / 256, 148 * 16), (unsigned)D);
-  k_transpose_datasets_in<float><<<blocks, 256>>>(h->stage, d_off, d_col, h->X32, d);
-  k_transpose_datasets_in<double><<<blocks, 256>>>(h->stage, d_off, d_col, h->X64, d);
-  k_transpose_datasets_in<float><<<blocks, 256>>>(ystage, d_off, d_col, h->y32, 1);
-  k_transpose_datasets_in<double><<<blocks, 256>>>(ystage, d_off, d_col, h->y64, 1);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(h->stage, d_off, d_off + D1, d_off + 2 * D1, d_nf, h->X32, d);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(h->stage, d_off, d_off + D1, d_off + 2 * D1, d_nf, h->X64, d);
+  k_transpose_datasets_in<float><<<blocks, 256>>>(ystage, d_off, d_off + D1, nullptr, nullptr, h->y32, 1);
+  k_transpose_datasets_in<double><<<blocks, 256>>>(ystage, d_off, d_off + D1, nullptr, nullptr, h->y64, 1);
   CK(cudaGetLastError());
   return 0;
 }
 
-// The checks every host upload makes before it reads any data, then the upload.  n_rows: D row counts (the caller checked them >= 1).
-static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, const double* y, const int64_t* n_rows, int32_t d,
-                         int64_t n_total, const int32_t* chain_dataset) {
+// The checks every host upload makes before it reads any data, then the upload.  n_rows, n_features: D row and feature counts (the
+// caller checked them); chain_dataset: nullptr (all chains on data set 0) or C indices in [0, D).
+static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, const double* y, const int64_t* n_rows,
+                         const int32_t* n_features, int64_t n_total, const int32_t* chain_dataset) {
   const std::string f(fn);
-  if (d < 1 || d > 65535) return fail(f + ": need n >= 1 and 1 <= d <= 65535");
   int64_t n = 0;
-  for (int b = 0; b < D; ++b) n = std::max(n, n_rows[b]);
+  int32_t d = 0;
+  for (int b = 0; b < D; ++b) { n = std::max(n, n_rows[b]); d = std::max(d, n_features[b]); }
+  if (d < 1 || d > 65535) return fail(f + ": need n >= 1 and 1 <= d <= 65535");
   if ((n + 3) / 4 * 4 * (int64_t)d * D >= (int64_t)1 << 32)
     return fail(f + ": n_datasets * d * n (the largest row count) must stay below 2^32 elements per device (shard the rows, or fit fewer data "
                 "sets per handle)");
+  const std::vector<int32_t> one_ds(chain_dataset ? 0 : (size_t)h->st.C, 0);
+  if (!chain_dataset) chain_dataset = one_ds.data();
+  if (check_live_features(h, fn, D, n_features, chain_dataset)) return 1;
   CK(cudaSetDevice(h->cfg.device));
-  if (upload_host(h, D, X, y, n_rows, d, n_total) || set_chain_datasets(h, D, n_rows, chain_dataset)) {
+  if (upload_host(h, D, X, y, n_rows, n_features, n_total) || set_chain_datasets(h, D, n_rows, n_features, chain_dataset)) {
     free_data(h);
     return 1;
   }
@@ -290,7 +355,7 @@ static int set_data_host(bsr_handle* h, const char* fn, int D, const double* X, 
 int bsr_set_data_host(bsr_handle* h, const double* X, const double* y, int64_t n, int32_t d, int64_t n_total) {
   if (!h || !X || !y) return fail("bsr_set_data_host: null argument");
   if (n < 1) return fail("bsr_set_data_host: need n >= 1 and 1 <= d <= 65535");
-  return set_data_host(h, "bsr_set_data_host", 1, X, y, &n, d, n_total, nullptr);
+  return set_data_host(h, "bsr_set_data_host", 1, X, y, &n, &d, n_total, nullptr);
 }
 
 // the refusals of every call that loads several data sets
@@ -316,20 +381,44 @@ int bsr_set_datasets_host(bsr_handle* h, int32_t n_datasets, const double* X, co
   if (check_datasets(h, "bsr_set_datasets_host", n_datasets, chain_dataset)) return 1;
   if (n < 1) return fail("bsr_set_datasets_host: need n >= 1 and 1 <= d <= 65535");
   const std::vector<int64_t> n_rows((size_t)n_datasets, n);
-  return set_data_host(h, "bsr_set_datasets_host", n_datasets, X, y, n_rows.data(), d, 0, chain_dataset);
+  const std::vector<int32_t> n_features((size_t)n_datasets, d);
+  return set_data_host(h, "bsr_set_datasets_host", n_datasets, X, y, n_rows.data(), n_features.data(), 0, chain_dataset);
+}
+
+// Data sets of any row and feature counts: the refusals of bsr_set_datasets_mixed_host (include/bsr_b200.h), then the upload.
+// n_features nullptr: every data set has d features (bsr_set_datasets_ragged_host).
+static int set_datasets_mixed(bsr_handle* h, const char* fn, int32_t n_datasets, const double* X, const double* y, const int64_t* n_rows,
+                              const int32_t* n_features, int32_t d, const int32_t* chain_dataset) {
+  if (check_datasets(h, fn, n_datasets, chain_dataset)) return 1;
+  for (int b = 0; b < n_datasets; ++b)
+    if (n_rows[b] < 1) {
+      char msg[160];
+      snprintf(msg, sizeof msg, "%s: n_rows[%d] = %lld: every data set needs at least one row", fn, b, (long long)n_rows[b]);
+      return fail(msg);
+    }
+  std::vector<int32_t> nf((size_t)n_datasets, d);
+  if (n_features) {
+    for (int b = 0; b < n_datasets; ++b)
+      if (n_features[b] < 1 || n_features[b] > 65535) {
+        char msg[160];
+        snprintf(msg, sizeof msg, "%s: n_features[%d] = %d is outside 1 .. 65535", fn, b, (int)n_features[b]);
+        return fail(msg);
+      }
+    nf.assign(n_features, n_features + n_datasets);
+  }
+  return set_data_host(h, fn, n_datasets, X, y, n_rows, nf.data(), 0, chain_dataset);
 }
 
 int bsr_set_datasets_ragged_host(bsr_handle* h, int32_t n_datasets, const double* X, const double* y, const int64_t* n_rows, int32_t d,
                                  const int32_t* chain_dataset) {
   if (!h || !X || !y || !n_rows || !chain_dataset) return fail("bsr_set_datasets_ragged_host: null argument");
-  if (check_datasets(h, "bsr_set_datasets_ragged_host", n_datasets, chain_dataset)) return 1;
-  for (int b = 0; b < n_datasets; ++b)
-    if (n_rows[b] < 1) {
-      char msg[160];
-      snprintf(msg, sizeof msg, "bsr_set_datasets_ragged_host: n_rows[%d] = %lld: every data set needs at least one row", b, (long long)n_rows[b]);
-      return fail(msg);
-    }
-  return set_data_host(h, "bsr_set_datasets_ragged_host", n_datasets, X, y, n_rows, d, 0, chain_dataset);
+  return set_datasets_mixed(h, "bsr_set_datasets_ragged_host", n_datasets, X, y, n_rows, nullptr, d, chain_dataset);
+}
+
+int bsr_set_datasets_mixed_host(bsr_handle* h, int32_t n_datasets, const double* X, const double* y, const int64_t* n_rows,
+                                const int32_t* n_features, const int32_t* chain_dataset) {
+  if (!h || !X || !y || !n_rows || !n_features || !chain_dataset) return fail("bsr_set_datasets_mixed_host: null argument");
+  return set_datasets_mixed(h, "bsr_set_datasets_mixed_host", n_datasets, X, y, n_rows, n_features, 0, chain_dataset);
 }
 
 int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n, int32_t d, int64_t ld, int64_t n_total) {
@@ -338,6 +427,8 @@ int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n
   if (ld % 4 != 0 || ld < (n + 3) / 4 * 4 || ((uintptr_t)X & 15) || ((uintptr_t)y & 15))
     return fail("bsr_set_data_device: X and y must be 16-byte aligned, ld a multiple of 4 and >= n rounded up to 4 (rows are read as float4)");
   if (ld * (int64_t)d >= (int64_t)1 << 32) return fail("bsr_set_data_device: d * ld must stay below 2^32 elements per device (shard the rows)");
+  const std::vector<int32_t> one_ds((size_t)h->st.C, 0);
+  if (check_live_features(h, "bsr_set_data_device", 1, &d, one_ds.data())) return 1;
   CK(cudaSetDevice(h->cfg.device));
   free_data(h);
   h->n = n; h->d = d; h->ld = ld; h->n_total = n_total > 0 ? n_total : n;
@@ -351,7 +442,7 @@ int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n
     CK(cudaDeviceSynchronize());
     return 0;
   };
-  if (upload() || set_chain_datasets(h, 1, nullptr, nullptr)) {
+  if (upload() || set_chain_datasets(h, 1, nullptr, &d, nullptr)) {
     free_data(h);
     return 1;
   }
@@ -522,6 +613,19 @@ int bsr_set_state(bsr_handle* h, const uint32_t* tok, const double* pa, const do
   const size_t CKn = (size_t)st.C * st.K;
   for (size_t g = 0; g < CKn; ++g)
     if (nn[g] < 2 || nn[g] > BSR_MAXN) return fail("bsr_set_state: tree size out of range [2, 64]");
+  if (h->mixed)             // data sets of different feature counts: every leaf within its chain's own
+    for (size_t g = 0; g < CKn; ++g) {
+      const int32_t d = chain_features(h, (int)(g / st.K));
+      for (int j = 0; j < nn[g]; ++j) {
+        const uint32_t t = tok[g * BSR_MAXN + j];
+        if (tok_op(t) == OP_LEAF && tok_ft(t) >= d) {
+          char msg[200];
+          snprintf(msg, sizeof msg, "bsr_set_state: tree %d of chain %d reads feature %d; the chain's data set has %d features",
+                   (int)(g % st.K), (int)(g / st.K), tok_ft(t), (int)d);
+          return fail(msg);
+        }
+      }
+    }
   CK(cudaMemcpy(st.tok[0], tok, CKn * BSR_MAXN * sizeof(uint32_t), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(st.pa[0], pa, CKn * BSR_MAXN * sizeof(double), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(st.pb[0], pb, CKn * BSR_MAXN * sizeof(double), cudaMemcpyHostToDevice));
@@ -1153,7 +1257,7 @@ static int predict_groups(const char* name, int32_t device, int32_t M, int32_t K
     const unsigned tx = (unsigned)std::min<int64_t>(((max_n + 3) / 4 * 4 * d + 255) / 256, 148 * 16);
     for (int s0 = 0; s0 < S; s0 += 65535)
       k_transpose_datasets_in<double><<<dim3(tx, (unsigned)std::min(65535, S - s0)), 256>>>(
-          (const double*)(buf + o_X), (const int64_t*)(buf + o_soff) + s0, p.col_off + s0, (double*)(buf + o_xc), d);
+          (const double*)(buf + o_X), (const int64_t*)(buf + o_soff) + s0, p.col_off + s0, nullptr, nullptr, (double*)(buf + o_xc), d);
     CK(cudaGetLastError());
     const size_t smem = (size_t)K * BSR_MAXN * sizeof(EvTok<double>);
     const unsigned by = (unsigned)std::max<int64_t>(1, std::min<int64_t>(((chunk + 1) / 2 + 127) / 128, 64));
@@ -1226,7 +1330,7 @@ int bsr_predict_many(int32_t device, int32_t M, int32_t K, const uint32_t* tok, 
 int bsr_predict(bsr_handle* h, int32_t chain, int32_t reported, const double* X, int64_t n_test, int32_t d, double* out) {
   if (!h) return fail("null handle");
   if (chain < 0 || chain >= h->st.C) return fail("bsr_predict: chain out of range");
-  if (d != h->d) return fail("bsr_predict: feature count differs from the training data");
+  if (d != chain_features(h, chain)) return fail("bsr_predict: feature count differs from the training data");
   const int K = h->st.K, C = h->st.C;
   std::vector<uint32_t> tok((size_t)C * K * BSR_MAXN);
   std::vector<double> pa(tok.size()), pb(tok.size()), beta((size_t)C * (K + 1));

@@ -7,15 +7,21 @@
 
 struct bsr_handle {
   bsr_config cfg;
-  PriorTables pt;
-  PriorTables* d_pt = nullptr;   // device copy (the kernels read the tables from global memory)
+  // prior tables, one per distinct feature count of the data sets (ascending; one entry on a handle of one feature count), in
+  // global memory: the kernels read them there.  chain_pt [C] (device): the table of every chain's data set.
+  PriorTables* d_pt = nullptr;
+  int n_pt = 0;
+  int* chain_pt = nullptr;
   ChainState st;
   std::vector<void*> allocs;
-  // data: n_ds data sets of d features, X column-major [n_ds][d][ld], y [n_ds][ld]; data set b holds ds_n[b] rows (n: the largest,
-  // ld: n rounded up to 4), zeros past them
+  // data: n_ds data sets, X column-major [n_ds][d][ld], y [n_ds][ld]; data set b holds ds_n[b] rows (n: the largest, ld: n rounded
+  // up to 4), zeros past them, and ds_d[b] features (d: the largest), zero columns past them that no chain of it reads
   float* X32 = nullptr; double* X64 = nullptr; float* y32 = nullptr; double* y64 = nullptr;
   int n_ds = 1;
   uint32_t* ds_n = nullptr;      // [n_ds] (device)
+  std::vector<int32_t> ds_d;     // [n_ds] (host)
+  std::vector<int32_t> chain_ds; // [C] (host copy of st.ds)
+  bool mixed = false;            // the data sets differ in feature count
   bool own_x32 = false;
   double* stage = nullptr;       // device staging of the host data and its row offsets (bsr_set_data_host / bsr_set_datasets_*host)
   size_t stage_bytes = 0;

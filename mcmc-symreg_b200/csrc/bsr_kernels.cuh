@@ -23,11 +23,12 @@ struct ProposeCtx {
 };
 
 template <int MODE>
-__global__ void k_init_chains(ChainState st, const PriorTables* __restrict__ ptp) {
-  const PriorTables& pt = *ptp;   // tables live in global memory: indexed divergently, and out-of-line callees take them by reference
+__global__ void k_init_chains(ChainState st, const PriorTables* __restrict__ ptp, const int* __restrict__ chain_pt) {
   int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= st.C * st.K) return;
   int c = g / st.K, k = g % st.K;
+  const PriorTables& pt = ptp[chain_pt[c]];   // tables live in global memory: indexed divergently, and out-of-line callees take them by
+                                              // reference; one per feature count, the chain's data set's
   Draws<MODE> dr;
   dr.init_philox(st.key_seed[c], (uint64_t)st.key_id[c], (uint32_t)k, 0u);
   size_t slot = (size_t)g * BSR_MAXN;

@@ -158,18 +158,21 @@ __global__ void k_convert(const TI* in, TO* out, int64_t n) {
 
 // row-major float64 -> column-major T for several data sets: data set b = blockIdx.y is rows row_off[b] .. row_off[b + 1] of the
 // input and goes to out + col_off[b] * d with leading dimension ld = col_off[b + 1] - col_off[b], with zeros on the rows past its own
-// (up to ld).
+// (up to ld).  The output has d columns; with in_off / d_in (nullptr: every data set is n x d, starting at row_off[b] * d), data set b
+// is n x d_in[b] (row-major) from element in_off[b] of the input, and its columns d_in[b] .. d - 1 are zeros.
 // A handle's data sets share one ld (col_off[b] = b * ld); the test sets of bsr_predict_groups each have their own.
 template <typename TO>
-__global__ void k_transpose_datasets_in(const double* in, const int64_t* row_off, const int64_t* col_off, TO* out, int d) {
+__global__ void k_transpose_datasets_in(const double* in, const int64_t* row_off, const int64_t* col_off, const int64_t* in_off,
+                                        const int* d_in, TO* out, int d) {
   const int64_t r0 = row_off[blockIdx.y], n = row_off[blockIdx.y + 1] - r0;
   const int64_t ld = col_off[blockIdx.y + 1] - col_off[blockIdx.y];
-  in += (size_t)r0 * d;
+  const int db = d_in != nullptr ? d_in[blockIdx.y] : d;
+  in += in_off != nullptr ? in_off[blockIdx.y] : r0 * d;
   out += (size_t)col_off[blockIdx.y] * d;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < ld * d; i += (int64_t)gridDim.x * blockDim.x) {
     int64_t row = i / d;
     int col = (int)(i % d);
-    out[(int64_t)col * ld + row] = row < n ? (TO)in[i] : (TO)0;
+    out[(int64_t)col * ld + row] = (row < n && col < db) ? (TO)in[row * db + col] : (TO)0;
   }
 }
 

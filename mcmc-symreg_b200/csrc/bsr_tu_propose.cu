@@ -5,7 +5,7 @@
 
 int bsr_launch_init_chains(bsr_handle* h, cudaStream_t s) {
   const int total = h->cfg.n_chains * h->cfg.K;
-  k_init_chains<0><<<(total + 63) / 64, 64, 0, s>>>(h->st, h->d_pt);
+  k_init_chains<0><<<(total + 63) / 64, 64, 0, s>>>(h->st, h->d_pt, h->chain_pt);
   CK(cudaGetLastError());
   return 0;
 }

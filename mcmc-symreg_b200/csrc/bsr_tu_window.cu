@@ -260,9 +260,9 @@ static int launch_wpropose(bsr_handle* h, const WinState& ws, cudaStream_t s, Wi
   k_wclassify<<<(total + 255) / 256, 256, 0, s>>>(h->st, ws, wc);
   const int threads = 64;
   const dim3 blocks((total + threads - 1) / threads + BSR_N_BINS);
-  if (wc.tape != nullptr) k_wpropose<1><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc);
-  else if (wc.rec_draws != nullptr) k_wpropose<2><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc);
-  else k_wpropose<0><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc);
+  if (wc.tape != nullptr) k_wpropose<1><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc, h->chain_pt);
+  else if (wc.rec_draws != nullptr) k_wpropose<2><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc, h->chain_pt);
+  else k_wpropose<0><<<blocks, threads, 0, s>>>(h->st, ws, h->d_pt, wc, h->chain_pt);
   k_wdedup<<<wc.cn, BSR_MAXW, 0, s>>>(h->st, ws, wc);
   CK(cudaGetLastError());
   return 0;
@@ -418,7 +418,7 @@ int bsr_window_refit(bsr_handle* h, cudaStream_t s) {
   const int threads = BSR_WEVAL_THREADS;
   CK(cudaMemsetAsync(h->ws.chead, 0xFF, (size_t)C, s));   // the live state is being refitted: no window of the past is a record cache
   if (h->ws.lcol_ok) CK(cudaMemsetAsync(h->ws.lcol_ok, 0, (size_t)C * K, s));   // ... and no cached column is a live tree's
-  k_wlive_prior<<<(C * K + 127) / 128, 128, 0, s>>>(h->st, h->d_pt);
+  k_wlive_prior<<<(C * K + 127) / 128, 128, 0, s>>>(h->st, h->d_pt, h->chain_pt);
   if (h->cfg.precision == 0) {
     CK(cudaMemsetAsync(h->st.live_bad, 0, (size_t)C * K, s));
     k_wlive_bad<<<dim3(C, S), threads, 0, s>>>(h->st, wc, S);

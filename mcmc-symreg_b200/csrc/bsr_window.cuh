@@ -218,8 +218,8 @@ static __global__ void k_wclassify(ChainState st, WinState ws, WinCtx wc) {
                           // kernel was no longer instruction-cache bound)
 #endif
 template <int MODE>
-__global__ void __launch_bounds__(64, BSR_WPROP_MINB) k_wpropose(ChainState st, WinState ws, const PriorTables* __restrict__ ptp, WinCtx wc) {
-  const PriorTables& pt = *ptp;
+__global__ void __launch_bounds__(64, BSR_WPROP_MINB) k_wpropose(ChainState st, WinState ws, const PriorTables* __restrict__ ptp, WinCtx wc,
+                                                                const int* __restrict__ chain_pt) {
   // block -> (move, first slot of the move's bucket): the buckets are laid end to end in units of blocks, so the grid holds the
   // blocks that have work plus at most one partly filled block per move (a grid of moves x all slots launched six empty blocks
   // for every working one)
@@ -261,7 +261,7 @@ __global__ void __launch_bounds__(64, BSR_WPROP_MINB) k_wpropose(ChainState st, 
   const size_t slot = (size_t)g * BSR_MAXN, wslot = wi * BSR_MAXN;
   PropInfo info;
   const WinState wv = win_half(ws, win_parity(ws, c), K);
-  propose_one<MODE>(pt, st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, st.nn[w][g], st.sa[g], st.sb[g], dr,
+  propose_one<MODE>(ptp[chain_pt[c]], st.tok[w] + slot, st.pa[w] + slot, st.pb[w] + slot, st.nn[w][g], st.sa[g], st.sb[g], dr,
                     wv.tok + wslot, wv.pa + wslot, wv.pb + wslot, wv.nn + wi, info, st.lfs + 2 * (size_t)g);
   wv.info[wi] = info;
   // what the duplicate search (k_wdedup) compares: computed here, where the tree was just written (L1 / L2 hot)
@@ -1027,7 +1027,7 @@ __device__ __forceinline__ int live_counts(const uint32_t* tk, int m) {
   const int D = det_count(tk, m, m - T);
   return m | (L << 8) | (T << 16) | (D << 24);
 }
-static __global__ void k_wlive_prior(ChainState st, const PriorTables* __restrict__ ptp) {
+static __global__ void k_wlive_prior(ChainState st, const PriorTables* __restrict__ ptp, const int* __restrict__ chain_pt) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= st.C * st.K) return;
   const int w = st.which[g];
@@ -1037,7 +1037,7 @@ static __global__ void k_wlive_prior(ChainState st, const PriorTables* __restric
   for (int j = 0; j < m; ++j) tk[j] = st.tok[w][slot + j];
   st.lcnt[g] = live_counts(tk, m);
   double ll, lp;
-  fstruc_tree(*ptp, tk, m, st.pa[w] + slot, st.pb[w] + slot, st.sa[g], st.sb[g], ll, lp);
+  fstruc_tree(ptp[chain_pt[g / st.K]], tk, m, st.pa[w] + slot, st.pb[w] + slot, st.sa[g], st.sb[g], ll, lp);
   st.lfs[2 * (size_t)g] = ll; st.lfs[2 * (size_t)g + 1] = lp;
 }
 

@@ -11,8 +11,12 @@
 3. Engine throughput: D data sets x 50 chains on n = 100 rows (the first of --rows), fixed sweeps, device-timed (CUDA events)
    proposals per second.  With several sizes, one more line: the largest D with the data sets cycling through the sizes (a ragged
    batch, every chain on its own rows) against the same chains on data sets of the largest size.
+4. A suite of different feature counts (``mixed``): d in {1, 2, 3, 5, 8} x R repeats on n = 100 rows (the first of --rows), the
+   synthetic targets of ``mixed_target``, BSR(3, 50, val=100).  The loop of BSR.fit calls against one
+   BSR.fit_many(mixed_features=True), alternated, each timing ending in a device synchronise, results compared.
 
     python scripts/bench_fit_many.py [--repeats 50] [--rounds 3] [--sweeps 300] [--datasets 1,16,128,1024] [--rows 100 | 30,100,300,1000]
+                                     [--sections suite,summaries,engine,mixed]
 """
 import argparse
 import json
@@ -163,6 +167,56 @@ def bench_engine(D, sweeps, n, C=50, K=3):
     return dict(datasets=D, chains=D * C, rows=n if np.isscalar(n) else list(n), sweeps=sweeps, device_ms=ms, proposals=p1 - p0, proposals_per_s=(p1 - p0) / (ms * 1e-3))
 
 
+MIXED_FEATURES = (1, 2, 3, 5, 8)
+
+
+def mixed_target(X):
+    """y of the mixed suite on an (n, d) X: sum_j g_j(x_j) / (j + 1) with g_j cycling through x, x^2, sin x, cos x, plus the
+    interaction x_0 x_{d-1} when d > 1"""
+    g = (lambda v: v, lambda v: v * v, np.sin, np.cos)
+    y = sum(g[j % 4](X[:, j]) / (j + 1) for j in range(X.shape[1]))
+    return y + (X[:, 0] * X[:, -1] if X.shape[1] > 1 else 0.0)
+
+
+def bench_mixed(repeats, rounds, n):
+    """fit loop against fit_many(mixed_features=True) on data sets of 1 ... 8 features"""
+    import torch
+    from sklearn.base import clone
+    from mcmc_symreg_b200 import BSR
+    rng = np.random.default_rng(12345)
+    feats = [d for d in MIXED_FEATURES for _ in range(repeats)]
+    pairs = []
+    for d in feats:
+        X = rng.uniform(-3, 3, (n, d))
+        pairs.append((X, mixed_target(X)))
+    seeds = list(range(len(pairs)))
+    est = BSR(3, 50, val=100)
+
+    def loop():
+        out = [clone(est).set_params(seed=s) for s in seeds]
+        for e, (X, y) in zip(out, pairs):
+            e.fit(X, y)
+        torch.cuda.synchronize()
+        return out
+
+    def batch():
+        out = est.fit_many(pairs, seeds=seeds, mixed_features=True)
+        torch.cuda.synchronize()
+        return out
+
+    loop(); batch()                               # module loads, allocations
+    t_loop, t_batch, equal = [], [], True
+    for _ in range(rounds):
+        t0 = time.perf_counter(); a = loop(); t_loop.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); b = batch(); t_batch.append(time.perf_counter() - t0)
+        equal = equal and all(fingerprint(x) == fingerprint(y) for x, y in zip(a, b))
+    assert equal, "fit_many(mixed_features=True) and the loop of fits disagree"
+    return dict(datasets=len(pairs), features=list(MIXED_FEATURES), repeats=repeats, chains_per_fit=50, rows=n, loop_seconds=t_loop,
+                fit_many_seconds=t_batch, loop_ms_per_fit=1e3 * float(np.median(t_loop)) / len(pairs),
+                fit_many_ms_per_fit=1e3 * float(np.median(t_batch)) / len(pairs), speedup_median=float(np.median(t_loop) / np.median(t_batch)),
+                results_equal=equal)
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("--repeats", type=int, default=50)
@@ -170,7 +224,9 @@ def main(argv=None):
     ap.add_argument("--rows", default="100", help="rows per data set, or a comma list of sizes (30,100,300,1000)")
     ap.add_argument("--sweeps", type=int, default=300)
     ap.add_argument("--datasets", default="1,16,128,1024")
+    ap.add_argument("--sections", default="suite,summaries,engine,mixed", help="comma list of the sections to run")
     a = ap.parse_args(argv)
+    sections = set(a.sections.split(","))
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("bench_fit_many: needs a CUDA device")
@@ -180,10 +236,15 @@ def main(argv=None):
     out = dict(gpu=name, power_limit=power)
     sizes = [int(v) for v in a.rows.split(",")]
     Ds = [int(D) for D in a.datasets.split(",")]
-    out["suite"] = bench_suite(a.repeats, a.rounds, sizes)
-    out["summaries"] = bench_summaries(a.repeats, a.rounds, sizes)
-    out["engine"] = [bench_engine(D, a.sweeps, sizes[0]) for D in Ds]
-    if len(sizes) > 1:
+    if "suite" in sections:
+        out["suite"] = bench_suite(a.repeats, a.rounds, sizes)
+    if "summaries" in sections:
+        out["summaries"] = bench_summaries(a.repeats, a.rounds, sizes)
+    if "engine" in sections:
+        out["engine"] = [bench_engine(D, a.sweeps, sizes[0]) for D in Ds]
+    if "mixed" in sections:
+        out["mixed"] = bench_mixed(a.repeats, a.rounds, sizes[0])
+    if "engine" in sections and len(sizes) > 1:
         # the same chains on the ragged batch and on data sets of the largest size: what rows a chain does not hold cost nothing
         r, p = bench_engine(max(Ds), a.sweeps, sizes), bench_engine(max(Ds), a.sweeps, max(sizes))
         out["engine_ragged"] = dict(ragged=r, padded=p, throughput_ratio=r["proposals_per_s"] / p["proposals_per_s"])
