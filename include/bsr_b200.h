@@ -138,6 +138,31 @@ int bsr_set_datasets_ragged_host(bsr_handle* h, int32_t n_datasets, const double
 int bsr_set_datasets_mixed_host(bsr_handle* h, int32_t n_datasets, const double* X_rowmajor, const double* y, const int64_t* n_rows,
                                 const int32_t* n_features, const int32_t* chain_dataset);
 
+/* The settings of bsr_config a chain may take on its own: operator set and weights, split exponent and stop rule. */
+typedef struct bsr_prior {
+  int32_t n_ops;                   /* 1 .. BSR_MAX_OPS */
+  int32_t ops[BSR_MAX_OPS];        /* opcodes, as bsr_config.ops */
+  double op_weights[BSR_MAX_OPS];  /* positive, summing to 1 */
+  double beta;                     /* split prior exponent */
+  int32_t val;                     /* consecutive rejections that stop the chain; <= 0: never */
+  int32_t plateau_rule;            /* 1: RMSE plateau stop */
+  int32_t reserved[6];
+} bsr_prior;
+
+/* Chain c samples under priors[chain_prior[c]] (chain_prior: host array [n_chains], entries in [0, n_priors)): its proposals, tree
+ * prior and stop rule are those of a handle created with that prior in its bsr_config, so with chains keyed alike (and the data-set
+ * conditions of bsr_set_datasets_*) chain c ends bit for bit where that handle's chain ends.  A handle on which this is never called
+ * has one prior, taken from bsr_config.  Prior tables are built once per distinct (feature count, prior) pair that some chain uses;
+ * the chain -> prior map is independent of the chain -> data set map and survives every later bsr_set_data* / bsr_set_datasets_*
+ * call.  Refused, before anything changes (a failed call leaves the previous priors in place): null arguments, n_priors < 1, a prior
+ * bsr_create would refuse (n_ops outside 1 .. 16, an unknown opcode, a non-positive weight, weights not summing to 1), a chain_prior
+ * entry outside [0, n_priors), initialised chains (set the priors before bsr_init_chains* / bsr_set_state; initialising again
+ * afterwards is fine) and row-sharded handles.  A handle of several distinct priors is treated as one of several data sets: the
+ * proposal-by-proposal pipeline, the phase API (bsr_sweep_*), bsr_peer_export / bsr_peer_import and bsr_eval_trees refuse it, and
+ * bsr_set_state refuses an operator token whose op_ind is >= its chain's n_ops or whose opcode is not in its chain's operator set.
+ * Fits a grid of prior settings -- cross-validation over beta, operator sets, stop rules -- in one run. */
+int bsr_set_chain_priors(bsr_handle* h, int32_t n_priors, const bsr_prior* priors, const int32_t* chain_prior);
+
 /* Prior initialisation of every chain: sigma ~ IG(1), per tree sigma_a, sigma_b ~ IG(1) and grow()
  * (codes/bsr_class.py:123-142, codes/funcs.py:74-119), then the initial intercept OLS (bsr_class.py:147-163). */
 /* Every chain draws from Philox under its own key (seed, id): bsr_init_chains keys chain c with (seed, chain_offset + c),

@@ -110,7 +110,7 @@ class BSR(BaseEstimator, RegressorMixin):
             print("chains: %d  proposals: %d  accepts: %d  rank-rejects: %d" % (MM, c[:, 0].sum(), c[:, 1].sum(), c[:, 2].sum()))
         return
 
-    def fit_many(self, datasets, seeds=None, *, ragged=False, mixed_features=False):
+    def fit_many(self, datasets, seeds=None, *, ragged=False, mixed_features=False, params=None):
         """Fit this estimator to each of several data sets in one GPU run; returns one fitted ``BSR`` per data set.
 
         ``datasets``: a sequence of (X, y) pairs of the same shape (n rows, d features); with ``ragged=True`` the row counts may
@@ -135,10 +135,23 @@ class BSR(BaseEstimator, RegressorMixin):
 
         ``seeds``: one seed per data set; None gives every data set ``self.seed``, or, when that is None, draws one seed per
         data set from numpy's global state, in order, exactly as a loop of ``fit`` calls would.  The returned estimators
-        carry the parameters of ``self``."""
+        carry the parameters of ``self``.
+
+        ``params``: None, or one dict per entry of ``datasets`` overriding the settings ``GRID_PARAMS`` names (``beta``, ``ops``,
+        ``op_weights``, ``val``, ``plateau_rule`` and the inert ``alpha1``, ``alpha2``) for that entry: a grid of prior settings
+        over cross-validation folds in one run.  Estimator b then equals ``clone(self).set_params(seed=seeds[b], **params[b])
+        .fit(*datasets[b])`` under the same row-split conditions, and its ``get_params()`` carries the overrides.  Every other key
+        raises ValueError before any library call (``treeNum``, ``itrNum``, ``precision``, the sweep budgets, ``err_cap``, ``device``
+        and ``distributed`` shape the whole run).  Under ``fixed_sweeps`` the stop rule is off for every entry, as in ``fit``.
+        Entries whose X and y are the same objects as an earlier entry's share its upload (a grid of G settings over F folds
+        uploads F data sets)."""
+        datasets = list(datasets)
+        entries = grid_estimators(self, params, len(datasets))
         data = [(_as_matrix(X), np.asarray(y, dtype=np.float64).ravel()) for X, y in datasets]
         check_datasets(data, ragged, mixed_features)
         B = len(data)
+        uploads, entry_ds = shared_uploads(datasets)
+        data = [data[b] for b in uploads]
         seeds = dataset_seeds(self.seed, B, seeds)
         MM, K = int(self.itrNum), int(self.treeNum)
         opcodes, w = self._op_tables()
@@ -153,14 +166,17 @@ class BSR(BaseEstimator, RegressorMixin):
                               err_cap=int(self.err_cap), device=self._device_index(), chain_offset=lo)
             try:
                 g = np.arange(lo, hi)
-                ds, ids = g // MM, g % MM
+                entry, ids = g // MM, g % MM
+                ds = entry_ds[entry]
+                if entries is not None:
+                    eng.set_chain_priors([e._prior(fixed) for e in entries], entry)
                 if mixed_features:
                     eng.set_datasets_mixed([X for X, _ in data], [y for _, y in data], ds)
                 elif ragged:
                     eng.set_datasets_ragged([X for X, _ in data], [y for _, y in data], ds)
                 else:
                     eng.set_datasets(np.stack([X for X, _ in data]), np.stack([y for _, y in data]), ds)
-                eng.init_chains_keyed(np.asarray(seeds, dtype=object)[ds], ids)
+                eng.init_chains_keyed(np.asarray(seeds, dtype=object)[entry], ids)
                 if fixed:
                     eng.run(int(self.fixed_sweeps))
                     sweeps = int(self.fixed_sweeps)
@@ -172,8 +188,8 @@ class BSR(BaseEstimator, RegressorMixin):
                 eng.close()
         res = dist.gather_results(res, B * MM, K)
         fits = []
-        for part in parallel.split_results(res, B, MM):
-            est = type(self)(**self.get_params())
+        for b, part in enumerate(parallel.split_results(res, B, MM)):
+            est = type(self)(**(self if entries is None else entries[b]).get_params())
             est._set_results(part)
             fits.append(est)
         open_sets = [b for b, est in enumerate(fits) if not np.all(est.done_)]
@@ -269,6 +285,12 @@ class BSR(BaseEstimator, RegressorMixin):
         opcodes = [NAME_OP[o] if isinstance(o, str) else int(o) for o in ops]
         w = list(self.op_weights) if self.op_weights is not None else [1.0 / len(ops)] * len(ops)
         return opcodes, w
+
+    def _prior(self, fixed):
+        """this estimator's settings as ``capi.Engine.set_chain_priors`` takes them (the stop rule off under ``fixed_sweeps``)"""
+        opcodes, w = self._op_tables()
+        return dict(ops=opcodes, op_weights=w, beta=float(self.beta), val=(0 if fixed else int(self.val)),
+                    plateau_rule=(bool(self.plateau_rule) and not fixed))
 
     def _device_index(self):
         if self.device is not None:
@@ -369,6 +391,53 @@ def check_datasets(data, ragged=False, mixed_features=False):
         if not ragged and X.shape != (n, d):
             raise ValueError("fit_many: data set %d is %d x %d, data set 0 is %d x %d: all data sets must have the same shape%s"
                              % (b, X.shape[0], X.shape[1], n, d, " (ragged=True accepts different row counts)" if X.shape[1] == d else ""))
+
+
+GRID_PARAMS = ("beta", "ops", "op_weights", "val", "plateau_rule", "alpha1", "alpha2")
+
+
+def grid_estimators(est, params, n_entries):
+    """``fit_many``'s ``params``: None (returns None), or one dict per entry of keys in ``GRID_PARAMS``; returns the estimator of
+    every entry, ``est`` with the entry's overrides.  ValueError for a wrong length, any other key, an unknown operator name, or
+    operators and weights of different lengths -- all before any library call."""
+    if params is None:
+        return None
+    params = list(params)
+    if len(params) != n_entries:
+        raise ValueError("fit_many: %d params for %d data sets" % (len(params), n_entries))
+    known = est.get_params()
+    out = []
+    for b, p in enumerate(params):
+        for k in p:
+            if k in GRID_PARAMS:
+                continue
+            if k in known:
+                raise ValueError("fit_many: params[%d] sets %r, which every entry of one run shares; only %s may differ"
+                                 % (b, k, ", ".join(GRID_PARAMS)))
+            raise ValueError("fit_many: params[%d] sets %r, which is not a parameter of %s" % (b, k, type(est).__name__))
+        e = type(est)(**dict(known, **p))
+        ops = list(e.ops) if e.ops is not None else list(DEFAULT_OPS)
+        bad = [o for o in ops if isinstance(o, str) and o not in NAME_OP]
+        if bad:
+            raise ValueError("fit_many: params[%d]: unknown operator %r (known: %s)" % (b, bad[0], ", ".join(sorted(NAME_OP))))
+        opcodes, w = e._op_tables()
+        if len(w) != len(opcodes):
+            raise ValueError("fit_many: params[%d]: %d operators and %d op_weights" % (b, len(opcodes), len(w)))
+        out.append(e)
+    return out
+
+
+def shared_uploads(datasets):
+    """Entries of ``datasets`` whose X and y are the same objects as an earlier entry's share its upload: returns the entries
+    uploaded (first of each such group, in order) and every entry's index among them.  Compared by identity, not by value."""
+    first, uploads, entry_ds = {}, [], []
+    for b, (X, y) in enumerate(datasets):
+        key = (id(X), id(y))
+        if key not in first:
+            first[key] = len(uploads)
+            uploads.append(b)
+        entry_ds.append(first[key])
+    return uploads, np.asarray(entry_ds, dtype=np.int64)
 
 
 def check_same_engine(fits):

@@ -24,6 +24,11 @@ class BsrConfig(C.Structure):
                 ("device", C.c_int32), ("row_sharded", C.c_int32), ("reserved", C.c_int32 * 7)]
 
 
+class BsrPrior(C.Structure):
+    _fields_ = [("n_ops", C.c_int32), ("ops", C.c_int32 * MAX_OPS), ("op_weights", C.c_double * MAX_OPS), ("beta", C.c_double),
+                ("val", C.c_int32), ("plateau_rule", C.c_int32), ("reserved", C.c_int32 * 6)]
+
+
 _P = C.c_void_p
 _SIGS = {
     "bsr_last_error": (C.c_char_p, []),
@@ -36,6 +41,7 @@ _SIGS = {
     "bsr_set_datasets_host": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64, C.c_int32, _P]),
     "bsr_set_datasets_ragged_host": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P]),
     "bsr_set_datasets_mixed_host": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
+    "bsr_set_chain_priors": (C.c_int, [_P, C.c_int32, _P, _P]),
     "bsr_init_chains": (C.c_int, [_P, C.c_uint64]),
     "bsr_init_chains_keyed": (C.c_int, [_P, _P, _P]),
     "bsr_set_state": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, C.c_uint64]),
@@ -384,6 +390,24 @@ class Engine:
     def set_data_device(self, x_ptr, y_ptr, n, d, ld, n_total=0):
         self.n, self.d = int(n), int(d)
         _ck(self._lib.bsr_set_data_device(self._h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), int(n), int(d), int(ld), int(n_total)))
+
+    def set_chain_priors(self, priors, chain_prior):
+        """Chain c samples under ``priors[chain_prior[c]]``: dicts of ``ops`` (opcodes), ``op_weights``, ``beta``, ``val`` and
+        ``plateau_rule``, the settings of the constructor a chain may take on its own.  Call before ``init_chains*`` / ``set_state``."""
+        priors = list(priors)
+        arr = (BsrPrior * max(1, len(priors)))()
+        for p, d in zip(arr, priors):
+            ops, w = list(d["ops"]), list(d["op_weights"])
+            if len(ops) != len(w) or not 1 <= len(ops) <= MAX_OPS:
+                raise ValueError("set_chain_priors: every prior needs 1 .. %d opcodes and one weight per opcode" % MAX_OPS)
+            p.n_ops = len(ops)
+            for i, (o, x) in enumerate(zip(ops, w)):
+                p.ops[i], p.op_weights[i] = int(o), float(x)
+            p.beta, p.val, p.plateau_rule = float(d["beta"]), int(d["val"]), int(bool(d["plateau_rule"]))
+        cp = np.ascontiguousarray(chain_prior, dtype=np.int32).ravel()
+        if cp.size != self.C:
+            raise ValueError("chain_prior must hold one prior index per chain")
+        _ck(self._lib.bsr_set_chain_priors(self._h, len(priors), C.cast(arr, _P), _ptr(cp)))
 
     # ---- state ------------------------------------------------------------------------------------
     def init_chains(self, seed):

@@ -47,6 +47,55 @@ struct Carve {
 
 extern "C" {
 
+// What bsr_create refuses of an operator set and its weights (nullptr: nothing).
+static const char* prior_error(int n_ops, const int32_t* ops, const double* w) {
+  if (n_ops < 1 || n_ops > BSR_MAX_OPS) return "n_ops must be in [1, 16]";
+  double wsum = 0;
+  for (int i = 0; i < n_ops; ++i) {
+    if (ops[i] < OP_INV || ops[i] > OP_MUL) return "unknown opcode";
+    if (!(w[i] > 0)) return "operator weights must be positive";
+    wsum += w[i];
+  }
+  if (fabs(wsum - 1.0) > 1e-8) return "operator weights must sum to 1";
+  return nullptr;
+}
+
+// A prior as the handle keeps it: the entries past n_ops and the reserved fields zero, val <= 0 as 0, plateau_rule 0 / 1 -- so that
+// two priors that sample alike compare equal field by field.
+static bsr_prior canonical_prior(int n_ops, const int32_t* ops, const double* w, double beta, int32_t val, int32_t plateau_rule) {
+  bsr_prior p;
+  memset(&p, 0, sizeof p);
+  p.n_ops = n_ops;
+  for (int i = 0; i < n_ops; ++i) { p.ops[i] = ops[i]; p.op_weights[i] = w[i]; }
+  p.beta = beta;
+  p.val = val > 0 ? val : 0;
+  p.plateau_rule = plateau_rule != 0;
+  return p;
+}
+static bool same_prior(const bsr_prior& a, const bsr_prior& b) {
+  if (a.n_ops != b.n_ops || a.beta != b.beta || a.val != b.val || a.plateau_rule != b.plateau_rule) return false;
+  for (int i = 0; i < a.n_ops; ++i)
+    if (a.ops[i] != b.ops[i] || a.op_weights[i] != b.op_weights[i]) return false;
+  return true;
+}
+
+static int build_tables(bsr_handle* h);
+
+// Commits h->priors / h->chain_prior: the stop rule of every chain (chain_stop, read by k_wresolve; st.val / st.plateau_rule, read
+// by the proposal-by-proposal pipeline, when all chains share one prior) and, once there is data, the prior tables.
+static int commit_priors(bsr_handle* h) {
+  ChainState& st = h->st;
+  h->several_priors = h->priors.size() > 1;
+  if (!h->several_priors) { st.val = h->priors[0].val; st.plateau_rule = h->priors[0].plateau_rule; }
+  std::vector<int> stop((size_t)st.C);
+  for (int c = 0; c < st.C; ++c) {
+    const bsr_prior& p = h->priors[(size_t)h->chain_prior[(size_t)c]];
+    stop[(size_t)c] = (int)((uint32_t)p.val | (p.plateau_rule ? 0x80000000u : 0u));
+  }
+  CK(cudaMemcpy(h->chain_stop, stop.data(), stop.size() * sizeof(int), cudaMemcpyHostToDevice));
+  return h->X32 ? build_tables(h) : 0;
+}
+
 const char* bsr_last_error(void) { return g_err.c_str(); }
 int bsr_version(void) { return 100; }
 int bsr_max_nodes(void) { return BSR_MAXN; }
@@ -61,16 +110,7 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
     return fail("bsr_create: no CUDA device (this library has no CPU fallback)");
   if (cfg->device < 0 || cfg->device >= ndev) return fail("bsr_create: bad device ordinal");
   CK(cudaSetDevice(cfg->device));
-  bool has_unary = false;
-  double wsum = 0;
-  for (int i = 0; i < cfg->n_ops; ++i) {
-    if (cfg->ops[i] < OP_INV || cfg->ops[i] > OP_MUL) return fail("bsr_create: unknown opcode");
-    if (!(cfg->op_weights[i] > 0)) return fail("bsr_create: operator weights must be positive");
-    wsum += cfg->op_weights[i];
-    has_unary = has_unary || cfg->ops[i] < OP_ADD;
-  }
-  (void)has_unary;
-  if (fabs(wsum - 1.0) > 1e-8) return fail("bsr_create: operator weights must sum to 1");
+  if (const char* e = prior_error(cfg->n_ops, cfg->ops, cfg->op_weights)) return fail(std::string("bsr_create: ") + e);
   bsr_handle* h = new bsr_handle();
   h->cfg = *cfg;
   if (h->cfg.err_cap <= 0) h->cfg.err_cap = 512;
@@ -105,6 +145,7 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
   rc |= dalloc(h, &st.key_id, (size_t)C);
   rc |= dalloc(h, &st.ds, (size_t)C);
   rc |= dalloc(h, &h->chain_pt, (size_t)C);
+  rc |= dalloc(h, &h->chain_stop, (size_t)C);
   const int P = 2 * K;
   rc |= dalloc(h, &h->gram, (size_t)2 * C * (gram_n_sum(P) + P));   // [sums | maxs | per-chain scratch records]
   rc |= dalloc(h, &h->need64, (size_t)C);
@@ -112,7 +153,9 @@ int bsr_create(const bsr_config* cfg, bsr_handle** out) {
   rc |= dalloc(h, &h->d_count, 2);      // [1]: abort flag of the peer-memory exchange (k_wwait)
   rc |= dalloc(h, &h->ystats, 2);
   rc |= dalloc(h, &h->ds_n, 1);
-  if (rc) { bsr_destroy(h); return 1; }
+  h->priors.assign(1, canonical_prior(cfg->n_ops, cfg->ops, cfg->op_weights, cfg->beta, cfg->val, cfg->plateau_rule));
+  h->chain_prior.assign((size_t)C, 0);
+  if (rc || commit_priors(h)) { bsr_destroy(h); return 1; }
   for (int i = 0; i < 8; ++i) cudaEventCreate(&h->ev[i]);
   if (const char* e = getenv("BSR_SEQ_PIPELINE")) h->seq_pipeline = atoi(e) != 0;
   if (const char* e = getenv("BSR_WINDOW")) h->window = std::max(1, std::min(BSR_MAXW, atoi(e)));
@@ -140,38 +183,44 @@ int bsr_destroy(bsr_handle* h) {
   return 0;
 }
 
-static PriorTables prior_tables(const bsr_handle* h, int n_feature) {
+static PriorTables prior_tables(const bsr_prior& p, int n_feature) {
   PriorTables pt;
   memset(&pt, 0, sizeof pt);
-  pt.n_ops = h->cfg.n_ops;
+  pt.n_ops = p.n_ops;
   pt.n_feature = n_feature;
-  pt.beta = h->cfg.beta;
+  pt.beta = p.beta;
   double acc = 0;
   for (int i = 0; i < pt.n_ops; ++i) {
-    pt.ops[i] = h->cfg.ops[i];
-    pt.w[i] = h->cfg.op_weights[i];
+    pt.ops[i] = p.ops[i];
+    pt.w[i] = p.op_weights[i];
     pt.logw[i] = log(pt.w[i]);
     acc += pt.w[i];
     pt.cdf[i] = acc;
   }
   for (int dpt = 0; dpt <= BSR_MAXN; ++dpt) {
-    double ps = 1.0 / pow((double)(1 + dpt), -h->cfg.beta);   // codes/funcs.py:79
+    double ps = 1.0 / pow((double)(1 + dpt), -p.beta);   // codes/funcs.py:79
     pt.psplit[dpt] = ps;
-    pt.logsplit[dpt] = log((double)(1 + dpt)) * h->cfg.beta;  // codes/funcs.py:370
-    pt.log1m[dpt] = log(1.0 - ps);                            // codes/funcs.py:362-363 (-inf at depth 0)
+    pt.logsplit[dpt] = log((double)(1 + dpt)) * p.beta;  // codes/funcs.py:370
+    pt.log1m[dpt] = log(1.0 - ps);                       // codes/funcs.py:362-363 (-inf at depth 0)
   }
   pt.lognf = log((double)n_feature);
   return pt;
 }
 
-// One table per distinct feature count of the data sets (a table is ~2 KB; a handle may hold 65535 data sets), and the table
-// of every chain's data set (chain_pt).  A handle of one feature count has one table, entry 0, and every chain reads it.
+static int32_t chain_features(const bsr_handle* h, int c);
+
+// One table per distinct (feature count, prior) pair that some chain uses -- never one per chain or per data set (a table is ~2 KB;
+// a handle may hold 65535 data sets) -- and the table of every chain (chain_pt).  A handle of one feature count and one prior has one
+// table, entry 0, and every chain reads it.
 static int build_tables(bsr_handle* h) {
-  std::vector<int32_t> counts(h->ds_d);
-  std::sort(counts.begin(), counts.end());
-  counts.erase(std::unique(counts.begin(), counts.end()), counts.end());
+  const int C = h->st.C;
+  std::vector<int64_t> key((size_t)C);     // feature count << 32 | prior
+  for (int c = 0; c < C; ++c) key[(size_t)c] = ((int64_t)chain_features(h, c) << 32) | h->chain_prior[(size_t)c];
+  std::vector<int64_t> keys(key);
+  std::sort(keys.begin(), keys.end());
+  keys.erase(std::unique(keys.begin(), keys.end()), keys.end());
   std::vector<PriorTables> pt;
-  for (int32_t d : counts) pt.push_back(prior_tables(h, d));
+  for (int64_t k : keys) pt.push_back(prior_tables(h->priors[(size_t)(k & 0xffffffff)], (int)(k >> 32)));
   if ((int)pt.size() != h->n_pt) {
     dfree(h, h->d_pt);
     h->d_pt = nullptr; h->n_pt = 0;
@@ -179,9 +228,8 @@ static int build_tables(bsr_handle* h) {
     h->n_pt = (int)pt.size();
   }
   CK(cudaMemcpy(h->d_pt, pt.data(), pt.size() * sizeof(PriorTables), cudaMemcpyHostToDevice));
-  std::vector<int> idx((size_t)h->st.C);
-  for (int c = 0; c < h->st.C; ++c)
-    idx[(size_t)c] = (int)(std::lower_bound(counts.begin(), counts.end(), h->ds_d[(size_t)h->chain_ds[(size_t)c]]) - counts.begin());
+  std::vector<int> idx((size_t)C);
+  for (int c = 0; c < C; ++c) idx[(size_t)c] = (int)(std::lower_bound(keys.begin(), keys.end(), key[(size_t)c]) - keys.begin());
   CK(cudaMemcpy(h->chain_pt, idx.data(), idx.size() * sizeof(int), cudaMemcpyHostToDevice));
   return 0;
 }
@@ -449,6 +497,45 @@ int bsr_set_data_device(bsr_handle* h, const float* X, const float* y, int64_t n
   return finish_data(h);
 }
 
+int bsr_set_chain_priors(bsr_handle* h, int32_t n_priors, const bsr_prior* priors, const int32_t* chain_prior) {
+  if (!h || !priors || !chain_prior) return fail("bsr_set_chain_priors: null argument");
+  if (n_priors < 1) return fail("bsr_set_chain_priors: n_priors must be >= 1");
+  char msg[200];
+  for (int b = 0; b < n_priors; ++b)
+    if (const char* e = prior_error(priors[b].n_ops, priors[b].ops, priors[b].op_weights)) {
+      snprintf(msg, sizeof msg, "bsr_set_chain_priors: priors[%d]: %s", b, e);
+      return fail(msg);
+    }
+  const int C = h->st.C;
+  for (int c = 0; c < C; ++c)
+    if (chain_prior[c] < 0 || chain_prior[c] >= n_priors) {
+      snprintf(msg, sizeof msg, "bsr_set_chain_priors: chain_prior[%d] = %d is outside [0, %d)", c, (int)chain_prior[c], (int)n_priors);
+      return fail(msg);
+    }
+  if (h->cfg.row_sharded) return fail("bsr_set_chain_priors: not available on row-sharded handles");
+  if (h->initialised)
+    return fail("bsr_set_chain_priors: the chains are initialised (set the priors before bsr_init_chains* / bsr_set_state)");
+  // the distinct priors the chains use, in order of first use
+  std::vector<bsr_prior> uniq;
+  std::vector<int32_t> slot((size_t)n_priors, -1), cp((size_t)C);
+  for (int c = 0; c < C; ++c) {
+    int32_t& s = slot[(size_t)chain_prior[c]];
+    if (s < 0) {
+      const bsr_prior& q = priors[chain_prior[c]];
+      const bsr_prior p = canonical_prior(q.n_ops, q.ops, q.op_weights, q.beta, q.val, q.plateau_rule);
+      s = (int32_t)(std::find_if(uniq.begin(), uniq.end(), [&](const bsr_prior& u) { return same_prior(u, p); }) - uniq.begin());
+      if (s == (int32_t)uniq.size()) uniq.push_back(p);
+    }
+    cp[(size_t)c] = s;
+  }
+  if (uniq.size() > 1 && h->seq_pipeline)
+    return fail("bsr_set_chain_priors: several priors need the window path of bsr_run (this handle uses the proposal-by-proposal pipeline)");
+  CK(cudaSetDevice(h->cfg.device));
+  h->priors = uniq;
+  h->chain_prior = cp;
+  return commit_priors(h);
+}
+
 // global sum(y), y'y for row-sharded runs (the caller all-reduces the local values): entry 0 of the data sets' statistics
 int bsr_get_y_stats(bsr_handle* h, double* sum_y, double* yy) {
   if (!h || !sum_y || !yy) return fail("bsr_get_y_stats: null argument");
@@ -493,6 +580,7 @@ static int check_ready(bsr_handle* h) {
 // the proposal-by-proposal pipeline and the phase API read one data set
 static int check_one_dataset(bsr_handle* h, const char* fn) {
   if (h->n_ds > 1) return fail(std::string(fn) + ": not available on a handle with several data sets (bsr_set_datasets_host); use bsr_run");
+  if (h->several_priors) return fail(std::string(fn) + ": not available on a handle with several priors (bsr_set_chain_priors); use bsr_run");
   return 0;
 }
 
@@ -622,6 +710,25 @@ int bsr_set_state(bsr_handle* h, const uint32_t* tok, const double* pa, const do
           char msg[200];
           snprintf(msg, sizeof msg, "bsr_set_state: tree %d of chain %d reads feature %d; the chain's data set has %d features",
                    (int)(g % st.K), (int)(g / st.K), tok_ft(t), (int)d);
+          return fail(msg);
+        }
+      }
+    }
+  if (h->several_priors)     // chains of different priors: every operator within its chain's own set (op_ind indexes its weights)
+    for (size_t g = 0; g < CKn; ++g) {
+      const bsr_prior& p = h->priors[(size_t)h->chain_prior[g / st.K]];
+      for (int j = 0; j < nn[g]; ++j) {
+        const uint32_t t = tok[g * BSR_MAXN + j];
+        const int op = tok_op(t), oi = tok_oi(t);
+        if (op == OP_LEAF) continue;
+        if (oi >= p.n_ops || std::find(p.ops, p.ops + p.n_ops, op) == p.ops + p.n_ops) {
+          char msg[240];
+          if (oi >= p.n_ops)
+            snprintf(msg, sizeof msg, "bsr_set_state: tree %d of chain %d has op_ind %d; the chain's prior has %d operators",
+                     (int)(g % st.K), (int)(g / st.K), oi, (int)p.n_ops);
+          else
+            snprintf(msg, sizeof msg, "bsr_set_state: tree %d of chain %d holds opcode %d, which is not in the chain's operator set",
+                     (int)(g % st.K), (int)(g / st.K), op);
           return fail(msg);
         }
       }

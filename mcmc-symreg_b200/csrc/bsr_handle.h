@@ -7,11 +7,16 @@
 
 struct bsr_handle {
   bsr_config cfg;
-  // prior tables, one per distinct feature count of the data sets (ascending; one entry on a handle of one feature count), in
-  // global memory: the kernels read them there.  chain_pt [C] (device): the table of every chain's data set.
+  // prior tables, one per distinct (feature count, prior) pair the chains use (one entry on a handle of one feature count and one
+  // prior), in global memory: the kernels read them there.  chain_pt [C] (device): the table of every chain.
   PriorTables* d_pt = nullptr;
   int n_pt = 0;
   int* chain_pt = nullptr;
+  // priors (bsr_set_chain_priors; bsr_create: the one prior of bsr_config), distinct, and the prior of every chain (host)
+  std::vector<bsr_prior> priors;
+  std::vector<int32_t> chain_prior;
+  bool several_priors = false;   // the chains use more than one prior
+  int* chain_stop = nullptr;     // [C] (device) stop rule of every chain: val (0: never) | plateau rule << 31 (k_wresolve)
   ChainState st;
   std::vector<void*> allocs;
   // data: n_ds data sets, X column-major [n_ds][d][ld], y [n_ds][ld]; data set b holds ds_n[b] rows (n: the largest, ld: n rounded

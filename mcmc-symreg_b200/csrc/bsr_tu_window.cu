@@ -107,9 +107,10 @@ static int ensure_window(bsr_handle* h, int S) {
     const size_t CW = (size_t)C * W;
     // the per-slot arrays hold R windows per chain (WinState: the earlier windows are the record cache of the current one): as many
     // as BSR_WIN_RING, fewer when they would take more than a third of the free device memory (65536 chains: 5.4 GB per window)
-    // (a handle with the stop rule on runs its chains for val consecutive rejections -- ~140 proposals per chain at val = 100, accepts every
+    // (a handle whose chains all have the stop rule on runs them for val consecutive rejections -- ~140 proposals per chain at val = 100, accepts every
     // hundred proposals: earlier windows are rarely valid, and a 30-ms fit should not allocate 2.7 GB: two windows)
-    int R = h->cfg.val > 0 ? 2 : BSR_WIN_RING;
+    const bool all_stop = std::all_of(h->priors.begin(), h->priors.end(), [](const bsr_prior& p) { return p.val > 0; });
+    int R = all_stop ? 2 : BSR_WIN_RING;
     if (const char* e = getenv("BSR_WIN_RING_DEPTH")) R = std::max(2, std::min(BSR_WIN_RING, atoi(e)));
     {
       size_t free_b = 0, total_b = 0;
@@ -268,25 +269,27 @@ static int launch_wpropose(bsr_handle* h, const WinState& ws, cudaStream_t s, Wi
   return 0;
 }
 
-template <bool MULTI>
+template <bool MULTI, bool PRIORS>
 static int launch_wresolve_m(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc) {
   const int K = h->cfg.K;
   const int threads = 128, lpc = ws.W > 32 ? 64 : 32, cpb = threads / lpc, blocks = (wc.cn + cpb - 1) / cpb;
   const size_t smem = (size_t)cpb * (sg_size(K) * sizeof(double) + 8 * sizeof(unsigned));
   switch (K) {
-    case 1: k_wresolve<1, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 2: k_wresolve<2, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 3: k_wresolve<3, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 4: k_wresolve<4, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 5: k_wresolve<5, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
-    case 10: k_wresolve<10, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;     // BASELINE configs[2]
-    default: k_wresolve<0, MULTI><<<blocks, threads, smem, s>>>(h->st, ws, wc); break;
+    case 1: k_wresolve<1, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
+    case 2: k_wresolve<2, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
+    case 3: k_wresolve<3, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
+    case 4: k_wresolve<4, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
+    case 5: k_wresolve<5, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
+    case 10: k_wresolve<10, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;     // BASELINE configs[2]
+    default: k_wresolve<0, MULTI, PRIORS><<<blocks, threads, smem, s>>>(h->st, ws, wc, h->chain_stop); break;
   }
   CK(cudaGetLastError());
   return 0;
 }
+// a handle of one data set runs the instances without a data-set term, one of one prior those without per-chain stop rules
 static int launch_wresolve(bsr_handle* h, const WinState& ws, cudaStream_t s, const WinCtx& wc) {
-  return h->n_ds > 1 ? launch_wresolve_m<true>(h, ws, s, wc) : launch_wresolve_m<false>(h, ws, s, wc);
+  if (h->several_priors) return h->n_ds > 1 ? launch_wresolve_m<true, true>(h, ws, s, wc) : launch_wresolve_m<false, true>(h, ws, s, wc);
+  return h->n_ds > 1 ? launch_wresolve_m<true, false>(h, ws, s, wc) : launch_wresolve_m<false, false>(h, ws, s, wc);
 }
 
 static WinCtx make_wc(bsr_handle* h, long long p_start, long long p_target, uint32_t rps, uint32_t TR) {
@@ -530,6 +533,7 @@ int bsr_get_window_geometry(bsr_handle* h, int64_t* geom5) {
 int bsr_peer_export(bsr_handle* h, int32_t world, void* ipc_handle_out) {
   if (!h || !ipc_handle_out) return bsr_fail("bsr_peer_export: null argument");
   if (h->n_ds > 1) return bsr_fail("bsr_peer_export: not available on a handle with several data sets (bsr_set_datasets_host)");
+  if (h->several_priors) return bsr_fail("bsr_peer_export: not available on a handle with several priors (bsr_set_chain_priors)");
   if (!h->cfg.row_sharded) return bsr_fail("bsr_peer_export: the handle was not created with row_sharded = 1");
   if (!h->X32) return bsr_fail("bsr_peer_export: call bsr_set_data_* first (the exchange buffer is sized from the data)");
   if (world < 1 || world > BSR_MAX_PEERS) return bsr_fail("bsr_peer_export: world must be in [1, 8]");
@@ -560,6 +564,7 @@ int bsr_peer_export(bsr_handle* h, int32_t world, void* ipc_handle_out) {
 int bsr_peer_import(bsr_handle* h, int32_t rank, int32_t world, const void* ipc_handles) {
   if (!h || !ipc_handles) return bsr_fail("bsr_peer_import: null argument");
   if (h->n_ds > 1) return bsr_fail("bsr_peer_import: not available on a handle with several data sets (bsr_set_datasets_host)");
+  if (h->several_priors) return bsr_fail("bsr_peer_import: not available on a handle with several priors (bsr_set_chain_priors)");
   if (!h->xbuf) return bsr_fail("bsr_peer_import: call bsr_peer_export first");
   if (world < 1 || world > BSR_MAX_PEERS || rank < 0 || rank >= world) return bsr_fail("bsr_peer_import: bad rank / world");
   CK(cudaSetDevice(h->cfg.device));

@@ -1182,9 +1182,12 @@ __global__ void __launch_bounds__(BSR_WEVAL_THREADS) k_wlive_gram(ChainState st,
 #endif
 // MULTI: as for k_weval -- the chain's sum(y), y'y come from its data set's entry of wc.ystats, else from wc.sum_y, wc.yy; its row
 // count from wc.ds_n (else wc.n_total, wc.n_local: a handle of several data sets is never row-sharded, so the two are one number),
-// and its records from the splits that hold its rows.
-template <int KT, bool MULTI>
-__global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(ChainState st, WinState ws, WinCtx wc) {
+// and its records from the splits that hold its rows.  PRIORS: the chains differ in their stop rule (bsr_set_chain_priors), chain c's
+// is chain_stop[c] = val (0: never) | plateau rule << 31; else every chain's is st.val, st.plateau_rule and chain_stop is not read (the
+// instances of one prior are those of a handle without per-chain priors, register for register).
+template <int KT, bool MULTI, bool PRIORS>
+__global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(ChainState st, WinState ws, WinCtx wc,
+                                                                               const int* __restrict__ chain_stop) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int LD = (KT > 0) ? KT + 1 : BSR_LDA;
   constexpr int PC = (KT > 0) ? KT + 1 : BSR_MAXK + 1;
@@ -1333,6 +1336,8 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
     if (!live) return;
   }
   int total = st.total[c];
+  const int stop_rule = PRIORS ? chain_stop[c] : 0;
+  const int val = PRIORS ? (stop_rule & 0x7fffffff) : st.val;
   int n_cons = 0, a = -1;
   bool done = false;
   {
@@ -1343,9 +1348,9 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
     n_cons = first_acc ? __ffsll((long long)first_acc) : n_valid;
     if (first_acc) a = n_cons - 1;
     // ... or up to the sweep boundary at which `total` consecutive rejections reach val (bsr_class.py:174)
-    if (st.val > 0) {
+    if (val > 0) {
       const int k0 = (int)(p0 % K);
-      int need = st.val - total;                      // rejections still missing
+      int need = val - total;                         // rejections still missing
       if (need < 1) need = 1;
       int stop = need + ((K - (k0 + need) % K) % K);  // first slot count >= need that ends a sweep
       if (stop <= n_cons - (a >= 0 ? 1 : 0)) { n_cons = stop; a = -1; done = true; }
@@ -1440,7 +1445,7 @@ __global__ void __launch_bounds__(128, (KT > 0 ? BSR_WRES_MINB : 1)) k_wresolve(
       ++nerr;
       st.nerr[c] = nerr;
       // plateau rule (bsr_class.py:248-252): len(errList) > 100 and 1 - min(last10)/mean(last10) < 0.05
-      if (st.plateau_rule && nerr > 100) {
+      if ((PRIORS ? stop_rule < 0 : st.plateau_rule != 0) && nerr > 100) {
         const int have = nerr < st.err_cap ? nerr : st.err_cap;
         const int k10 = have < 10 ? have : 10;
         double mn = DBL_MAX, sm = 0.0;

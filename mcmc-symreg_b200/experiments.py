@@ -11,6 +11,7 @@ The genetic-programming comparison of the script (gplearn, ``codes/simulations.p
 """
 import argparse
 import json
+import sys
 import time
 
 import numpy as np
@@ -126,41 +127,51 @@ def suite_jobs(funcs, repeats, n_train=100, seed=0):
     return [(f, n, r, seed + r) for f in funcs for n in sizes for r in range(repeats)]
 
 
-def run_suite(funcs=("f1", "f2", "f3", "f4", "f5", "f6"), repeats=1, batched=False, **kw):
+def run_suite(funcs=("f1", "f2", "f3", "f4", "f5", "f6"), repeats=1, batched=False, params=None, **kw):
     """The whole benchmark suite (the paper's Table 1 recipe: every function, ``repeats`` independent data sets).
 
     ``n_train`` may be a sequence of training sizes: the suite then runs every function at every size (a learning curve), and every
-    row carries its ``n_train``.  batched=True fits all data sets in one GPU run (``BSR.fit_many``, ``ragged=True`` for several
-    sizes) with the seeds the loop uses and summarizes the fits with one grouped prediction call (``summarize_many``); the rows are the
-    loop's rows, except that ``fit_seconds`` is the batch's wall clock (fit and
-    summaries) divided by the number of data sets, and ``batch_seconds`` is that wall clock."""
+    row carries its ``n_train``.  ``params``: None, or a list of dicts of estimator settings (``beta``, ``ops``, ``op_weights``, ``val``,
+    ``plateau_rule``): every (function, size, repeat) job then runs once per dict, job by job, and every row carries its ``params``.
+    batched=True fits all data sets in one GPU run (``BSR.fit_many``, ``ragged=True`` for several sizes, one upload per job and
+    ``params`` for the settings) with the seeds the loop uses and summarizes the fits with one grouped prediction call
+    (``summarize_many``); the rows are the loop's rows, except that ``fit_seconds`` is the batch's wall clock (fit and summaries)
+    divided by the number of fits, and ``batch_seconds`` is that wall clock."""
     rows = []
     seed0 = kw.pop("seed", 0)
     n_train = kw.pop("n_train", 100)
     grid = not np.isscalar(n_train)
     jobs = suite_jobs(funcs, repeats, n_train, seed0)
+    settings = [None] if params is None else [dict(p) for p in params]
+    runs = [(job, p) for job in jobs for p in settings]
     if not batched:
-        for f, n, r, s in jobs:
-            out, _, _ = run_experiment(f, n_train=n, seed=s, **kw)
+        for (f, n, r, s), p in runs:
+            out, _, _ = run_experiment(f, n_train=n, seed=s, **dict(kw, **(p or {})))
             if grid:
                 out["n_train"] = n
             out["repeat"] = r
+            if p is not None:
+                out["params"] = p
             rows.append(out)
         return rows
     from .bsr_class import BSR
     K, MM, n_test, val = kw.pop("K", 3), kw.pop("MM", 50), kw.pop("n_test", 30), kw.pop("val", 100)
     data_seed = kw.pop("data_seed", None)
     data = [make_dataset(f, n, n_test, seed=s if data_seed is None else data_seed) for f, n, _, s in jobs]
+    run_data = [d for d in data for _ in settings]
     t0 = time.perf_counter()
-    fits = BSR(K, MM, val=val, **kw).fit_many([(d["X"], d["y"]) for d in data], seeds=[s for _, _, _, s in jobs], ragged=grid)
-    rows = summarize_many(fits, data)
+    fits = BSR(K, MM, val=val, **kw).fit_many([(d["X"], d["y"]) for d in run_data], seeds=[s for (_, _, _, s), _ in runs], ragged=grid,
+                                              params=None if params is None else [p for _, p in runs])
+    rows = summarize_many(fits, run_data)
     batch = time.perf_counter() - t0
-    for o, (_, n, r, _) in zip(rows, jobs):
-        o["fit_seconds"] = batch / len(jobs)
+    for o, ((_, n, r, _), p) in zip(rows, runs):
+        o["fit_seconds"] = batch / len(runs)
         o["batch_seconds"] = batch
         if grid:
             o["n_train"] = n
         o["repeat"] = r
+        if p is not None:
+            o["params"] = p
     return rows
 
 
@@ -178,6 +189,11 @@ def _sizes(text):
     return tuple(parts) if "," in text else parts[0]
 
 
+def _floats(text):
+    """--beta: a comma list of numbers"""
+    return [float(v) for v in text.split(",") if v.strip()]
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="BSR benchmark-function experiments on the GPU (codes/simulations.py recipe)")
     ap.add_argument("--func", default="sim", help="one of %s, or 'all'" % ", ".join(sorted(TARGETS)))
@@ -191,14 +207,22 @@ def main(argv=None):
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp64"])
     ap.add_argument("--json", action="store_true", help="one JSON object per experiment instead of the table")
     ap.add_argument("--batched", action="store_true", help="fit all (function, size, repeat) data sets in one GPU run (BSR.fit_many)")
+    ap.add_argument("--beta", type=_floats, default=None, help="split exponents to run every data set with, a comma list (-1,-0.5,-2)")
+    argv = list(sys.argv[1:] if argv is None else argv)
+    # "--beta -1,-0.5": argparse takes a value that starts with "-" and is not a single number for an option
+    argv = [a + "=" + argv[i + 1] if a == "--beta" and i + 1 < len(argv) else a for i, a in enumerate(argv)
+            if not (i > 0 and argv[i - 1] == "--beta")]
     a = ap.parse_args(argv)
     funcs = ("f1", "f2", "f3", "f4", "f5", "f6") if a.func == "all" else (a.func,)
-    rows = run_suite(funcs, a.repeats, batched=a.batched, K=a.K, MM=a.MM, n_train=a.n_train, n_test=a.n_test, val=a.val, seed=a.seed,
-                     precision=a.precision)
+    params = None if a.beta is None else [dict(beta=b) for b in a.beta]
+    rows = run_suite(funcs, a.repeats, batched=a.batched, params=params, K=a.K, MM=a.MM, n_train=a.n_train, n_test=a.n_test, val=a.val,
+                     seed=a.seed, precision=a.precision)
     for o in rows:
         if a.json:
             print(json.dumps(o))
         else:
+            if "params" in o:
+                print("     params %s" % json.dumps(o["params"], sort_keys=True))
             print(format_row(o))
             print("     target     y = %s" % o["formula"])
             print("     best model y = %.4g + %s" % (o["beta_best"][0], " + ".join("%.4g * [%s]" % (b, e) for b, e in zip(o["beta_best"][1:], o["model_best"]))))

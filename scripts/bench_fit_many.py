@@ -14,9 +14,13 @@
 4. A suite of different feature counts (``mixed``): d in {1, 2, 3, 5, 8} x R repeats on n = 100 rows (the first of --rows), the
    synthetic targets of ``mixed_target``, BSR(3, 50, val=100).  The loop of BSR.fit calls against one
    BSR.fit_many(mixed_features=True), alternated, each timing ending in a device synchronise, results compared.
+5. A grid of prior settings (``grid``): f1 ... f6 x 10 repeats (--grid-repeats) on n = 100 rows (the first of --rows), each with
+   beta in {-1, -0.5, -2} x {the default operators, GRID_OPS7: seven operators with non-uniform weights}, BSR(3, 50, val=100).  The
+   loop of BSR.fit calls (one per data set and setting) against one BSR.fit_many(params=...), in which the settings of a data set
+   share its upload, alternated, each timing ending in a device synchronise, results compared.
 
     python scripts/bench_fit_many.py [--repeats 50] [--rounds 3] [--sweeps 300] [--datasets 1,16,128,1024] [--rows 100 | 30,100,300,1000]
-                                     [--sections suite,summaries,engine,mixed]
+                                     [--grid-repeats 10] [--sections suite,summaries,engine,mixed,grid]
 """
 import argparse
 import json
@@ -49,7 +53,9 @@ def suite_data(repeats, sizes):
 
 
 def fingerprint(est):
-    return (est.model(), [b.ravel().tolist() for b in est.betas_], est.train_err_, est.counters_.tolist(), est.done_.tolist())
+    """what must be equal bit for bit; floats as bytes, so that a NaN beta (a degenerate intercept fit) equals itself"""
+    return (est.model(), [b.tobytes() for b in est.betas_], [np.asarray(e, dtype=np.float64).tobytes() for e in est.train_err_],
+            est.counters_.tolist(), est.done_.tolist())
 
 
 def bench_suite(repeats, rounds, sizes):
@@ -217,6 +223,52 @@ def bench_mixed(repeats, rounds, n):
                 results_equal=equal)
 
 
+GRID_BETAS = (-1.0, -0.5, -2.0)
+GRID_OPS7 = dict(ops=["+", "*", "sin", "cos", "exp", "square", "ln"], op_weights=[0.3, 0.2, 0.1, 0.1, 0.1, 0.1, 0.1])
+
+
+def bench_grid(repeats, rounds, n):
+    """fit loop against fit_many(params=...) over a grid of beta x operator sets, every data set uploaded once"""
+    import torch
+    from sklearn.base import clone
+    from mcmc_symreg_b200 import BSR
+    jobs, data = suite_data(repeats, [n])
+    grid = [dict(beta=b, **ops) for b in GRID_BETAS for ops in (dict(ops=None, op_weights=None), GRID_OPS7)]
+    pairs = [(d["X"], d["y"]) for d in data for _ in grid]          # the same objects for every setting of a data set
+    seeds = [s for _, _, _, s in jobs for _ in grid]
+    params = [p for _ in data for p in grid]
+    est = BSR(3, 50, val=100)
+
+    def loop():
+        out = [clone(est).set_params(seed=s, **p) for s, p in zip(seeds, params)]
+        for e, (X, y) in zip(out, pairs):
+            e.fit(X, y)
+        torch.cuda.synchronize()
+        return out
+
+    def batch():
+        out = est.fit_many(pairs, seeds=seeds, params=params)
+        torch.cuda.synchronize()
+        return out
+
+    loop(); batch()                               # module loads, allocations
+    t_loop, t_batch, equal = [], [], True
+    for _ in range(rounds):
+        t0 = time.perf_counter(); a = loop(); t_loop.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); b = batch(); t_batch.append(time.perf_counter() - t0)
+        for i, (x, y) in enumerate(zip(a, b)):
+            fx, fy = fingerprint(x), fingerprint(y)
+            if fx != fy:
+                parts = [name for name, u, v in zip(("model", "betas", "train_err", "counters", "done"), fx, fy) if u != v]
+                raise AssertionError("fit_many(params=...) and the loop of fits disagree: fit %d (params %s) differs in %s: %s / %s"
+                                     % (i, params[i], parts, [u for u, v in zip(fx[1], fy[1]) if u != v][:2],
+                                        [v for u, v in zip(fx[1], fy[1]) if u != v][:2]))
+    return dict(fits=len(pairs), datasets=len(data), settings=len(grid), betas=list(GRID_BETAS), ops7=GRID_OPS7, repeats=repeats,
+                chains_per_fit=50, rows=n, loop_seconds=t_loop, fit_many_seconds=t_batch,
+                loop_ms_per_fit=1e3 * float(np.median(t_loop)) / len(pairs), fit_many_ms_per_fit=1e3 * float(np.median(t_batch)) / len(pairs),
+                speedup_median=float(np.median(t_loop) / np.median(t_batch)), results_equal=equal)
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("--repeats", type=int, default=50)
@@ -224,7 +276,8 @@ def main(argv=None):
     ap.add_argument("--rows", default="100", help="rows per data set, or a comma list of sizes (30,100,300,1000)")
     ap.add_argument("--sweeps", type=int, default=300)
     ap.add_argument("--datasets", default="1,16,128,1024")
-    ap.add_argument("--sections", default="suite,summaries,engine,mixed", help="comma list of the sections to run")
+    ap.add_argument("--grid-repeats", type=int, default=10, help="repeats of every function in the grid section")
+    ap.add_argument("--sections", default="suite,summaries,engine,mixed,grid", help="comma list of the sections to run")
     a = ap.parse_args(argv)
     sections = set(a.sections.split(","))
     import torch
@@ -244,6 +297,8 @@ def main(argv=None):
         out["engine"] = [bench_engine(D, a.sweeps, sizes[0]) for D in Ds]
     if "mixed" in sections:
         out["mixed"] = bench_mixed(a.repeats, a.rounds, sizes[0])
+    if "grid" in sections:
+        out["grid"] = bench_grid(a.grid_repeats, a.rounds, sizes[0])
     if "engine" in sections and len(sizes) > 1:
         # the same chains on the ragged batch and on data sets of the largest size: what rows a chain does not hold cost nothing
         r, p = bench_engine(max(Ds), a.sweeps, sizes), bench_engine(max(Ds), a.sweeps, max(sizes))
